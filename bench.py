@@ -2,6 +2,7 @@
 """Contract benchmark of the RAG stereo hot path (cost volume + disparity regression) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload infer|train|router|sweep192|sweep288] [--impl reference]
+                    [--dump-outputs DIR]
 
 A step = one pass of the hot path over one batch of synthetic stereo pairs.  Default workload
 (BASELINE.json configs[1]): inference batch 8 per GPU at DrivingStereo half-res 400x880, which the
@@ -25,8 +26,8 @@ Prints ONE JSON line (rank 0).  Top level:
   e2e                   the same metric through rag_b200.pipeline.HostPipeline (HostTrainPipeline for `train`): pinned HOST
                         buffers, ONE host->device and ONE device->host copy per step inside the timed region, and the box's
                         host->device ceiling measured in the same run (`frac_of_h2d_ceiling`);
-  cpu_baseline          the UNMODIFIED reference (baseline/_ref, tools/install_ref.sh) timed on this box's host cores
-                        (kind "reference"; "port" = the oracle restatement when baseline/_ref is absent);
+  cpu_baseline          the UNMODIFIED reference (oracle/_ref, tools/install_ref.sh) timed on this box's host cores
+                        (kind "reference"; "port" = the oracle restatement when oracle/_ref is absent);
   torch_cuda_reference  the same unmodified reference modules run by PyTorch eager on this GPU (the honest GPU bar);
   next_rows             the SURVEY.md section 8f rows (fused stem, last_3_3d conv, ...) beside the headline.
 `--impl reference` times the reference's own CPU implementation on the same config (rank 0 only).
@@ -94,12 +95,12 @@ def ncu_traffic(kernel):
 
 
 # --------------------------------------------------------------------------------------------
-# the reference: the unmodified modules from baseline/_ref when installed, else the oracle port
+# the reference: the unmodified modules from oracle/_ref when installed, else the oracle port
 # --------------------------------------------------------------------------------------------
 class Reference:
     """Callable view of the reference's hot path.  kind == "reference": rag_model.Network.forward's own lines 375-383
     (driven through stub feature/matching callables, as tests/golden/make_golden.py does) and rag_model.Disp, imported
-    unmodified from baseline/_ref; kind == "port": oracle/rag_oracle.py (the same op sequence restated)."""
+    unmodified from oracle/_ref; kind == "port": oracle/rag_oracle.py (the same op sequence restated)."""
 
     def __init__(self, cpu: bool):
         import types
@@ -203,14 +204,14 @@ def cpu_reference(workload, warmup=1, steps=3, budget_s=25.0):
         "sample": f"1 pair of the {workload} workload per step ({3*hf}x{3*wf}, maxdisp {md}, {'fwd+bwd' if bwd else 'fwd'}), mean of {len(times)} steps after warm-up, "
                   f"torch {torch.__version__} CPU, {torch.get_num_threads()} threads; pairs are independent, so pairs/s does not depend on the batch "
                   "(the reference head needs ~1.8 GB of temporaries per pair at 480x960)",
-        "what": ("unmodified reference: models.rag_model.Network.forward lines 375-383 + models.rag_model.Disp from baseline/_ref" if refm.kind == "reference"
-                 else "oracle port of rag_model.py:375-383,18-44 (baseline/_ref not installed)"),
+        "what": ("unmodified reference: models.rag_model.Network.forward lines 375-383 + models.rag_model.Disp from oracle/_ref" if refm.kind == "reference"
+                 else "oracle port of rag_model.py:375-383,18-44 (oracle/_ref not installed)"),
     }, times
 
 
 def config1_full_network_cpu(budget_s=20.0):
     """BASELINE.json configs[0] / BASELINE.md section 4.5: the reference's full Network.forward (Feature Net + cost volume +
-    Matching Net + head), synthetic 1x3x288x576, maxdisp 192, on the host cores.  Needs baseline/_ref."""
+    Matching Net + head), synthetic 1x3x288x576, maxdisp 192, on the host cores.  Needs oracle/_ref."""
     import torch
 
     from oracle import refimport as R
@@ -260,7 +261,7 @@ def run_reference(args):
     if rank != 0:
         return
     b, c, hf, wf, df, md, bwd, desc = WORKLOADS[args.workload]
-    base, times = cpu_reference(args.workload, warmup=args.warmup, steps=args.steps, budget_s=90.0)
+    base, times = cpu_reference(args.workload, warmup=args.warmup, steps=args.steps, budget_s=float("inf"))   # exactly --steps
     v = base["value"]
     line = {
         "impl": "reference", "metric": METRIC, "value": v, "unit": "pairs/s", "n_gpus": args.gpus,
@@ -334,7 +335,7 @@ class ClockSampler:
 # GPU arm
 # --------------------------------------------------------------------------------------------
 def torch_cuda_reference(workload, dev, reps=5):
-    """The UNMODIFIED reference modules (baseline/_ref; oracle port if absent) run by PyTorch eager ON THE SAME GPU: the
+    """The UNMODIFIED reference modules (oracle/_ref; oracle port if absent) run by PyTorch eager ON THE SAME GPU: the
     honest GPU baseline (SURVEY.md section 8d).  One pair per call (its temporaries are ~1.8 GB/pair at 480x960)."""
     import torch
 
@@ -556,6 +557,47 @@ def tail_rows(dev):
 
 EXTRA_NEXT_ROWS = [("stem3d0_train", stem_train_row), ("tail_train", tail_rows)]     # (name, fn(dev) -> dict)
 
+DUMP_BYTES = 60 * 2**20         # --dump-outputs: all arrays together stay under 64 MB, .npy headers included
+DUMP_ARRAY_BYTES = 16 * 2**20   # an output larger than its share is stored as a sample of its elements
+DUMP_SEED = 20240601
+
+
+def sample_outputs(outputs):
+    """{name: [device tensor per call]} (the calls' results concatenated along dim 0 are the output) -> {name: (float32 numpy
+    array, description)}.  An output of at most min(DUMP_ARRAY_BYTES, DUMP_BYTES / #outputs) bytes is kept whole; a larger
+    one becomes `<name>_sample`: its elements at sorted flat indices (row-major over the concatenated shape) drawn with
+    DUMP_SEED, which depend only on the shape, so two builds run with the same arguments compare element for element."""
+    import torch
+
+    cap = min(DUMP_ARRAY_BYTES, DUMP_BYTES // len(outputs))
+    out = {}
+    for name, parts in outputs.items():
+        shape = [sum(p.shape[0] for p in parts)] + list(parts[0].shape[1:])
+        per = parts[0].numel()
+        total = per * len(parts)
+        if total * 4 <= cap:
+            out[name] = (torch.cat([p.float().cpu() for p in parts]).numpy(), {"shape": shape, "stored": "all"})
+            continue
+        g = torch.Generator().manual_seed(DUMP_SEED)
+        idx = torch.unique(torch.randint(total, (cap // 4,), generator=g))      # sorted, no repeats
+        vals = torch.empty(idx.numel(), dtype=torch.float32)
+        for j, p in enumerate(parts):
+            sel = (idx >= j * per) & (idx < (j + 1) * per)
+            vals[sel] = p.reshape(-1)[(idx[sel] - j * per).to(p.device)].float().cpu()
+        out[name + "_sample"] = (vals.numpy(), {"shape": shape, "stored": "%d elements at seeded flat indices (seed %d)" % (idx.numel(), DUMP_SEED)})
+    return out
+
+
+def write_outputs(sampled, out_dir):
+    """Write sample_outputs()' arrays as out_dir/<name>.npy; returns their description for the JSON line."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (arr, _) in sampled.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+    return {"dir": out_dir, "step": "last timed step of the overlapped pass", "dtype": "float32",
+            "arrays": {name: desc for name, (_, desc) in sampled.items()}}
+
 
 def run_gpu(args):
     import torch
@@ -595,8 +637,9 @@ def run_gpu(args):
     peak, peak_src = measured_peak()
     sampler = ClockSampler(local) if rank == 0 else None
 
-    def measure(workload, with_clocks):
-        """Serial pass (kernels back to back on one stream, events around each) + overlapped pass (two streams)."""
+    def measure(workload, with_clocks, dump=False):
+        """Serial pass (kernels back to back on one stream, events around each) + overlapped pass (two streams).  With
+        `dump`, the record's "outputs" holds sample_outputs() of the timed pass's last step."""
         b, c, hf, wf, df, md, bwd, desc = WORKLOADS[workload]
         # identical bits for CPU reference and GPU: generate on the host with a fixed seed, then copy
         g = torch.Generator().manual_seed(1234 + rank)
@@ -661,8 +704,7 @@ def run_gpu(args):
             opath.join()
             t1.record()
             torch.cuda.synchronize()
-            del outs
-            return t0.elapsed_time(t1)
+            return t0.elapsed_time(t1), outs
 
         def graph_pass():
             """The same two-stream step captured ONCE into a CUDA graph (fork/join included) and replayed K times."""
@@ -687,12 +729,17 @@ def run_gpu(args):
         serial_ms = serial_pass()
         barrier()
         n0 = _cabi.launch_count()
-        eager_ms = overlapped_pass()       # untimed for `value`: a second, independent sample of the same schedule
+        eager_ms = overlapped_pass()[0]    # untimed for `value`: a second, independent sample of the same schedule
         barrier()
         n0 = _cabi.launch_count()
         if with_clocks and sampler: sampler.start()
-        total_ms = overlapped_pass()
+        total_ms, outs = overlapped_pass()
         clocks = sampler.stop() if (with_clocks and sampler) else None
+        # what the caller of the timed path received in its last step, reduced to host arrays before anything else runs
+        names = ("cost", "disp", "gcl", "gx", "gy") if bwd else ("cost", "disp")
+        parts = [outs] if bwd else outs            # inference: one (cost, disp, stats) per sub-batch call
+        dumped = sample_outputs({n: [p[i] for p in parts] for i, n in enumerate(names)}) if dump else None
+        del outs, parts
         # --graph: additionally time the same two-stream step captured ONCE into a CUDA graph and replayed (one host launch per
         # step).  Reported beside the headline, never as it: the launch order of the two branches inside a graph is not
         # defined, and the SM-sharing only works when the persistent volume kernel is dispatched first (0.42 or 0.53 ms per
@@ -750,16 +797,17 @@ def run_gpu(args):
             "note": "the head kernels are FP32-pipe bound (one exp2 + 7-12 FP32 ops per pixel per low-res bin), not HBM bound; see DESIGN.md",
         }
         rec = {"value": world * b * K / (total_ms * 1e-3), "value_serial": world * b * K / (serial_ms * 1e-3), "ms_per_step": step_ms,
-               "ms_per_step_serial": sstep_ms, "schedule": "overlapped, CUDA-graph replay" if used_graph else "overlapped, eager two-stream", "roofline": roofline, "path": path, "gpu_launches": int(launches), "clocks": clocks}
+               "ms_per_step_serial": sstep_ms, "schedule": "overlapped, CUDA-graph replay" if used_graph else "overlapped, eager two-stream", "roofline": roofline, "path": path, "gpu_launches": int(launches), "clocks": clocks,
+               "outputs": dumped}
         return rec, (x, y, cl, gcost, gdisp)
 
-    main, tensors = measure(args.workload, with_clocks=True)
+    main, tensors = measure(args.workload, with_clocks=True, dump=args.dump_outputs is not None and rank == 0)
     b, c, hf, wf, df, md, bwd, desc = WORKLOADS[args.workload]
     x, y, cl, gcost, gdisp = tensors
 
     # ---- e2e: HOST buffers through the public pipeline (ONE H2D + kernels + ONE D2H per step) ----
     pipe = HostTrainPipeline(md, dev) if bwd else HostPipeline(md, dev)
-    Ke = max(3, min(K, 50))
+    Ke = K
     gh = torch.Generator().manual_seed(99 + rank)
 
     def host_step():
@@ -883,6 +931,8 @@ def run_gpu(args):
             "cpu_baseline": cpu, "config1_full_network_cpu": config1, "torch_cuda_reference": torch_gpu, "next_rows": next_rows,
             "e2e": e2e, "gpu_launches": main["gpu_launches"], "clocks": main["clocks"],
         }
+        if args.dump_outputs is not None:
+            line["dump_outputs"] = write_outputs(main["outputs"], args.dump_outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -900,7 +950,13 @@ def main():
                     help="kernel variants of the two-stream schedule (rag_b200.pipeline.SCHEDULES)")
     ap.add_argument("--graph", action="store_true", help="additionally time the two-stream step as CUDA-graph replays (path.overlapped_graph)")
     ap.add_argument("--no-train-record", action="store_true", help="default workload only: skip the configs[2] training sub-record")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (float32; see sample_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,9 +1,10 @@
 """Import the UNMODIFIED reference (chzhang18/RAG ``src/``) -- TEST / BASELINE INFRASTRUCTURE ONLY.
 
 The reference is a tree of plain Python files without a package or a setup.py; ``tools/install_ref.sh``
-copies it to the git-ignored ``baseline/_ref/src`` (which travels to the GPU box).  This helper puts that
-directory on ``sys.path`` and imports the modules the hot path lives in.  Nothing under ``rag_b200/`` imports
-this file; users are ``tests/``, ``__graft_entry__.smoke()`` and bench.py's reference / cpu_baseline legs.
+(run by ``__graft_entry__.build()``) copies it to the git-ignored ``oracle/_ref/src``, inside the repository tree, so
+that it goes wherever the built tree goes.  This helper reads the reference from there only: it puts that directory
+on ``sys.path`` and imports the modules the hot path lives in.  Nothing under ``rag_b200/`` imports this file; users
+are ``tests/``, ``__graft_entry__.smoke()`` and bench.py's reference / cpu_baseline legs.
 
 On a machine without a CUDA driver the reference's head cannot run as written (``rag_model.py:26`` builds its
 ``arange`` on ``torch.cuda.current_device()``); ``cpu_patch=True`` applies the one monkeypatch that makes the
@@ -17,14 +18,12 @@ import sys
 import types
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CANDIDATES = (os.path.join(ROOT, "baseline", "_ref", "src"), "/root/reference/src")
+BASE = os.path.join(ROOT, "oracle", "_ref")
+SRC = os.path.join(BASE, "src")
 
 
 def ref_src() -> str | None:
-    for c in CANDIDATES:
-        if os.path.isdir(os.path.join(c, "models")):
-            return c
-    return None
+    return SRC if os.path.isdir(os.path.join(SRC, "models")) else None
 
 
 def available() -> bool:
@@ -32,16 +31,14 @@ def available() -> bool:
 
 
 def verify_manifest() -> int:
-    """Check baseline/_ref against the sha256 manifest written at install time; returns #files checked."""
-    base = os.path.join(ROOT, "baseline", "_ref")
-    man = os.path.join(base, "MANIFEST.sha256")
+    """Check oracle/_ref against the sha256 manifest written at install time; returns #files checked."""
     n = 0
-    with open(man) as f:
+    with open(os.path.join(BASE, "MANIFEST.sha256")) as f:
         for line in f:
             digest, rel = line.split()
-            with open(os.path.join(base, "src", rel), "rb") as g:
+            with open(os.path.join(SRC, rel), "rb") as g:
                 if hashlib.sha256(g.read()).hexdigest() != digest:
-                    raise RuntimeError(f"baseline/_ref/src/{rel} differs from the installed reference")
+                    raise RuntimeError(f"oracle/_ref/src/{rel} differs from the installed reference")
             n += 1
     return n
 
@@ -51,7 +48,7 @@ def import_reference(cpu_patch: bool = False) -> types.SimpleNamespace:
     genotypes_2d, utils, metrics.  Raises RuntimeError when the reference is not installed."""
     src = ref_src()
     if src is None:
-        raise RuntimeError("the reference is not installed: run tools/install_ref.sh in the build container")
+        raise RuntimeError("the reference is not installed: run tools/install_ref.sh (RAG_REFERENCE = a checkout of it)")
     if src not in sys.path:
         sys.path.insert(0, src)
     if cpu_patch:

@@ -40,3 +40,29 @@ class MirrorNet(nn.Module):
 
 def arch(i):
     return {"stem2d": [i], "last2d": [i], "stem3d": [i], "last3d": [i]}
+
+
+def reference_modules():
+    """Fresh stand-ins for the three reference modules that ``rag_b200.network.install()`` rebinds, with the names it
+    touches: ``models.rag_model`` (``Network.forward`` / ``search_forward``, ``Disp``, ``DisparityRegression``, ``nn``),
+    ``automl.mdenas_basicmodel`` (``BasicNetwork.forward``, ``Disp``, ``DisparityRegression``) and
+    ``automl.operations_3d`` (``ConvBR_3d.forward``).  Only the bindings are real: the stand-in methods raise."""
+    import types
+
+    def unpatched(*args, **kwargs):
+        raise NotImplementedError("stand-in of a reference method: only its binding exists")
+
+    def cls(name, *methods):                    # a distinct function object per method, so a crossed restore is visible
+        return type(name, (nn.Module,), {m: (lambda *a, **k: unpatched()) for m in methods})
+
+    def module(name, **attrs):
+        m = types.ModuleType(name)
+        m.__dict__.update(attrs)
+        return m
+
+    rag_model = module("models.rag_model", nn=nn, Network=cls("Network", "forward", "search_forward"),
+                       Disp=cls("Disp", "forward"), DisparityRegression=cls("DisparityRegression", "forward"))
+    mdenas_basicmodel = module("automl.mdenas_basicmodel", BasicNetwork=cls("BasicNetwork", "forward"),
+                               Disp=cls("Disp", "forward"), DisparityRegression=cls("DisparityRegression", "forward"))
+    operations_3d = module("automl.operations_3d", ConvBR_3d=cls("ConvBR_3d", "forward"))
+    return rag_model, mdenas_basicmodel, operations_3d

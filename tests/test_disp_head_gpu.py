@@ -248,7 +248,7 @@ def test_full_size_properties(F_):
 
 
 def _reference_head(md):
-    """The unmodified reference's Disp (baseline/_ref) when installed, else the oracle port of the same lines."""
+    """The unmodified reference's Disp (oracle/_ref) when installed, else the oracle port of the same lines."""
     from oracle import refimport as R
 
     if R.available():

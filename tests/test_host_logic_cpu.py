@@ -1,7 +1,6 @@
 """CPU tests of the host-side logic: metric reduction semantics against the reference goldens,
 pair sharding, the world_size-2 gloo path of the metric all-reduce, and install() on the reference."""
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -92,21 +91,25 @@ def test_metric_allreduce_gloo_world2():
         assert abs(got[k] - want[k]) <= 1e-12 * max(1.0, abs(want[k])), k
 
 
-REF = "/root/reference/src"
+def _reference_modules():
+    """(rag_model, mdenas_basicmodel, operations_3d): the unmodified reference's modules when oracle/_ref is installed,
+    else stand-ins with the names install() rebinds (tests/_mirror_net.py)."""
+    from oracle import refimport as R
+    from tests._mirror_net import reference_modules
+
+    if R.available():
+        ref = R.import_reference()
+        return ref.rag_model, ref.mdenas_basicmodel, ref.operations_3d
+    return reference_modules()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (only in the build container)")
 def test_install_patches_the_reference_classes():
-    """install() on the UNMODIFIED reference: the three forwards and the head classes are swapped, a
-    network built afterwards is stateless in its head, and a CPU call fails loudly (no fallback)."""
-    sys.path.insert(0, REF)
-    try:
-        import automl.mdenas_basicmodel as mb
-        import models.rag_model as rm
-    finally:
-        sys.path.remove(REF)
+    """install() on the reference modules (the unmodified ones when installed, else stand-ins): the three forwards and the
+    head classes are swapped, a network built afterwards is stateless in its head, and a CPU call fails loudly (no fallback)."""
     from rag_b200 import network as N
     from rag_b200.modules import Disp
+
+    rm, mb, _ = _reference_modules()
 
     orig = rm.Network.forward
     done = N.install(rm, mb)
@@ -126,20 +129,15 @@ def test_install_patches_the_reference_classes():
         rm.Network.forward = orig
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (only in the build container)")
 def test_install_uninstall_flags_and_upsample_proxy_on_the_reference():
-    """install() / uninstall() bookkeeping on the UNMODIFIED reference (CPU: only the bindings, no kernels): every binding is
-    restored, install(fuse_stem=False) after a fused install switches the default off, and install(upsample=True) exposes
-    rag_b200.upsample.Upsample as rag_model.nn.Upsample while every other name still resolves to torch.nn."""
-    sys.path.insert(0, REF)
-    try:
-        import automl.mdenas_basicmodel as mb
-        import automl.operations_3d as ops3d
-        import models.rag_model as rm
-    finally:
-        sys.path.remove(REF)
+    """install() / uninstall() bookkeeping on the reference modules (the unmodified ones when installed, else stand-ins; CPU:
+    only the bindings, no kernels): every binding is restored, install(fuse_stem=False) after a fused install switches the
+    default off, and install(upsample=True) exposes rag_b200.upsample.Upsample as rag_model.nn.Upsample while every other
+    name still resolves to torch.nn."""
     from rag_b200 import network as N
     from rag_b200.upsample import Upsample
+
+    rm, mb, ops3d = _reference_modules()
 
     N.uninstall()
     orig = (rm.Network.forward, rm.Network.search_forward, mb.BasicNetwork.forward, ops3d.ConvBR_3d.forward, rm.Disp, rm.nn)
@@ -167,17 +165,19 @@ def test_install_uninstall_flags_and_upsample_proxy_on_the_reference():
     assert rm.nn is torch.nn and not N._FUSE_STEM and not N._STEM_AWARE
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (only in the build container)")
 def test_refimport_installs_and_verifies_the_reference(tmp_path):
-    """tools/install_ref.sh + oracle/refimport.py: the copy under baseline/_ref is byte-identical (sha256 manifest), imports, and the
+    """tools/install_ref.sh + oracle/refimport.py: the copy under oracle/_ref is byte-identical (sha256 manifest), imports, and the
     scoped CPU monkeypatch restores torch.cuda.current_device."""
     import subprocess
 
     from oracle import refimport as R
 
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    subprocess.run(["bash", os.path.join(root, "tools", "install_ref.sh")], check=True, capture_output=True)
-    assert R.available() and R.verify_manifest() >= 20
+    res = subprocess.run(["bash", os.path.join(root, "tools", "install_ref.sh")], capture_output=True, text=True)
+    assert res.returncode in (0, 3), res.stderr               # 3: no checkout of the reference to install from
+    if not R.available():
+        pytest.skip("the unmodified reference is neither installed in oracle/_ref nor available to tools/install_ref.sh")
+    assert R.verify_manifest() >= 20
     ref = R.import_reference(cpu_patch=True)
     g = R.make_genotype(ref, 0)
     assert g.normal.shape == (6, 2) and g.reduce.shape == (6, 2) and set(g.normal[:, 1]) <= {0, 1}

@@ -1,7 +1,7 @@
 """The drop-in proven on the REAL reference network, on the GPU (SURVEY.md section 8 N-0; VERDICT r1 #1).
 
-``baseline/_ref/src`` is the unmodified reference installed by ``tools/install_ref.sh`` (git-ignored, travels to
-the GPU box).  These tests build the reference's own ``Network(genotype, device)`` and ``BasicNetwork`` on CUDA and
+``oracle/_ref/src`` is the unmodified reference installed by ``tools/install_ref.sh`` (run by ``build()``; git-ignored,
+inside the tree).  These tests build the reference's own ``Network(genotype, device)`` and ``BasicNetwork`` on CUDA and
 compare the UNPATCHED reference forward/backward with the ``rag_b200.network.install()``-patched one on the same
 weights and inputs:
 
@@ -31,8 +31,8 @@ sys.path.insert(0, ROOT)
 from oracle import refimport as R  # noqa: E402
 
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "src", "models")),
-                                 reason="baseline/_ref absent: run tools/install_ref.sh in the build container")]
+              pytest.mark.skipif(not R.available(),
+                                 reason="the unmodified reference is not installed in oracle/_ref (tools/install_ref.sh, run by build())")]
 
 H, W = 96, 192          # image size: multiples of 6 with H/3, W/3 even down to /4 (the Matching Net's level 2)
 

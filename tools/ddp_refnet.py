@@ -3,7 +3,7 @@ EPE/D1 metric sums and DDP gradients when training".
 
     python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/ddp_refnet.py
 
-Per rank: the unmodified reference `Network` (baseline/_ref) with rag_b200.network.install(fuse_stem=True, upsample=True), stereo
+Per rank: the unmodified reference `Network` (oracle/_ref) with rag_b200.network.install(fuse_stem=True, upsample=True), stereo
 pairs sharded across ranks, the fused masked loss, DDP gradient all-reduce, SGD step (approaches/rag.py:205-216), then the
 growth step `expand` -> `select` with DDP RE-WRAPPED (parameters are added / deleted / frozen per task), a step on the grown
 path, and the metric all-reduce.  Checks: weights identical on every rank after each phase; the world-N run reproduces the

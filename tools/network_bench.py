@@ -1,4 +1,4 @@
-"""Whole-network timing of the REAL reference Network (baseline/_ref) on this GPU, unpatched vs rag_b200.network.install():
+"""Whole-network timing of the REAL reference Network (oracle/_ref) on this GPU, unpatched vs rag_b200.network.install():
 how much of a full forward / training step the hot path (and the rows next to it) is worth end to end.
 
     python tools/network_bench.py [--size 288x576] [--batch 4]
