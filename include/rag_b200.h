@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define RAG_B200_ABI_VERSION 13
+#define RAG_B200_ABI_VERSION 14
 
 #if defined(__GNUC__)
 #define RAG_API __attribute__((visibility("default")))
@@ -252,6 +252,29 @@ RAG_API int rag_conv3d_c1_fwd(const float* in, const float* w, float* out, int B
 RAG_API size_t rag_conv3d_c1_bwd_workspace_bytes(int C);
 RAG_API int rag_conv3d_c1_bwd(const float* g, const float* in, const float* w, float* gin, float* gw, void* workspace,
                       int B, int C, int D, int H, int W, void* stream);
+
+/* The Matching Net's interior 3x3x3 layers: ConvBR_3d(C, O, 3, 1, 1) of src/automl/operations_3d.py:31-47 = bias-free
+ * Conv3d C -> O (3x3x3, stride 1, zero padding 1) + BatchNorm3d + ReLU -- `stem3d1` (12 -> 12, src/models/rag_model.py) and
+ * the `conv_3x3` ops of the Cell_3d's.  Compiled for (C, O) in {(4,4), (8,8), (12,12)}; any other pair is RAG_E_SHAPE.  fp32 accumulation (cuDNN's default for these layers is TF32).  Stateless and capturable.
+ * Forward:  out[b,o,p] = relu?( fma(z[b,o,p], scale[o], shift[o]) ),  z[b,o,p] = sum_{c,k} w[o,c,k] in[b,c,p+k-1]
+ *   in [B,C,D,H,W]; w [O,C,3,3,3] (Conv3d.weight); scale / shift [O] (both NULL = identity: raw z, the training path;
+ *   eval-mode BatchNorm folded: scale = gamma/sqrt(var+eps), shift = beta - mean*scale); relu != 0 clamps at 0;
+ *   out [B,O,D,H,W].  Needs W % 4 == 0, 3*H*W < 2^31, B*ceil(D/8) <= 65535, 16-byte aligned in / out.
+ * BatchNorm backward to the convolution output (with the helpers of the fused stem, which are generic over [B,O,D,H,W]):
+ *   rag_cv_stem_bn_bwd_sums(g, z, bn) + rag_cv_stem_bwd_consts -> consts [O,7] = (a, m1, m2, scale, shift, mean, rstd), then
+ *   rag_conv3d_cc_bn_bwd_gz: gz = a (g' - m1 - zh m2), g' = g [fma(z, scale, shift) > 0] (the forward's own ReLU decision, bit
+ *   for bit), zh = (z - mean) rstd; m1 = m2 = 0 in eval mode.  g, z, gz [B,O,D,H,W], W % 4 == 0, 16-byte aligned.
+ * rag_conv3d_cc_bwd, from gz:
+ *   gin [B,C,D,H,W] (nullable; needs w):            gin[b,c,p] = sum_{o,k} w[o,c,k] gz[b,o,p-k+1]
+ *   gw  [O,C,3,3,3] (nullable; needs in, workspace): gw[o,c,k]  = sum_{b,p} gz[b,o,p] in[b,c,p+k-1]
+ *   workspace: rag_conv3d_cc_bwd_workspace_bytes(B,C,O,D,H,W) bytes (0 = unsupported pair), caller-owned.  Bitwise
+ *   repeatable: fixed-order per-CTA partials, fp64 final pass, no atomics.  Same shape limits as the forward. */
+RAG_API int rag_conv3d_cc_fwd(const float* in, const float* w, const float* scale, const float* shift, int relu, float* out,
+                      int B, int C, int O, int D, int H, int W, void* stream);
+RAG_API int rag_conv3d_cc_bn_bwd_gz(const float* g, const float* z, const float* consts, float* gz, int B, int O, int D, int H, int W, void* stream);
+RAG_API size_t rag_conv3d_cc_bwd_workspace_bytes(int B, int C, int O, int D, int H, int W);
+RAG_API int rag_conv3d_cc_bwd(const float* gz, const float* in, const float* w, float* gin, float* gw, void* workspace,
+                      int B, int C, int O, int D, int H, int W, void* stream);
 
 /* Trilinear resize of [B*C, Di,Hi,Wi] -> [B*C, Do,Ho,Wo] with PyTorch's fp32 index arithmetic: the `upsample_6` /
  * `upsample_12` steps of the Matching Net's tail, nn.Upsample(size=..., mode='trilinear', align_corners=True) at

@@ -12,7 +12,7 @@ import os
 
 from . import build as _build
 
-ABI_VERSION = 13
+ABI_VERSION = 14
 
 _f = C.POINTER(C.c_float)
 _d = C.POINTER(C.c_double)
@@ -55,6 +55,10 @@ SIGNATURES = {
     "rag_conv3d_c1_fwd": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "rag_conv3d_c1_bwd_workspace_bytes": (C.c_size_t, [_i]),
     "rag_conv3d_c1_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
+    "rag_conv3d_cc_fwd": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "rag_conv3d_cc_bn_bwd_gz": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
+    "rag_conv3d_cc_bwd_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i, _i]),
+    "rag_conv3d_cc_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_trilinear_resize_fwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_trilinear_resize_bwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_normalize_pad": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp]),

@@ -31,6 +31,10 @@ int cv_stem_bn_finalize(const double*, const float*, const float*, float*, float
 int cv_stem_bwd_consts(const double*, const float*, float*, float*, int, double, int, cudaStream_t);
 size_t cv_stem_bwd_workspace_bytes(int, int, int, int, int);
 int cv_stem_bwd(const float*, const float*, const float*, const float*, const float*, const float*, float*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
+int conv3d_cc_fwd(const float*, const float*, const float*, const float*, int, float*, int, int, int, int, int, int, cudaStream_t);
+int conv3d_cc_bn_bwd_gz(const float*, const float*, const float*, float*, int, int, int, int, int, cudaStream_t);
+size_t conv3d_cc_bwd_workspace_bytes(int, int, int, int, int, int);
+int conv3d_cc_bwd(const float*, const float*, const float*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
 }  // namespace rag
 
 using namespace rag;
@@ -141,6 +145,18 @@ RAG_API size_t rag_conv3d_c1_bwd_workspace_bytes(int C) { return conv3d_c1_bwd_w
 RAG_API int rag_conv3d_c1_bwd(const float* g, const float* in, const float* w, float* gin, float* gw, void* workspace,
                       int B, int C, int D, int H, int W, void* stream) {
     return conv3d_c1_bwd(g, in, w, gin, gw, static_cast<float*>(workspace), B, C, D, H, W, ST(stream));
+}
+RAG_API int rag_conv3d_cc_fwd(const float* in, const float* w, const float* scale, const float* shift, int relu, float* out,
+                      int B, int C, int O, int D, int H, int W, void* stream) {
+    return conv3d_cc_fwd(in, w, scale, shift, relu, out, B, C, O, D, H, W, ST(stream));
+}
+RAG_API int rag_conv3d_cc_bn_bwd_gz(const float* g, const float* z, const float* consts, float* gz, int B, int O, int D, int H, int W, void* stream) {
+    return conv3d_cc_bn_bwd_gz(g, z, consts, gz, B, O, D, H, W, ST(stream));
+}
+RAG_API size_t rag_conv3d_cc_bwd_workspace_bytes(int B, int C, int O, int D, int H, int W) { return conv3d_cc_bwd_workspace_bytes(B, C, O, D, H, W); }
+RAG_API int rag_conv3d_cc_bwd(const float* gz, const float* in, const float* w, float* gin, float* gw, void* workspace,
+                      int B, int C, int O, int D, int H, int W, void* stream) {
+    return conv3d_cc_bwd(gz, in, w, gin, gw, static_cast<float*>(workspace), B, C, O, D, H, W, ST(stream));
 }
 RAG_API int rag_trilinear_resize_fwd(const float* in, float* out, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int align_corners, void* stream) {
     return trilinear_resize_fwd(in, out, BC, Di, Hi, Wi, Do, Ho, Wo, align_corners, ST(stream));

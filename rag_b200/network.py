@@ -78,7 +78,8 @@ def basic_network_forward(self, left, right, fea_ops, mat_ops):
     return _head(self, cost)
 
 
-def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_stem: bool = False, upsample: bool = False) -> dict:
+def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_stem: bool = False, upsample: bool = False,
+            matching_convs: bool = False) -> dict:
     """Bind the B200 hot path onto the reference's modules (pass the imported module objects
     ``models.rag_model`` and/or ``automl.mdenas_basicmodel``).  Returns what was patched.
     New networks constructed afterwards get ``rag_b200.Disp``; existing instances keep working
@@ -95,7 +96,14 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
 
     ``upsample=True`` (needs ``rag_model``) sends the ``upsample_6`` / ``upsample_12`` steps of ``matching()`` /
     ``search_matching()`` (``nn.Upsample(..., mode='trilinear', align_corners=True)``, rag_model.py:356-357,675-676) through
-    csrc/trilinear.cu, forward and deterministic backward (rag_b200/upsample.py)."""
+    csrc/trilinear.cu, forward and deterministic backward (rag_b200/upsample.py).
+
+    ``matching_convs=True`` (needs ``operations_3d``) binds ``ConvBR_3d.forward`` to ``rag_b200.matching_conv.matching_forward``:
+    the Matching Net's interior 3x3x3 ConvBR_3d layers with (C, O) in ``matching_conv.PAIRS`` (``stem3d1``, the cells'
+    ``conv_3x3`` ops -- also those of the search supernet) run on csrc/conv3d_cc.cu in inference and training (folded
+    BatchNorm + ReLU in eval(); batch statistics, running-estimate updates and the backward otherwise).  Every call that does
+    not qualify (``matching_conv.qualifies``) goes to the ``fuse_stem`` binding unchanged, so the fused stem, ``last_3_3d``
+    and the cuDNN fallback behave as without the flag."""
     global _FUSE_STEM, _STEM_AWARE
     done = {}
 
@@ -107,6 +115,14 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
         if operations_3d is None:
             raise ValueError("fuse_stem=True needs operations_3d (the reference's automl.operations_3d module)")
         bind(operations_3d.ConvBR_3d, "forward", stem_forward)
+        _STEM_AWARE = True
+        done["operations_3d"] = ["ConvBR_3d.forward"]
+    if matching_convs:
+        if operations_3d is None:
+            raise ValueError("matching_convs=True needs operations_3d (the reference's automl.operations_3d module)")
+        from .matching_conv import matching_forward
+
+        bind(operations_3d.ConvBR_3d, "forward", matching_forward)   # delegates to stem_forward: fusion-aware as well
         _STEM_AWARE = True
         done["operations_3d"] = ["ConvBR_3d.forward"]
     _FUSE_STEM = bool(fuse_stem)          # always (re)set: install(fuse_stem=False) after a fused install turns it off

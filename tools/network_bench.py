@@ -3,10 +3,11 @@ how much of a full forward / training step the hot path (and the rows next to it
 
     python tools/network_bench.py [--size 288x576] [--batch 4]
 
-Three configurations, same weights and inputs: (a) the unmodified reference (PyTorch eager + cuDNN, TF32 on as by default),
+Four configurations, same weights and inputs: (a) the unmodified reference (PyTorch eager + cuDNN, TF32 on as by default),
 (b) install() -- cost volume + disparity head through the hand-written kernels, (c) install(fuse_stem=True, upsample=True) --
 additionally the first Matching-Net layer fused with the volume (never materialised, forward and backward) and the tail
-(upsample_12/6, last_3_3d).  Forward = eval() under no_grad (approaches/rag.py:408-441); training step = train() forward +
+(upsample_12/6, last_3_3d), (d) as (c) plus matching_convs=True -- the interior 3x3x3 ConvBR_3d layers on csrc/conv3d_cc.cu.
+Forward = eval() under no_grad (approaches/rag.py:408-441); training step = train() forward +
 masked smooth-L1 + backward (approaches/rag.py:205-216, optimizer step excluded).  Prints one JSON line per configuration."""
 import argparse
 import json
@@ -60,7 +61,9 @@ def main():
 
     rows = []
     for name, kw in (("reference (unpatched)", None), ("install()", {}),
-                     ("install(fuse_stem=True, upsample=True)", dict(operations_3d=ref.operations_3d, fuse_stem=True, upsample=True))):
+                     ("install(fuse_stem=True, upsample=True)", dict(operations_3d=ref.operations_3d, fuse_stem=True, upsample=True)),
+                     ("install(fuse_stem=True, upsample=True, matching_convs=True)",
+                      dict(operations_3d=ref.operations_3d, fuse_stem=True, upsample=True, matching_convs=True))):
         N.uninstall()
         if kw is not None:
             N.install(ref.rag_model, ref.mdenas_basicmodel, **kw)
