@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define RAG_B200_ABI_VERSION 14
+#define RAG_B200_ABI_VERSION 15
 
 #if defined(__GNUC__)
 #define RAG_API __attribute__((visibility("default")))
@@ -195,42 +195,42 @@ RAG_API int rag_cv_stem_fwd_v(const float* x, const float* y, const float* w, co
 RAG_API int rag_cv_stem_moments(const float* x, const float* y, const float* w, double* moments,
                         int B, int C, int O, int Df, int Hf, int Wf, void* workspace, void* stream);
 
+/* ---- training-mode BatchNorm3d + ReLU -----------------------------------------------------------------------------------
+ * The BatchNorm half of ConvBR_3d (src/automl/operations_3d.py:31-47) in the training paths of the fused stem and of the
+ * interior layers, on the convolution output z [B,O,D,H,W], for BatchNorm in train() (batch statistics) or eval() (running
+ * statistics).  n = B*D*H*W; bn [O,4] = (scale, shift, mean, rstd) fp32, scale = gamma*rstd, shift = beta - mean*scale.
+ * Forward:
+ *   rag_bn3d_moments: sums [O,2] DOUBLE = (sum z, sum z^2);
+ *   rag_bn3d_finalize: bn from sums (batch != 0: mean, biased variance) or from the running statistics (batch == 0; sums may
+ *     be NULL); with batch and update != 0 the running estimates move in place as nn.BatchNorm's do in train()
+ *     (r = (1-momentum) r + momentum * batch value, unbiased variance n/(n-1));
+ *   rag_bn3d_relu: z <- max(fma(z, scale[o], shift[o]), 0) IN PLACE = the layer output.
+ * Backward, with g [B,O,D,H,W] the upstream gradient of the layer output, g' = g [fma(z, scale, shift) > 0] (the forward's own
+ * ReLU decision, bit for bit) and zh = (z - mean)*rstd:
+ *   rag_bn3d_bwd_sums: sums [O,2] DOUBLE = (sum g', sum g'*zh);
+ *   rag_bn3d_bwd_consts: consts [O,7] = (a, m1, m2, scale, shift, mean, rstd) with a = gamma*rstd and, when batch != 0,
+ *     m1 = sums[o,0]/n, m2 = sums[o,1]/n, else m1 = m2 = 0; gparam [2,O] = (d/d gamma, d/d beta);
+ *   rag_bn3d_bwd_gz: gz [B,O,D,H,W] = a (g' - m1 - zh m2), the gradient at the convolution output.
+ * rows_ws: caller-owned DOUBLE workspace [B*H*O*2].  The entry points that take a [B,O,D,H,W] tensor need O <= 32, D >= 3,
+ * 8 <= W <= 1016, W % 4 == 0, B <= 32767, H <= 65535 and 16-byte aligned z / g / gz.  Deterministic (fixed-order reductions,
+ * no atomics). */
+RAG_API int rag_bn3d_moments(const float* z, double* sums, double* rows_ws, int B, int O, int D, int H, int W, void* stream);
+RAG_API int rag_bn3d_finalize(const double* sums, const float* gamma, const float* beta, float* running_mean, float* running_var,
+                      float* bn, int O, double n, double eps, double momentum, int batch, int update, void* stream);
+RAG_API int rag_bn3d_relu(float* z, const float* bn, int B, int O, int D, int H, int W, void* stream);
+RAG_API int rag_bn3d_bwd_sums(const float* g, const float* z, const float* bn, double* sums, double* rows_ws,
+                      int B, int O, int D, int H, int W, void* stream);
+RAG_API int rag_bn3d_bwd_consts(const double* sums, const float* bn, float* consts, float* gparam, int O, double n, int batch, void* stream);
+RAG_API int rag_bn3d_bwd_gz(const float* g, const float* z, const float* consts, float* gz, int B, int O, int D, int H, int W, void* stream);
+
 /* The fused layer with autograd (training; DESIGN.md section 5.7) -- again without the volume, its gradient, or any other
- * [B,2C,Df,Hf,Wf] tensor.  Replaces src/models/rag_model.py:375-383 + ConvBR_3d (operations_3d.py:31-47: Conv3d ->
- * BatchNorm3d -> ReLU) and their autograd, for BatchNorm in train() (batch statistics) or eval() (running statistics).
- * Forward:  z = rag_cv_stem_fwd(x, y, w, scale = NULL, shift = NULL, relu = 0)            the convolution output
- *           rag_cv_stem_z_moments(z) -> sums [O,2] DOUBLE = (sum z, sum z^2) over (B,Df,Hf,Wf)   (train(): mean, biased variance)
- *           rag_cv_stem_bn_relu(z, scale, shift): z <- max(fma(z, scale[o], shift[o]), 0) IN PLACE = the layer output,
- *           scale = gamma*rstd, shift = beta - mean*scale.
- * Backward: z is RECOMPUTED with rag_cv_stem_fwd (the host side does not keep it alive), then, with g [B,O,Df,Hf,Wf] the
- *   upstream gradient of the layer output and bn [O,4] = (scale, shift, mean, rstd):
- *   rag_cv_stem_bn_bwd_sums -> sums [O,2] DOUBLE = (sum g', sum g'*zh), g' = g [fma(z,scale,shift) > 0] (the forward's own ReLU
- *     decision, bit for bit), zh = (z - mean)*rstd: the BatchNorm bias / weight gradients and the two means of the train-mode
- *     BatchNorm backward;
- *   rag_cv_stem_bwd, consts [O,7] = (a, m1, m2, scale, shift, mean, rstd) with a = gamma*rstd and, in train mode,
- *     m1 = sums[o,0]/n, m2 = sums[o,1]/n (n = B*Df*Hf*Wf), in eval mode m1 = m2 = 0: the gradient at the convolution output
- *     gz = a (g' - m1 - zh m2) is formed on the fly and reduced along d into the 2-D maps the transpose needs, then
- *     gx, gy [B,C,Hf,Wf] (both or neither; need w) and gw [O,2C,3,3,3] (nullable; needs x, y) are 2-D contractions.
- * rows_ws: DOUBLE workspace [B*Hf*O*2]; workspace: rag_cv_stem_bwd_workspace_bytes(B,C,O,Hf,Wf) bytes, 16-byte aligned;
- * both caller-owned.  Deterministic (fixed-order reductions, no atomics).
- * Needs C == 12, O <= 32, Df >= 3, 8 <= Wf <= 1016, Wf % 4 == 0. */
-RAG_API int rag_cv_stem_z_moments(const float* z, double* sums, double* rows_ws, int B, int O, int Df, int Hf, int Wf, void* stream);
-/* Per-channel finalisers (one tiny launch each instead of a dozen elementwise framework kernels):
- * rag_cv_stem_bn_finalize: sums [O,2] DOUBLE (from rag_cv_stem_z_moments; used when batch != 0) or the running statistics
- *   (batch == 0) -> bn [O,4] = (scale, shift, mean, rstd) fp32 and stats [O,2] DOUBLE = (mean, biased variance); with batch and
- *   update != 0 the running estimates are updated in place as nn.BatchNorm does in train() (r = (1-momentum) r + momentum * batch
- *   value, unbiased variance n/(n-1)); n = B*Df*Hf*Wf.  scale / shift for rag_cv_stem_bn_relu are columns 0 / 1 of bn (stride 4:
- *   pass bn and bn + 1 is NOT valid -- use rag_cv_stem_bn_relu_bn below).
- * rag_cv_stem_bwd_consts: sums [O,2] DOUBLE (from rag_cv_stem_bn_bwd_sums) + bn -> consts [O,7] for rag_cv_stem_bwd and
- *   gparam [2,O] = (d/d gamma, d/d beta). */
-RAG_API int rag_cv_stem_bn_finalize(const double* sums, const float* gamma, const float* beta, float* running_mean, float* running_var,
-                            double* stats, float* bn, int O, double n, double eps, double momentum, int batch, int update, void* stream);
-RAG_API int rag_cv_stem_bwd_consts(const double* sums, const float* bn, float* consts, float* gparam, int O, double n, int batch, void* stream);
-RAG_API int rag_cv_stem_bn_relu(float* z, const float* scale, const float* shift, int B, int O, int Df, int Hf, int Wf, void* stream);
-/* the same with scale / shift taken from columns 0 / 1 of bn [O,4] */
-RAG_API int rag_cv_stem_bn_relu_bn(float* z, const float* bn, int B, int O, int Df, int Hf, int Wf, void* stream);
-RAG_API int rag_cv_stem_bn_bwd_sums(const float* g, const float* z, const float* bn, double* sums,
-                            double* rows_ws, int B, int O, int Df, int Hf, int Wf, void* stream);
+ * [B,2C,Df,Hf,Wf] tensor.  Replaces src/models/rag_model.py:375-383 + ConvBR_3d and their autograd.
+ * Forward:  z = rag_cv_stem_fwd(x, y, w, NULL, NULL, 0, ...), then the BatchNorm3d forward above: z becomes the layer output.
+ * Backward: z is RECOMPUTED with rag_cv_stem_fwd; rag_bn3d_bwd_sums + rag_bn3d_bwd_consts give consts [O,7]; rag_cv_stem_bwd
+ *   forms gz on the fly and reduces it along d into 2-D maps, then gx, gy [B,C,Hf,Wf] (both or neither; need w) and
+ *   gw [O,2C,3,3,3] (nullable; needs x, y) are 2-D contractions.
+ * workspace: rag_cv_stem_bwd_workspace_bytes(B,C,O,Hf,Wf) bytes, 16-byte aligned, caller-owned.  Deterministic (fixed-order
+ * reductions, no atomics).  Needs C == 12, O <= 32, Df >= 3, 8 <= Wf <= 1016, Wf % 4 == 0. */
 RAG_API size_t rag_cv_stem_bwd_workspace_bytes(int B, int C, int O, int Hf, int Wf);
 RAG_API int rag_cv_stem_bwd(const float* g, const float* z, const float* consts, const float* x, const float* y, const float* w,
                     float* gx, float* gy, float* gw, void* workspace, int B, int C, int O, int Df, int Hf, int Wf, void* stream);
@@ -260,10 +260,8 @@ RAG_API int rag_conv3d_c1_bwd(const float* g, const float* in, const float* w, f
  *   in [B,C,D,H,W]; w [O,C,3,3,3] (Conv3d.weight); scale / shift [O] (both NULL = identity: raw z, the training path;
  *   eval-mode BatchNorm folded: scale = gamma/sqrt(var+eps), shift = beta - mean*scale); relu != 0 clamps at 0;
  *   out [B,O,D,H,W].  Needs W % 4 == 0, 3*H*W < 2^31, B*ceil(D/8) <= 65535, 16-byte aligned in / out.
- * BatchNorm backward to the convolution output (with the helpers of the fused stem, which are generic over [B,O,D,H,W]):
- *   rag_cv_stem_bn_bwd_sums(g, z, bn) + rag_cv_stem_bwd_consts -> consts [O,7] = (a, m1, m2, scale, shift, mean, rstd), then
- *   rag_conv3d_cc_bn_bwd_gz: gz = a (g' - m1 - zh m2), g' = g [fma(z, scale, shift) > 0] (the forward's own ReLU decision, bit
- *   for bit), zh = (z - mean) rstd; m1 = m2 = 0 in eval mode.  g, z, gz [B,O,D,H,W], W % 4 == 0, 16-byte aligned.
+ * Training: z = the raw forward output (scale = shift = NULL, relu = 0) goes through the BatchNorm3d section above, whose
+ * rag_bn3d_bwd_gz gives the gradient gz at the convolution output.
  * rag_conv3d_cc_bwd, from gz:
  *   gin [B,C,D,H,W] (nullable; needs w):            gin[b,c,p] = sum_{o,k} w[o,c,k] gz[b,o,p-k+1]
  *   gw  [O,C,3,3,3] (nullable; needs in, workspace): gw[o,c,k]  = sum_{b,p} gz[b,o,p] in[b,c,p+k-1]
@@ -271,7 +269,6 @@ RAG_API int rag_conv3d_c1_bwd(const float* g, const float* in, const float* w, f
  *   repeatable: fixed-order per-CTA partials, fp64 final pass, no atomics.  Same shape limits as the forward. */
 RAG_API int rag_conv3d_cc_fwd(const float* in, const float* w, const float* scale, const float* shift, int relu, float* out,
                       int B, int C, int O, int D, int H, int W, void* stream);
-RAG_API int rag_conv3d_cc_bn_bwd_gz(const float* g, const float* z, const float* consts, float* gz, int B, int O, int D, int H, int W, void* stream);
 RAG_API size_t rag_conv3d_cc_bwd_workspace_bytes(int B, int C, int O, int D, int H, int W);
 RAG_API int rag_conv3d_cc_bwd(const float* gz, const float* in, const float* w, float* gin, float* gw, void* workspace,
                       int B, int C, int O, int D, int H, int W, void* stream);

@@ -12,7 +12,7 @@ import os
 
 from . import build as _build
 
-ABI_VERSION = 14
+ABI_VERSION = 15
 
 _f = C.POINTER(C.c_float)
 _d = C.POINTER(C.c_double)
@@ -44,19 +44,18 @@ SIGNATURES = {
     "rag_cv_stem_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "rag_cv_stem_fwd_v": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp, _i, _vp]),
     "rag_cv_stem_moments": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
-    "rag_cv_stem_z_moments": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
-    "rag_cv_stem_bn_relu": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
-    "rag_cv_stem_bn_relu_bn": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp]),
-    "rag_cv_stem_bn_finalize": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, C.c_double, C.c_double, C.c_double, _i, _i, _vp]),
-    "rag_cv_stem_bwd_consts": (_i, [_vp, _vp, _vp, _vp, _i, C.c_double, _i, _vp]),
-    "rag_cv_stem_bn_bwd_sums": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
+    "rag_bn3d_moments": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
+    "rag_bn3d_finalize": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, C.c_double, C.c_double, C.c_double, _i, _i, _vp]),
+    "rag_bn3d_relu": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp]),
+    "rag_bn3d_bwd_sums": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
+    "rag_bn3d_bwd_consts": (_i, [_vp, _vp, _vp, _vp, _i, C.c_double, _i, _vp]),
+    "rag_bn3d_bwd_gz": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "rag_cv_stem_bwd_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i]),
     "rag_cv_stem_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_conv3d_c1_fwd": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "rag_conv3d_c1_bwd_workspace_bytes": (C.c_size_t, [_i]),
     "rag_conv3d_c1_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "rag_conv3d_cc_fwd": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp]),
-    "rag_conv3d_cc_bn_bwd_gz": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "rag_conv3d_cc_bwd_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i, _i]),
     "rag_conv3d_cc_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_trilinear_resize_fwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),

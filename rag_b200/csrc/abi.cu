@@ -24,15 +24,15 @@ int conv3d_c1_bwd(const float*, const float*, const float*, float*, float*, floa
 size_t conv3d_c1_bwd_workspace_bytes(int);
 int trilinear_resize_fwd(const float*, float*, int, int, int, int, int, int, int, int, cudaStream_t);
 int trilinear_resize_bwd(const float*, float*, int, int, int, int, int, int, int, int, cudaStream_t);
-int cv_stem_bn_bwd_sums(const float*, const float*, const float*, double*, double*, int, int, int, int, int, cudaStream_t);
-int cv_stem_z_moments(const float*, double*, double*, int, int, int, int, int, cudaStream_t);
-int cv_stem_bn_relu(float*, const float*, const float*, int, int, int, int, int, int, cudaStream_t);
-int cv_stem_bn_finalize(const double*, const float*, const float*, float*, float*, double*, float*, int, double, double, double, int, int, cudaStream_t);
-int cv_stem_bwd_consts(const double*, const float*, float*, float*, int, double, int, cudaStream_t);
+int bn3d_moments(const float*, double*, double*, int, int, int, int, int, cudaStream_t);
+int bn3d_finalize(const double*, const float*, const float*, float*, float*, float*, int, double, double, double, int, int, cudaStream_t);
+int bn3d_relu(float*, const float*, int, int, int, int, int, cudaStream_t);
+int bn3d_bwd_sums(const float*, const float*, const float*, double*, double*, int, int, int, int, int, cudaStream_t);
+int bn3d_bwd_consts(const double*, const float*, float*, float*, int, double, int, cudaStream_t);
+int bn3d_bwd_gz(const float*, const float*, const float*, float*, int, int, int, int, int, cudaStream_t);
 size_t cv_stem_bwd_workspace_bytes(int, int, int, int, int);
 int cv_stem_bwd(const float*, const float*, const float*, const float*, const float*, const float*, float*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
 int conv3d_cc_fwd(const float*, const float*, const float*, const float*, int, float*, int, int, int, int, int, int, cudaStream_t);
-int conv3d_cc_bn_bwd_gz(const float*, const float*, const float*, float*, int, int, int, int, int, cudaStream_t);
 size_t conv3d_cc_bwd_workspace_bytes(int, int, int, int, int, int);
 int conv3d_cc_bwd(const float*, const float*, const float*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
 }  // namespace rag
@@ -113,26 +113,6 @@ RAG_API int rag_cv_stem_fwd_v(const float* x, const float* y, const float* w, co
                       int relu, float* out, int B, int C, int O, int Df, int Hf, int Wf, void* workspace, int variant, void* stream) {
     return cv_stem_fwd(x, y, w, scale, shift, relu, out, B, C, O, Df, Hf, Wf, static_cast<float*>(workspace), variant, ST(stream));
 }
-RAG_API int rag_cv_stem_z_moments(const float* z, double* sums, double* rows_ws, int B, int O, int Df, int Hf, int Wf, void* stream) {
-    return cv_stem_z_moments(z, sums, rows_ws, B, O, Df, Hf, Wf, ST(stream));
-}
-RAG_API int rag_cv_stem_bn_relu(float* z, const float* scale, const float* shift, int B, int O, int Df, int Hf, int Wf, void* stream) {
-    return cv_stem_bn_relu(z, scale, shift, 1, B, O, Df, Hf, Wf, ST(stream));
-}
-RAG_API int rag_cv_stem_bn_relu_bn(float* z, const float* bn, int B, int O, int Df, int Hf, int Wf, void* stream) {
-    return cv_stem_bn_relu(z, bn, bn ? bn + 1 : nullptr, 4, B, O, Df, Hf, Wf, ST(stream));
-}
-RAG_API int rag_cv_stem_bn_finalize(const double* sums, const float* gamma, const float* beta, float* running_mean, float* running_var,
-                            double* stats, float* bn, int O, double n, double eps, double momentum, int batch, int update, void* stream) {
-    return cv_stem_bn_finalize(sums, gamma, beta, running_mean, running_var, stats, bn, O, n, eps, momentum, batch, update, ST(stream));
-}
-RAG_API int rag_cv_stem_bwd_consts(const double* sums, const float* bn, float* consts, float* gparam, int O, double n, int batch, void* stream) {
-    return cv_stem_bwd_consts(sums, bn, consts, gparam, O, n, batch, ST(stream));
-}
-RAG_API int rag_cv_stem_bn_bwd_sums(const float* g, const float* z, const float* bn, double* sums,
-                            double* rows_ws, int B, int O, int Df, int Hf, int Wf, void* stream) {
-    return cv_stem_bn_bwd_sums(g, z, bn, sums, rows_ws, B, O, Df, Hf, Wf, ST(stream));
-}
 RAG_API size_t rag_cv_stem_bwd_workspace_bytes(int B, int C, int O, int Hf, int Wf) { return cv_stem_bwd_workspace_bytes(B, C, O, Hf, Wf); }
 RAG_API int rag_cv_stem_bwd(const float* g, const float* pre, const float* consts, const float* x, const float* y, const float* w,
                     float* gx, float* gy, float* gw, void* workspace, int B, int C, int O, int Df, int Hf, int Wf, void* stream) {
@@ -150,13 +130,30 @@ RAG_API int rag_conv3d_cc_fwd(const float* in, const float* w, const float* scal
                       int B, int C, int O, int D, int H, int W, void* stream) {
     return conv3d_cc_fwd(in, w, scale, shift, relu, out, B, C, O, D, H, W, ST(stream));
 }
-RAG_API int rag_conv3d_cc_bn_bwd_gz(const float* g, const float* z, const float* consts, float* gz, int B, int O, int D, int H, int W, void* stream) {
-    return conv3d_cc_bn_bwd_gz(g, z, consts, gz, B, O, D, H, W, ST(stream));
-}
 RAG_API size_t rag_conv3d_cc_bwd_workspace_bytes(int B, int C, int O, int D, int H, int W) { return conv3d_cc_bwd_workspace_bytes(B, C, O, D, H, W); }
 RAG_API int rag_conv3d_cc_bwd(const float* gz, const float* in, const float* w, float* gin, float* gw, void* workspace,
                       int B, int C, int O, int D, int H, int W, void* stream) {
     return conv3d_cc_bwd(gz, in, w, gin, gw, static_cast<float*>(workspace), B, C, O, D, H, W, ST(stream));
+}
+RAG_API int rag_bn3d_moments(const float* z, double* sums, double* rows_ws, int B, int O, int D, int H, int W, void* stream) {
+    return bn3d_moments(z, sums, rows_ws, B, O, D, H, W, ST(stream));
+}
+RAG_API int rag_bn3d_finalize(const double* sums, const float* gamma, const float* beta, float* running_mean, float* running_var,
+                      float* bn, int O, double n, double eps, double momentum, int batch, int update, void* stream) {
+    return bn3d_finalize(sums, gamma, beta, running_mean, running_var, bn, O, n, eps, momentum, batch, update, ST(stream));
+}
+RAG_API int rag_bn3d_relu(float* z, const float* bn, int B, int O, int D, int H, int W, void* stream) {
+    return bn3d_relu(z, bn, B, O, D, H, W, ST(stream));
+}
+RAG_API int rag_bn3d_bwd_sums(const float* g, const float* z, const float* bn, double* sums, double* rows_ws,
+                      int B, int O, int D, int H, int W, void* stream) {
+    return bn3d_bwd_sums(g, z, bn, sums, rows_ws, B, O, D, H, W, ST(stream));
+}
+RAG_API int rag_bn3d_bwd_consts(const double* sums, const float* bn, float* consts, float* gparam, int O, double n, int batch, void* stream) {
+    return bn3d_bwd_consts(sums, bn, consts, gparam, O, n, batch, ST(stream));
+}
+RAG_API int rag_bn3d_bwd_gz(const float* g, const float* z, const float* consts, float* gz, int B, int O, int D, int H, int W, void* stream) {
+    return bn3d_bwd_gz(g, z, consts, gz, B, O, D, H, W, ST(stream));
 }
 RAG_API int rag_trilinear_resize_fwd(const float* in, float* out, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int align_corners, void* stream) {
     return trilinear_resize_fwd(in, out, BC, Di, Hi, Wi, Do, Ho, Wo, align_corners, ST(stream));

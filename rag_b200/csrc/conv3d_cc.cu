@@ -166,26 +166,6 @@ conv3d_cc_fwd_kernel(const float* __restrict__ in, const float* __restrict__ w, 
     }
 }
 
-// gz = a (g' - m1 - zh m2), g' = g [fma(z, scale, shift) > 0] (the forward's own ReLU decision, bit for bit), zh = (z - mean) rstd;
-// consts [O][7] = (a, m1, m2, scale, shift, mean, rstd) from rag_cv_stem_bwd_consts.  Grid-stride over float4.
-__global__ void __launch_bounds__(256)
-conv3d_cc_bn_gz_kernel(const float* __restrict__ g, const float* __restrict__ z, const float* __restrict__ consts, float* __restrict__ gz,
-                       size_t n4, size_t chan4, int O) {
-    for (size_t i = (size_t)blockIdx.x * 256 + threadIdx.x; i < n4; i += (size_t)gridDim.x * 256) {
-        const int o = (int)((i / chan4) % O);
-        const float* cs = consts + 7 * o;
-        const float a = __ldg(cs), m1 = __ldg(cs + 1), m2 = __ldg(cs + 2), sc = __ldg(cs + 3), sh = __ldg(cs + 4), mu = __ldg(cs + 5), rs = __ldg(cs + 6);
-        const float4 zv = ld_stream(reinterpret_cast<const float4*>(z) + i);
-        const float4 gv = ld_stream(reinterpret_cast<const float4*>(g) + i);
-        float4 r;
-        r.x = a * ((__fmaf_rn(zv.x, sc, sh) > 0.f ? gv.x : 0.f) - m1 - ((zv.x - mu) * rs) * m2);
-        r.y = a * ((__fmaf_rn(zv.y, sc, sh) > 0.f ? gv.y : 0.f) - m1 - ((zv.y - mu) * rs) * m2);
-        r.z = a * ((__fmaf_rn(zv.z, sc, sh) > 0.f ? gv.z : 0.f) - m1 - ((zv.z - mu) * rs) * m2);
-        r.w = a * ((__fmaf_rn(zv.w, sc, sh) > 0.f ? gv.w : 0.f) - m1 - ((zv.w - mu) * rs) * m2);
-        reinterpret_cast<float4*>(gz)[i] = r;
-    }
-}
-
 // Weight-gradient partials: part [G][CO][CI][27].  grid G (<= kCcWgGroups), cc_wg_threads(CI) threads.
 // smem: 2 slots of cc_wg_slot(CI, CO) floats = x [3 planes][CI][4 rows][76] | gz [CO][2 rows][64].
 template <int CI, int CO>
@@ -359,16 +339,6 @@ int conv3d_cc_fwd(const float* in, const float* w, const float* scale, const flo
         case 8: return cc_launch_fwd<8, 8, false>(in, w, scale, shift, relu, out, B, D, H, W, st);
         default: return cc_launch_fwd<12, 12, false>(in, w, scale, shift, relu, out, B, D, H, W, st);
     }
-}
-
-int conv3d_cc_bn_bwd_gz(const float* g, const float* z, const float* consts, float* gz, int B, int O, int D, int H, int W, cudaStream_t st) {
-    if (!g || !z || !consts || !gz) return fail(RAG_E_NULL, "conv3d_cc_bn_bwd_gz: null pointer");
-    if (B <= 0 || O <= 0 || D <= 0 || H <= 0 || W <= 0 || W % 4 != 0) return fail(RAG_E_SHAPE, "conv3d_cc_bn_bwd_gz: needs positive dimensions and W %% 4 == 0");
-    if (!aligned(g, 16) || !aligned(z, 16) || !aligned(gz, 16) || !aligned(consts, 4)) return fail(RAG_E_ALIGN, "conv3d_cc_bn_bwd_gz: g/z/gz must be 16-byte aligned");
-    const size_t chan4 = (size_t)D * H * W / 4, n4 = chan4 * O * B;
-    const unsigned grid = (unsigned)std::min<size_t>((n4 + 255) / 256, (size_t)num_sms() * 16);
-    conv3d_cc_bn_gz_kernel<<<grid, 256, 0, st>>>(g, z, consts, gz, n4, chan4, O);
-    return check_launch("conv3d_cc_bn_bwd_gz");
 }
 
 size_t conv3d_cc_bwd_workspace_bytes(int B, int C, int O, int D, int H, int W) {

@@ -15,18 +15,12 @@
 //     gW[o,  c,kd,kh,kw] = sum_{b,h,w'} x[c,h',w'] Tw[kd,kw][o,h,w'-kw+1]
 //     gW[o,C+c,kd,kh,kw] = sum_{b,h,u } y[c,h',u ] S[kd,kw==2][o,h,u+kd-kw]
 // (the fp64 prototype of this algebra is checked against the reference's autograd through the materialised volume in the
-// CPU test-suite: stem_backward_volume_free_f64, tests/test_oracle_golden.py).  gz itself is never stored either: it is rebuilt on the fly from
-// the upstream gradient g of the layer OUTPUT and the convolution output z (before BatchNorm):
-//     pre = fma(z, scale, shift),  g' = g [pre > 0],  zh = (z - mean) * rstd          (scale = gamma*rstd, shift = beta - mean*scale)
-//     gz = a (g' - m1 - zh m2),  a = gamma*rstd,  m1 = mean(g'), m2 = mean(g' zh)   (train)   |   gz = a g'   (eval)
-// In train mode the -a (m1 + zh m2) term reaches every element, also where the ReLU is off, so the saved OUTPUT is not
-// enough; instead of keeping a second [B,O,Df,Hf,Wf] tensor alive between forward and backward the host side RECOMPUTES z
-// with the forward kernel into a temporary that dies with the backward call.  The forward of the autograd path is the same
-// z kernel followed by stem_bn_relu_kernel (in place), which thresholds the SAME expression fma(z, scale, shift): forward
-// and backward agree on the ReLU decision bit for bit.
-// Forward passes over [B,O,Df,Hf,Wf]: z written once, read once for the batch moments (stem_z_rows_kernel, fp64), normalised
-// in place.  Backward passes over g and z: ONE for the two BatchNorm sums (bnb_rows), ONE for the maps (bwd_maps);
-// everything after that works on 2-D maps (15/Df of the tensor size).
+// CPU test-suite: stem_backward_volume_free_f64, tests/test_oracle_golden.py).  gz itself is never stored either: the maps
+// kernel rebuilds it on the fly from the upstream gradient g of the layer OUTPUT and the convolution output z, with the
+// BatchNorm constants and the ReLU decision of bn3d.cu.  The BatchNorm backward needs z, not only the output, so instead of
+// keeping a second [B,O,Df,Hf,Wf] tensor alive the host side RECOMPUTES z with the forward kernel into a temporary.
+// Backward passes over g and z: ONE for the two BatchNorm sums (bn3d.cu), ONE for the maps (bwd_maps); everything after that
+// works on 2-D maps (15/Df of the tensor size).
 // CV-2's descending-d summation order does not apply here: the reference's own gz comes out of cuDNN, so the bar is
 // the 1e-5 max-norm of the other floating-point rows, not bit equality.
 #include <algorithm>
@@ -39,145 +33,7 @@ constexpr int kStC = 12;          // feature channels (the fused stem is special
 constexpr int kStWC = 128;        // column chunk of the contraction kernels
 constexpr int kStQ = 3 * kStC;    // (c, kh) pairs
 
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-    return v;
-}
-
-// ---- forward helpers: batch moments of z and the in-place BatchNorm + ReLU -------------------------------------------
-// rows[B,Hf,O,2] fp64 = per (b,o,h) row (sum z, sum z^2).  grid (Hf, O, B), 256 threads; Wf % 4 == 0.
-__global__ void __launch_bounds__(256)
-stem_z_rows_kernel(const float* __restrict__ z, double* __restrict__ rows, int O, int Df, int Hf, int Wf) {
-    const int h = blockIdx.x, o = blockIdx.y, b = blockIdx.z, tid = threadIdx.x;
-    const int Wv = Wf >> 2;
-    const size_t plane = (size_t)Hf * Wf;
-    const size_t base = ((size_t)(b * O + o) * Df) * plane + (size_t)h * Wf;
-    double s0 = 0.0, s1 = 0.0;
-    for (int i = tid; i < Df * Wv; i += 256) {
-        const int d = i / Wv, v = i - d * Wv;
-        const float4 zv = __ldg(reinterpret_cast<const float4*>(z + base + (size_t)d * plane + 4 * v));   // just written: L2
-        const float a = (zv.x + zv.y) + (zv.z + zv.w);
-        const float q = __fmaf_rn(zv.x, zv.x, zv.y * zv.y) + __fmaf_rn(zv.z, zv.z, zv.w * zv.w);
-        s0 += (double)a;
-        s1 += (double)q;
-    }
-    __shared__ double red[2][8];
-    s0 = warp_sum(s0); s1 = warp_sum(s1);
-    if ((tid & 31) == 0) { red[0][tid >> 5] = s0; red[1][tid >> 5] = s1; }
-    __syncthreads();
-    if (tid == 0) {
-        double a0 = 0.0, a1 = 0.0;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) { a0 += red[0][i]; a1 += red[1][i]; }
-        double* r = rows + ((size_t)(b * Hf + h) * O + o) * 2;
-        r[0] = a0; r[1] = a1;
-    }
-}
-
-// z <- max(fma(z, scale[o], shift[o]), 0) in place.  grid-stride over float4; n4 = B*O*Df*Hf*Wf / 4, chan4 = Df*Hf*Wf / 4
-__global__ void __launch_bounds__(256)
-stem_bn_relu_kernel(float* __restrict__ z, const float* __restrict__ scale, const float* __restrict__ shift, size_t n4, size_t chan4, int O, int stride) {
-    for (size_t i = (size_t)blockIdx.x * 256 + threadIdx.x; i < n4; i += (size_t)gridDim.x * 256) {
-        const int o = (int)((i / chan4) % O);
-        const float sc = __ldg(scale + o * stride), sh = __ldg(shift + o * stride);
-        float4 v = reinterpret_cast<float4*>(z)[i];
-        v.x = fmaxf(__fmaf_rn(v.x, sc, sh), 0.f); v.y = fmaxf(__fmaf_rn(v.y, sc, sh), 0.f);
-        v.z = fmaxf(__fmaf_rn(v.z, sc, sh), 0.f); v.w = fmaxf(__fmaf_rn(v.w, sc, sh), 0.f);
-        reinterpret_cast<float4*>(z)[i] = v;
-    }
-}
-
-// ---- per-channel finalisers: a handful of values per channel, one tiny launch instead of ~15 elementwise torch kernels ----
-// sums [O][2] fp64 = (sum z, sum z^2) when batch != 0, else unused.  bn [O][4] = (scale, shift, mean, rstd) fp32;
-// stats [O][2] fp64 = (mean, biased variance) the layer normalises with.  With batch and running != NULL the running
-// estimates are updated as nn.BatchNorm does in train(): r = (1-f) r + f * batch value, variance unbiased (n/(n-1)).
-__global__ void stem_bn_finalize_kernel(const double* __restrict__ sums, const float* __restrict__ gamma, const float* __restrict__ beta,
-                                        float* __restrict__ running_mean, float* __restrict__ running_var, double* __restrict__ stats,
-                                        float* __restrict__ bn, int O, double n, double eps, double f, int batch, int update) {
-    const int o = blockIdx.x * blockDim.x + threadIdx.x;
-    if (o >= O) return;
-    double mean, var;
-    if (batch) {
-        mean = sums[2 * o] / n;
-        var = fmax(sums[2 * o + 1] / n - mean * mean, 0.0);
-        if (update) {
-            running_mean[o] = (float)((1.0 - f) * (double)running_mean[o] + f * mean);
-            running_var[o] = (float)((1.0 - f) * (double)running_var[o] + f * var * (n / fmax(n - 1.0, 1.0)));
-        }
-    } else {
-        mean = (double)running_mean[o];
-        var = (double)running_var[o];
-    }
-    const float rstd = (float)(1.0 / sqrt(var + eps));
-    const float mu = (float)mean;
-    const float sc = gamma[o] * rstd;
-    stats[2 * o] = mean; stats[2 * o + 1] = var;
-    bn[4 * o] = sc; bn[4 * o + 1] = beta[o] - mu * sc; bn[4 * o + 2] = mu; bn[4 * o + 3] = rstd;
-}
-
-// sums [O][2] fp64 = (sum g', sum g' zh) -> consts [O][7] = (a, m1, m2, scale, shift, mean, rstd), gparam [2][O] = (ggamma, gbeta)
-__global__ void stem_bwd_consts_kernel(const double* __restrict__ sums, const float* __restrict__ bn, float* __restrict__ consts,
-                                       float* __restrict__ gparam, int O, double n, int batch) {
-    const int o = blockIdx.x * blockDim.x + threadIdx.x;
-    if (o >= O) return;
-    const double s0 = sums[2 * o], s1 = sums[2 * o + 1];
-    float* c = consts + 7 * o;
-    c[0] = bn[4 * o];                                       // a = gamma * rstd = scale
-    c[1] = batch ? (float)(s0 / n) : 0.f;
-    c[2] = batch ? (float)(s1 / n) : 0.f;
-    c[3] = bn[4 * o]; c[4] = bn[4 * o + 1]; c[5] = bn[4 * o + 2]; c[6] = bn[4 * o + 3];
-    gparam[o] = (float)s1;                                   // d/d gamma
-    gparam[O + o] = (float)s0;                               // d/d beta
-}
-
-// ---- pass A: per (b,o,h) row  (sum g', sum g'*zh)  ->  rows[B,Hf,O,2] fp64 ---------------------------------------
-// bn [O][4] = (scale, shift, mean, rstd).  grid (Hf, O, B), 256 threads; Wf % 4 == 0.
-__global__ void __launch_bounds__(256)
-stem_bnb_rows_kernel(const float* __restrict__ g, const float* __restrict__ z, const float* __restrict__ bn,
-                     double* __restrict__ rows, int O, int Df, int Hf, int Wf) {
-    const int h = blockIdx.x, o = blockIdx.y, b = blockIdx.z, tid = threadIdx.x;
-    const int Wv = Wf >> 2;
-    const size_t plane = (size_t)Hf * Wf;
-    const size_t base = ((size_t)(b * O + o) * Df) * plane + (size_t)h * Wf;
-    const float sc = __ldg(bn + 4 * o), sh = __ldg(bn + 4 * o + 1), mu = __ldg(bn + 4 * o + 2), rs = __ldg(bn + 4 * o + 3);
-    float s0 = 0.f, s1 = 0.f;
-    for (int i = tid; i < Df * Wv; i += 256) {
-        const int d = i / Wv, v = i - d * Wv;
-        const size_t idx = base + (size_t)d * plane + 4 * v;
-        const float4 zv = ld_stream(reinterpret_cast<const float4*>(z + idx));
-        const float4 gv = ld_stream(reinterpret_cast<const float4*>(g + idx));
-        const float g0 = __fmaf_rn(zv.x, sc, sh) > 0.f ? gv.x : 0.f, g1 = __fmaf_rn(zv.y, sc, sh) > 0.f ? gv.y : 0.f;
-        const float g2 = __fmaf_rn(zv.z, sc, sh) > 0.f ? gv.z : 0.f, g3 = __fmaf_rn(zv.w, sc, sh) > 0.f ? gv.w : 0.f;
-        s0 += (g0 + g1) + (g2 + g3);
-        s1 += (g0 * ((zv.x - mu) * rs) + g1 * ((zv.y - mu) * rs)) + (g2 * ((zv.z - mu) * rs) + g3 * ((zv.w - mu) * rs));
-    }
-    __shared__ double red[2][8];
-    double d0 = warp_sum((double)s0), d1 = warp_sum((double)s1);
-    if ((tid & 31) == 0) { red[0][tid >> 5] = d0; red[1][tid >> 5] = d1; }
-    __syncthreads();
-    if (tid == 0) {
-        double a0 = 0.0, a1 = 0.0;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) { a0 += red[0][i]; a1 += red[1][i]; }
-        double* r = rows + ((size_t)(b * Hf + h) * O + o) * 2;
-        r[0] = a0; r[1] = a1;
-    }
-}
-
-// rows[B*Hf][O][2] -> sums[O][2], fixed order (deterministic).  grid O, 32 threads.
-__global__ void stem_bnb_final_kernel(const double* __restrict__ rows, double* __restrict__ sums, int n_rows, int O) {
-    const int o = blockIdx.x, lane = threadIdx.x;
-    double a0 = 0.0, a1 = 0.0;
-    for (int i = lane; i < n_rows; i += 32) {
-        a0 += rows[((size_t)i * O + o) * 2];
-        a1 += rows[((size_t)i * O + o) * 2 + 1];
-    }
-    a0 = warp_sum(a0); a1 = warp_sum(a1);
-    if (lane == 0) { sums[2 * o] = a0; sums[2 * o + 1] = a1; }
-}
-
-// ---- pass B: the d-sums of gz ---------------------------------------------------------------------------------------
+// ---- the d-sums of gz -----------------------------------------------------------------------------------------------
 // grid (Hf, O, B); blockDim = roundup32(Wf + 4): thread t owns column w = t (t < Wf) and diagonal e = t - 2 (t < Wf + 2).
 // consts [O][7] = (a, m1, m2, scale, shift, mean, rstd).  tmap [B,O,Hf,9,Wf]; umap [B,O,Hf,6,Wf+4] (entry e+2; the last two are 0).
 // U = rows per batch (divides Df: no row predicates in the loop).  smem: 2 x U rows of gz for the column -> diagonal
@@ -514,58 +370,6 @@ static int check_stem_train(const char* who, int B, int C, int O, int Df, int Hf
                     who, B, C, O, Df, Hf, Wf);
     if ((size_t)B * O * Df * Hf * Wf >= ((size_t)1 << 40)) return fail(RAG_E_SHAPE, "%s: tensor too large", who);
     return RAG_OK;
-}
-
-// sums[O][2] (fp64) = (sum z, sum z^2) over (B, Df, Hf, Wf): the batch statistics of a training-mode BatchNorm from the
-// convolution output itself; rows_ws: fp64 workspace of B*Hf*O*2 doubles
-int cv_stem_z_moments(const float* z, double* sums, double* rows_ws, int B, int O, int Df, int Hf, int Wf, cudaStream_t st) {
-    if (!z || !sums || !rows_ws) return fail(RAG_E_NULL, "cv_stem_z_moments: null pointer");
-    if (int e = check_stem_train("cv_stem_z_moments", B, kStC, O, Df, Hf, Wf)) return e;
-    if (!aligned(z, 16) || !aligned(sums, 8) || !aligned(rows_ws, 8)) return fail(RAG_E_ALIGN, "cv_stem_z_moments: z must be 16-byte aligned");
-    stem_z_rows_kernel<<<dim3(Hf, O, B), 256, 0, st>>>(z, rows_ws, O, Df, Hf, Wf);
-    if (int e = check_launch("cv_stem_z_moments(rows)")) return e;
-    stem_bnb_final_kernel<<<O, 32, 0, st>>>(rows_ws, sums, B * Hf, O);
-    return check_launch("cv_stem_z_moments(final)");
-}
-
-// bn [O][4] / stats [O][2] from the batch moments (batch != 0) or the running statistics; see stem_bn_finalize_kernel
-int cv_stem_bn_finalize(const double* sums, const float* gamma, const float* beta, float* running_mean, float* running_var, double* stats,
-                        float* bn, int O, double n, double eps, double momentum, int batch, int update, cudaStream_t st) {
-    if (!gamma || !beta || !stats || !bn || (batch && !sums) || ((!batch || update) && (!running_mean || !running_var)))
-        return fail(RAG_E_NULL, "cv_stem_bn_finalize: null pointer");
-    if (O <= 0 || n < 1.0) return fail(RAG_E_SHAPE, "cv_stem_bn_finalize: bad O or n");
-    stem_bn_finalize_kernel<<<(O + 63) / 64, 64, 0, st>>>(sums, gamma, beta, running_mean, running_var, stats, bn, O, n, eps, momentum, batch, update);
-    return check_launch("cv_stem_bn_finalize");
-}
-
-int cv_stem_bwd_consts(const double* sums, const float* bn, float* consts, float* gparam, int O, double n, int batch, cudaStream_t st) {
-    if (!sums || !bn || !consts || !gparam) return fail(RAG_E_NULL, "cv_stem_bwd_consts: null pointer");
-    if (O <= 0 || n < 1.0) return fail(RAG_E_SHAPE, "cv_stem_bwd_consts: bad O or n");
-    stem_bwd_consts_kernel<<<(O + 63) / 64, 64, 0, st>>>(sums, bn, consts, gparam, O, n, batch);
-    return check_launch("cv_stem_bwd_consts");
-}
-
-// z <- relu(z * scale[o] + shift[o]) in place (one fused multiply-add per element: the expression the backward re-evaluates)
-int cv_stem_bn_relu(float* z, const float* scale, const float* shift, int stride, int B, int O, int Df, int Hf, int Wf, cudaStream_t st) {
-    if (!z || !scale || !shift) return fail(RAG_E_NULL, "cv_stem_bn_relu: null pointer");
-    if (int e = check_stem_train("cv_stem_bn_relu", B, kStC, O, Df, Hf, Wf)) return e;
-    if (!aligned(z, 16)) return fail(RAG_E_ALIGN, "cv_stem_bn_relu: z must be 16-byte aligned");
-    const size_t chan4 = (size_t)Df * Hf * Wf / 4, n4 = chan4 * O * B;
-    const unsigned grid = (unsigned)std::min<size_t>((n4 + 255) / 256, (size_t)num_sms() * 32);
-    stem_bn_relu_kernel<<<grid, 256, 0, st>>>(z, scale, shift, n4, chan4, O, stride);
-    return check_launch("cv_stem_bn_relu");
-}
-
-// sums[O][2] (fp64) = (sum g', sum g'*zh) over (B, Df, Hf, Wf); bn [O][4] = (scale, shift, mean, rstd); rows_ws: B*Hf*O*2 doubles
-int cv_stem_bn_bwd_sums(const float* g, const float* z, const float* bn, double* sums, double* rows_ws,
-                        int B, int O, int Df, int Hf, int Wf, cudaStream_t st) {
-    if (!g || !z || !bn || !sums || !rows_ws) return fail(RAG_E_NULL, "cv_stem_bn_bwd_sums: null pointer");
-    if (int e = check_stem_train("cv_stem_bn_bwd_sums", B, kStC, O, Df, Hf, Wf)) return e;
-    if (!aligned(g, 16) || !aligned(z, 16) || !aligned(sums, 8) || !aligned(rows_ws, 8)) return fail(RAG_E_ALIGN, "cv_stem_bn_bwd_sums: g/z must be 16-byte aligned");
-    stem_bnb_rows_kernel<<<dim3(Hf, O, B), 256, 0, st>>>(g, z, bn, rows_ws, O, Df, Hf, Wf);
-    if (int e = check_launch("cv_stem_bn_bwd_sums(rows)")) return e;
-    stem_bnb_final_kernel<<<O, 32, 0, st>>>(rows_ws, sums, B * Hf, O);
-    return check_launch("cv_stem_bn_bwd_sums(final)");
 }
 
 size_t cv_stem_bwd_workspace_bytes(int B, int C, int O, int Hf, int Wf) {

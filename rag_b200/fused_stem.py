@@ -21,7 +21,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import _cabi
+from . import _cabi, batchnorm
 from .functional import _require, _stream, cost_volume
 from .last_conv import conv_forward
 
@@ -110,87 +110,50 @@ def cv_stem_batch_stats(x, y, weight, maxdisp=192):
 class FusedStemFn(torch.autograd.Function):
     """out = relu(batchnorm(conv3d(cost_volume(x, y), weight))) with gradients w.r.t. x, y, weight, gamma, beta.
 
-    Forward: the convolution output z from the fused kernel (the volume is never built), its batch moments in one read
-    (``batch_stats``; else the given running statistics), BatchNorm + ReLU IN PLACE.  Returns ``(out, mean, var)`` -- the
-    statistics the layer normalised with, fp64, non-differentiable (the caller updates the running estimates from them).
-    Saved for the backward: the two feature maps, the weight and a few [O] vectors -- no [B,*,Df,Hf,Wf] tensor: z is
-    RECOMPUTED by the forward kernel inside ``backward`` into a temporary, and the backward kernels re-evaluate the forward's
-    own expression ``fma(z, scale, shift) > 0`` for the ReLU decision (bit-identical)."""
+    Forward: the convolution output z from the fused kernel (the volume is never built), then the BatchNorm + ReLU of
+    ``batchnorm.forward`` IN PLACE.  Saved for the backward: the two feature maps, the weight and the [O,4] table -- no
+    [B,*,Df,Hf,Wf] tensor: z is RECOMPUTED by the forward kernel inside ``backward`` into a temporary, and the backward kernels
+    re-evaluate the forward's own expression ``fma(z, scale, shift) > 0`` for the ReLU decision (bit-identical)."""
 
     @staticmethod
-    def forward(ctx, x, y, weight, gamma, beta, running_mean, running_var, batch_stats, update_running, momentum, eps, maxdisp):
-        b, c, hf, wf = x.shape
-        o = weight.shape[0]
-        dev = x.device
-        L = _cabi.lib()
+    def forward(ctx, x, y, weight, maxdisp, gamma, beta, running_mean, running_var, batch_stats, update_running, momentum, eps):
         z = cv_stem_forward(x, y, weight, None, None, False, maxdisp)
-        df = z.shape[2]
-        n = b * df * hf * wf
-        gamma, beta = gamma.contiguous(), beta.contiguous()
-        with torch.cuda.device(dev):
-            st = _stream(x)
-            sums = None
-            if batch_stats:
-                sums = torch.empty((o, 2), dtype=torch.float64, device=dev)
-                rows = torch.empty((b * hf * o * 2,), dtype=torch.float64, device=dev)
-                _cabi.check(L.rag_cv_stem_z_moments(z.data_ptr(), sums.data_ptr(), rows.data_ptr(), b, o, df, hf, wf, st), "rag_cv_stem_z_moments")
-            stats = torch.empty((o, 2), dtype=torch.float64, device=dev)         # (mean, biased variance) the layer normalises with
-            bn = torch.empty((o, 4), dtype=torch.float32, device=dev)            # (scale, shift, mean, rstd)
-            rc = L.rag_cv_stem_bn_finalize(sums.data_ptr() if sums is not None else None, gamma.data_ptr(), beta.data_ptr(),
-                                           running_mean.data_ptr() if running_mean is not None else None,
-                                           running_var.data_ptr() if running_var is not None else None,
-                                           stats.data_ptr(), bn.data_ptr(), o, float(n), float(eps), float(momentum), int(bool(batch_stats)),
-                                           int(bool(update_running)), st)
-            _cabi.check(rc, "rag_cv_stem_bn_finalize")
-            _cabi.check(L.rag_cv_stem_bn_relu_bn(z.data_ptr(), bn.data_ptr(), b, o, df, hf, wf, st), "rag_cv_stem_bn_relu")
+        bn = batchnorm.forward(z, z, gamma, beta, running_mean, running_var, batch_stats, update_running, momentum, eps)
         ctx.save_for_backward(x, y, weight, bn)
         ctx.batch_stats, ctx.maxdisp = bool(batch_stats), maxdisp
-        ctx.mark_non_differentiable(stats)
-        return z, stats                               # z now holds the layer output
+        return z                                      # z now holds the layer output
 
     @staticmethod
     @torch.autograd.function.once_differentiable
-    def backward(ctx, g, _gstats):
+    def backward(ctx, g):
         x, y, weight, bn = ctx.saved_tensors
         g = g.contiguous()
         b, c, hf, wf = x.shape
-        o = weight.shape[0]
-        df = g.shape[2]
-        n = b * df * hf * wf
-        dev = x.device
+        o, df = weight.shape[0], g.shape[2]
         L = _cabi.lib()
         need_in = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
         need_w = ctx.needs_input_grad[2]
-        with torch.cuda.device(dev):
-            st = _stream(x)
+        with torch.cuda.device(x.device):
             z = cv_stem_forward(x, y, weight, None, None, False, ctx.maxdisp)           # temporary: the convolution output again
-            sums = torch.empty((o, 2), dtype=torch.float64, device=dev)
-            rows = torch.empty((b * hf * o * 2,), dtype=torch.float64, device=dev)
-            rc = L.rag_cv_stem_bn_bwd_sums(g.data_ptr(), z.data_ptr(), bn.data_ptr(), sums.data_ptr(), rows.data_ptr(), b, o, df, hf, wf, st)
-            _cabi.check(rc, "rag_cv_stem_bn_bwd_sums")
-            consts = torch.empty((o, 7), dtype=torch.float32, device=dev)
-            gparam = torch.empty((2, o), dtype=torch.float32, device=dev)
-            _cabi.check(L.rag_cv_stem_bwd_consts(sums.data_ptr(), bn.data_ptr(), consts.data_ptr(), gparam.data_ptr(), o, float(n), int(ctx.batch_stats), st),
-                        "rag_cv_stem_bwd_consts")
+            consts, ggamma, gbeta, _ = batchnorm.backward(g, z, bn, ctx.batch_stats, want_gz=False)
             gx = gy = gw = None
             if need_in or need_w:
-                ws = torch.empty(int(L.rag_cv_stem_bwd_workspace_bytes(b, c, o, hf, wf)) // 4, dtype=torch.float32, device=dev)
+                ws = torch.empty(int(L.rag_cv_stem_bwd_workspace_bytes(b, c, o, hf, wf)) // 4, dtype=torch.float32, device=x.device)
                 if need_in:
                     gx, gy = torch.empty_like(x), torch.empty_like(y)
-                if need_w:
-                    gw = torch.empty_like(weight)
+                gw = torch.empty_like(weight) if need_w else None
                 rc = L.rag_cv_stem_bwd(g.data_ptr(), z.data_ptr(), consts.data_ptr(), x.data_ptr(), y.data_ptr(), weight.data_ptr(),
                                        gx.data_ptr() if gx is not None else None, gy.data_ptr() if gy is not None else None,
-                                       gw.data_ptr() if gw is not None else None, ws.data_ptr(), b, c, o, df, hf, wf, st)
+                                       gw.data_ptr() if gw is not None else None, ws.data_ptr(), b, c, o, df, hf, wf, _stream(x))
                 _cabi.check(rc, "rag_cv_stem_bwd")
-        return (gx if ctx.needs_input_grad[0] else None, gy if ctx.needs_input_grad[1] else None, gw,
-                gparam[0] if ctx.needs_input_grad[3] else None, gparam[1] if ctx.needs_input_grad[4] else None,
-                None, None, None, None, None, None, None)
+        return (gx if ctx.needs_input_grad[0] else None, gy if ctx.needs_input_grad[1] else None, gw, None,
+                ggamma if ctx.needs_input_grad[4] else None, gbeta if ctx.needs_input_grad[5] else None,
+                None, None, None, None, None, None)
 
 
 def _train_fusable(self, vol: VirtualCostVolume) -> bool:
-    """The layer csrc/cv_stem_train.cu differentiates: Conv3d(2*12 -> O <= 32, 3x3x3) + affine BatchNorm3d + ReLU on a volume
-    with Wf % 4 == 0, 8 <= Wf <= 1016 and Df >= 3."""
+    """The layer csrc/cv_stem_train.cu (the convolution) and csrc/bn3d.cu (its BatchNorm) differentiate: Conv3d(2*12 -> O <= 32,
+    3x3x3) + affine BatchNorm3d + ReLU on a volume with Wf % 4 == 0, 8 <= Wf <= 1016 and Df >= 3."""
     bn = self.bn
     b, c, hf, wf = vol.x.shape
     return (self.use_bn and bool(self.relu) and isinstance(bn, nn.BatchNorm3d) and bn.affine and bn.weight.dtype == torch.float32
@@ -201,18 +164,7 @@ def _train_fusable(self, vol: VirtualCostVolume) -> bool:
 def stem_train_forward(self, vol: VirtualCostVolume) -> torch.Tensor:
     """ConvBR_3d.forward on a VirtualCostVolume with autograd (train() or eval() BatchNorm), fused.  Updates the running
     statistics exactly like nn.BatchNorm3d does in train() (momentum / cumulative average, unbiased variance)."""
-    bn = self.bn
-    x, y = vol.x.contiguous(), vol.y.contiguous()
-    use_batch = bn.training or not bn.track_running_stats
-    update = use_batch and bn.training and bn.track_running_stats
-    f = 0.0
-    if update:
-        if bn.num_batches_tracked is not None:
-            bn.num_batches_tracked.add_(1)
-        f = (1.0 / float(bn.num_batches_tracked)) if bn.momentum is None else float(bn.momentum)
-    out, _stats = FusedStemFn.apply(x, y, self.conv.weight, bn.weight, bn.bias, bn.running_mean, bn.running_var,
-                                    use_batch, update, f, bn.eps, vol.maxdisp)
-    return out
+    return batchnorm.apply(FusedStemFn, self.bn, vol.x.contiguous(), vol.y.contiguous(), self.conv.weight, vol.maxdisp)
 
 
 def _fusable(conv: nn.Conv3d, vol: VirtualCostVolume) -> bool:
@@ -243,11 +195,7 @@ def stem_forward(self, x):
         out = cv_stem_forward(x.x, x.y, self.conv.weight, maxdisp=x.maxdisp)
         out = self.bn(out)
         return F.relu(out, inplace=True) if self.relu else out
-    scale = shift = None
-    if self.use_bn:
-        bn = self.bn
-        scale = (bn.weight if bn.weight is not None else torch.ones_like(bn.running_var)) * torch.rsqrt(bn.running_var + bn.eps)
-        shift = (bn.bias if bn.bias is not None else torch.zeros_like(bn.running_mean)) - bn.running_mean * scale
+    scale, shift = batchnorm.eval_fold(self.bn) if self.use_bn else (None, None)
     return cv_stem_forward(x.x, x.y, self.conv.weight, scale, shift, bool(self.relu), x.maxdisp)
 
 

@@ -6,11 +6,10 @@ every ``conv_3x3`` op of the ``Cell_3d``s.  cuDNN is poor at these small-channel
 runs them in fp32 for (C, O) in ``PAIRS``:
 
 * inference (BatchNorm in eval(), no gradient): one pass, the BatchNorm folded into the store with the ReLU;
-* with batch statistics or a gradient: ``ConvBR3dFn`` -- the raw convolution output z, its batch moments and the running
-  estimates (``rag_cv_stem_z_moments`` / ``rag_cv_stem_bn_finalize``, the fused stem's helpers), and BatchNorm + ReLU into a
-  second tensor (``rag_cv_stem_bn_relu_bn`` on a copy: z survives for the backward).  The backward forms the gradient at
-  the convolution output once (``rag_conv3d_cc_bn_bwd_gz``), runs the forward kernel on it with the weights transposed and
-  flipped for the data gradient, and reduces the weight gradient in a fixed order (bitwise repeatable).
+* with batch statistics or a gradient: ``ConvBR3dFn`` -- the raw convolution output z, then the BatchNorm + ReLU of
+  ``batchnorm`` (csrc/bn3d.cu) into a copy of z (z survives for the backward).  The backward forms the gradient at the
+  convolution output once (``batchnorm.backward``), runs the forward kernel on it with the weights transposed and flipped for
+  the data gradient, and reduces the weight gradient in a fixed order (bitwise repeatable).
 
 ``qualifies(layer, x)`` is the only routing decision; ``matching_forward`` -- bound onto ``ConvBR_3d.forward`` by
 ``rag_b200.network.install(..., matching_convs=True)`` -- sends qualifying plain-tensor calls here and everything else to
@@ -20,9 +19,8 @@ from __future__ import annotations
 
 import torch
 import torch.nn as nn
-from torch.autograd.graph import increment_version
 
-from . import _cabi
+from . import _cabi, batchnorm
 from .functional import _require, _stream
 from .fused_stem import stem_forward
 
@@ -67,28 +65,9 @@ class ConvBR3dFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, weight, gamma, beta, running_mean, running_var, batch_stats, update_running, momentum, eps):
-        b, c, d, h, w = x.shape
-        o = weight.shape[0]
-        dev = x.device
-        L = _cabi.lib()
         z = conv3d_cc_forward(x, weight)
-        n = b * d * h * w
-        gamma, beta = gamma.contiguous(), beta.contiguous()
-        with torch.cuda.device(dev):
-            st = _stream(x)
-            sums = None
-            if batch_stats:
-                sums = torch.empty((o, 2), dtype=torch.float64, device=dev)
-                rows = torch.empty((b * h * o * 2,), dtype=torch.float64, device=dev)
-                _cabi.check(L.rag_cv_stem_z_moments(z.data_ptr(), sums.data_ptr(), rows.data_ptr(), b, o, d, h, w, st), "rag_cv_stem_z_moments")
-            stats = torch.empty((o, 2), dtype=torch.float64, device=dev)
-            bn = torch.empty((o, 4), dtype=torch.float32, device=dev)            # (scale, shift, mean, rstd)
-            rc = L.rag_cv_stem_bn_finalize(sums.data_ptr() if sums is not None else None, gamma.data_ptr(), beta.data_ptr(),
-                                           running_mean.data_ptr(), running_var.data_ptr(), stats.data_ptr(), bn.data_ptr(), o,
-                                           float(n), float(eps), float(momentum), int(bool(batch_stats)), int(bool(update_running)), st)
-            _cabi.check(rc, "rag_cv_stem_bn_finalize")
-            out = z.clone()
-            _cabi.check(L.rag_cv_stem_bn_relu_bn(out.data_ptr(), bn.data_ptr(), b, o, d, h, w, st), "rag_cv_stem_bn_relu")
+        out = z.clone()
+        bn = batchnorm.forward(z, out, gamma, beta, running_mean, running_var, batch_stats, update_running, momentum, eps)
         ctx.save_for_backward(x, weight, z, bn)
         ctx.batch_stats = bool(batch_stats)
         return out
@@ -97,43 +76,22 @@ class ConvBR3dFn(torch.autograd.Function):
     @torch.autograd.function.once_differentiable
     def backward(ctx, g):
         x, weight, z, bn = ctx.saved_tensors
-        g = g.contiguous()
         b, c, d, h, w = x.shape
         o = weight.shape[0]
-        n = b * d * h * w
-        dev = x.device
-        L = _cabi.lib()
         need_x, need_w, need_gamma, need_beta = ctx.needs_input_grad[:4]
-        gx = gw = ggamma = gbeta = None
-        with torch.cuda.device(dev):
-            st = _stream(x)
-            sums = torch.empty((o, 2), dtype=torch.float64, device=dev)
-            rows = torch.empty((b * h * o * 2,), dtype=torch.float64, device=dev)
-            _cabi.check(L.rag_cv_stem_bn_bwd_sums(g.data_ptr(), z.data_ptr(), bn.data_ptr(), sums.data_ptr(), rows.data_ptr(), b, o, d, h, w, st),
-                        "rag_cv_stem_bn_bwd_sums")
-            consts = torch.empty((o, 7), dtype=torch.float32, device=dev)
-            gparam = torch.empty((2, o), dtype=torch.float32, device=dev)
-            _cabi.check(L.rag_cv_stem_bwd_consts(sums.data_ptr(), bn.data_ptr(), consts.data_ptr(), gparam.data_ptr(), o, float(n), int(ctx.batch_stats), st),
-                        "rag_cv_stem_bwd_consts")
-            if need_gamma:
-                ggamma = gparam[0]
-            if need_beta:
-                gbeta = gparam[1]
-            if need_x or need_w:
-                gz = torch.empty_like(z)
-                _cabi.check(L.rag_conv3d_cc_bn_bwd_gz(g.data_ptr(), z.data_ptr(), consts.data_ptr(), gz.data_ptr(), b, o, d, h, w, st),
-                            "rag_conv3d_cc_bn_bwd_gz")
-                if need_x:
-                    gx = torch.empty_like(x)
-                ws = None
-                if need_w:
-                    gw = torch.empty_like(weight)
-                    ws = torch.empty(int(L.rag_conv3d_cc_bwd_workspace_bytes(b, c, o, d, h, w)) // 4, dtype=torch.float32, device=dev)
+        _, ggamma, gbeta, gz = batchnorm.backward(g.contiguous(), z, bn, ctx.batch_stats, want_gz=need_x or need_w)
+        gx = gw = None
+        if need_x or need_w:
+            L = _cabi.lib()
+            with torch.cuda.device(x.device):
+                gx = torch.empty_like(x) if need_x else None
+                gw = torch.empty_like(weight) if need_w else None
+                ws = torch.empty(int(L.rag_conv3d_cc_bwd_workspace_bytes(b, c, o, d, h, w)) // 4, dtype=torch.float32, device=x.device) if need_w else None
                 rc = L.rag_conv3d_cc_bwd(gz.data_ptr(), x.data_ptr(), weight.data_ptr(), gx.data_ptr() if gx is not None else None,
                                          gw.data_ptr() if gw is not None else None, ws.data_ptr() if ws is not None else None,
-                                         b, c, o, d, h, w, st)
-                _cabi.check(rc, "rag_conv3d_cc_bwd")
-        return gx, gw, ggamma, gbeta, None, None, None, None, None, None
+                                         b, c, o, d, h, w, _stream(x))
+            _cabi.check(rc, "rag_conv3d_cc_bwd")
+        return gx, gw, ggamma if need_gamma else None, gbeta if need_beta else None, None, None, None, None, None, None
 
 
 def _wants_grad(layer: nn.Module, x: torch.Tensor) -> bool:
@@ -158,7 +116,7 @@ def layer_qualifies(layer: nn.Module) -> bool:
 def qualifies(layer: nn.Module, x) -> bool:
     """True when ``layer(x)`` is the layer csrc/conv3d_cc.cu implements: ``layer_qualifies(layer)`` with the weight on CUDA,
     and x a CUDA fp32 [B,C,D,H,W] tensor on the weight's device with W % 4 == 0 and within the kernels' limits.  Whenever
-    batch statistics are used or a gradient is wanted, also the limits of the BatchNorm helpers (csrc/cv_stem_train.cu):
+    batch statistics are used or a gradient is wanted, also the limits of the BatchNorm kernels (csrc/bn3d.cu):
     O <= 32, D >= 3, 8 <= W <= 1016."""
     if not layer_qualifies(layer) or not layer.conv.weight.is_cuda:
         return False
@@ -179,23 +137,10 @@ def qualifies(layer: nn.Module, x) -> bool:
 
 def convbr_forward(layer: nn.Module, x: torch.Tensor) -> torch.Tensor:
     """A qualifying ConvBR_3d call on the kernels.  Updates the running statistics exactly like nn.BatchNorm3d does in
-    train() (momentum or cumulative average, unbiased variance, num_batches_tracked)."""
-    bn = layer.bn
-    if not bn.training and not _wants_grad(layer, x):
-        scale = bn.weight * torch.rsqrt(bn.running_var + bn.eps)
-        shift = bn.bias - bn.running_mean * scale
-        return conv3d_cc_forward(x, layer.conv.weight, scale, shift, relu=True)
-    f = 0.0
-    if bn.training:
-        if bn.num_batches_tracked is not None:
-            bn.num_batches_tracked.add_(1)
-        f = (1.0 / float(bn.num_batches_tracked)) if bn.momentum is None else float(bn.momentum)
-    out = ConvBR3dFn.apply(x.contiguous(), layer.conv.weight, bn.weight, bn.bias, bn.running_mean, bn.running_var,
-                           bn.training, bn.training, f, bn.eps)
-    if bn.training:     # the finaliser wrote the running estimates in place: bump their version counters as F.batch_norm does
-        increment_version(bn.running_mean)
-        increment_version(bn.running_var)
-    return out
+    train() (momentum or cumulative average, unbiased variance, batch count)."""
+    if not layer.bn.training and not _wants_grad(layer, x):
+        return conv3d_cc_forward(x, layer.conv.weight, *batchnorm.eval_fold(layer.bn), relu=True)
+    return batchnorm.apply(ConvBR3dFn, layer.bn, x.contiguous(), layer.conv.weight)
 
 
 def matching_forward(self, x):

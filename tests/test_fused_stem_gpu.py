@@ -287,8 +287,10 @@ def test_training_stem_matches_the_reference_golden():
         layer.conv.weight.copy_(t("weight")); layer.bn.weight.copy_(t("bn_weight")); layer.bn.bias.copy_(t("bn_bias"))
         layer.bn.running_mean.copy_(t("bn_mean0")); layer.bn.running_var.copy_(t("bn_var0"))
     x, y = t("x").requires_grad_(True), t("y").requires_grad_(True)
+    v0 = (layer.bn.running_mean._version, layer.bn.running_var._version)
     out = stem_forward(layer, VirtualCostVolume(x, y, md))
     assert out.grad_fn is not None and "FusedStemFn" in type(out.grad_fn).__name__
+    assert layer.bn.running_mean._version > v0[0] and layer.bn.running_var._version > v0[1]      # written in place, as F.batch_norm marks it
     out.backward(t("gout"))
     tol = 1e-5
     assert _mx(out.detach(), t("out")) <= tol

@@ -14,7 +14,7 @@ def test_exports_answer_errors_without_gpu():
     L = _cabi.lib()
     assert L.rag_conv3d_cc_fwd(None, None, None, None, 1, None, 1, 12, 12, 4, 4, 8, None) == -1
     assert b"null" in L.rag_last_error()
-    assert L.rag_conv3d_cc_bn_bwd_gz(None, None, None, None, 1, 12, 4, 4, 8, None) == -1
+    assert L.rag_bn3d_bwd_gz(None, None, None, None, 1, 12, 4, 4, 8, None) == -1
     assert L.rag_conv3d_cc_bwd(None, None, None, None, None, None, 1, 12, 12, 4, 4, 8, None) == -1
     # an unsupported (C, O) is a shape error, reported before any pointer is touched
     fake = 256

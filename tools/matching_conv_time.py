@@ -105,7 +105,7 @@ def main():
                 res["ours_data_grad_kernel"] = timed(lambda: _cabi.check(L.rag_conv3d_cc_bwd(gout.data_ptr(), x.data_ptr(), wt.data_ptr(), gin.data_ptr(), None, None, b, c, o, d, h, w, st), "bwd"))
                 res["ours_weight_grad_kernels"] = timed(lambda: _cabi.check(L.rag_conv3d_cc_bwd(gout.data_ptr(), x.data_ptr(), wt.data_ptr(), None, gw.data_ptr(), ws.data_ptr(), b, c, o, d, h, w, st), "bwd"))
                 consts = torch.rand(o, 7, device=dev)
-                res["ours_gz_kernel"] = timed(lambda: _cabi.check(L.rag_conv3d_cc_bn_bwd_gz(gout.data_ptr(), gout.data_ptr(), consts.data_ptr(), gz.data_ptr(), b, o, d, h, w, st), "gz"))
+                res["ours_gz_kernel"] = timed(lambda: _cabi.check(L.rag_bn3d_bwd_gz(gout.data_ptr(), gout.data_ptr(), consts.data_ptr(), gz.data_ptr(), b, o, d, h, w, st), "gz"))
             # ---- cuDNN through the mirror layer ----
             ref = copy.deepcopy(lay)
             for tf32 in (True, False):

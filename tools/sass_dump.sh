@@ -33,7 +33,7 @@ summ "head_bwd_x3w_kernelILb1ELb1" r2_head_bwd_x3w
 summ "stem_bwd_maps_kernelILi8" r2_stem_train
 summ "stem_bwd_inputs_kernel" r2_stem_train
 summ "stem_bwd_weight_kernel" r2_stem_train
-summ "stem_bnb_rows_kernel" r2_stem_train
+summ "bn3d_bwd_rows_kernel" r2_stem_train
 summ "conv3d_c1_bwd_data" r2_tail
 summ "conv3d_c1_bwd_weight_kernel" r2_tail
 summ "trilinear_fwd_kernelILb1" r2_tail
