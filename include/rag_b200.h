@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define RAG_B200_ABI_VERSION 15
+#define RAG_B200_ABI_VERSION 16
 
 #if defined(__GNUC__)
 #define RAG_API __attribute__((visibility("default")))
@@ -272,6 +272,29 @@ RAG_API int rag_conv3d_cc_fwd(const float* in, const float* w, const float* scal
 RAG_API size_t rag_conv3d_cc_bwd_workspace_bytes(int B, int C, int O, int D, int H, int W);
 RAG_API int rag_conv3d_cc_bwd(const float* gz, const float* in, const float* w, float* gin, float* gw, void* workspace,
                       int B, int C, int O, int D, int H, int W, void* stream);
+
+/* The Matching Net's pointwise layers: ConvBR_3d(C, O, 1, 1, 0) of src/automl/operations_3d.py:31-47 = bias-free Conv3d
+ * C -> O (1x1x1) + BatchNorm3d + ReLU -- `last_12_3d` (48 -> 24) and `last_6_3d` (24 -> 12) of src/models/rag_model.py.
+ * Any (C, O) with 1 <= C <= 64 and 1 <= O <= 32 at run time; fp32 accumulation over c = 0..C-1 in order (cuDNN's default
+ * for these layers is TF32).  Stateless and capturable.  S = D*H*W.
+ * Forward:  out[b,o,s] = relu?( fma(z[b,o,s], scale[o], shift[o]) ),  z[b,o,s] = sum_c w[o,c] in[b,c,s]
+ *   in [B,C,D,H,W]; w [O,C,1,1,1] (Conv3d.weight); scale / shift [O] (both NULL = identity: raw z, the training path;
+ *   eval-mode BatchNorm folded: scale = gamma/sqrt(var+eps), shift = beta - mean*scale); relu != 0 clamps at 0;
+ *   out [B,O,D,H,W].  Reads in once, writes out once.
+ * Training: z = the raw forward output goes through the BatchNorm3d section above; rag_bn3d_bwd_sums + rag_bn3d_bwd_consts give
+ * consts [O,7].  rag_conv3d_pw_bwd, from g [B,O,D,H,W] (upstream gradient of the layer output), z and consts, forms the
+ * gradient at the convolution output gz = a (g' - m1 - zh m2) on the fly -- the expression of rag_bn3d_bwd_gz, bit for bit --
+ * without writing it, and from it:
+ *   gin [B,C,D,H,W] (nullable; needs w):            gin[b,c,s] = sum_o w[o,c] gz[b,o,s]
+ *   gw  [O,C,1,1,1] (nullable; needs in, workspace): gw[o,c]    = sum_{b,s} gz[b,o,s] in[b,c,s]
+ *   workspace: rag_conv3d_pw_bwd_workspace_bytes(B,C,O,D,H,W) bytes (0 = outside the limits), caller-owned.  Bitwise
+ *   repeatable: fixed-order per-CTA partials of a fixed grid, fp64 final pass, no atomics.
+ * Needs 1 <= C <= 64, 1 <= O <= 32, B <= 65535, S % 4 == 0 and 16-byte aligned in / out / g / z / gin. */
+RAG_API int rag_conv3d_pw_fwd(const float* in, const float* w, const float* scale, const float* shift, int relu, float* out,
+                      int B, int C, int O, int D, int H, int W, void* stream);
+RAG_API size_t rag_conv3d_pw_bwd_workspace_bytes(int B, int C, int O, int D, int H, int W);
+RAG_API int rag_conv3d_pw_bwd(const float* g, const float* z, const float* consts, const float* in, const float* w, float* gin,
+                      float* gw, void* workspace, int B, int C, int O, int D, int H, int W, void* stream);
 
 /* Trilinear resize of [B*C, Di,Hi,Wi] -> [B*C, Do,Ho,Wo] with PyTorch's fp32 index arithmetic: the `upsample_6` /
  * `upsample_12` steps of the Matching Net's tail, nn.Upsample(size=..., mode='trilinear', align_corners=True) at

@@ -12,7 +12,7 @@ import os
 
 from . import build as _build
 
-ABI_VERSION = 15
+ABI_VERSION = 16
 
 _f = C.POINTER(C.c_float)
 _d = C.POINTER(C.c_double)
@@ -58,6 +58,9 @@ SIGNATURES = {
     "rag_conv3d_cc_fwd": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_conv3d_cc_bwd_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i, _i]),
     "rag_conv3d_cc_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "rag_conv3d_pw_fwd": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "rag_conv3d_pw_bwd_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i, _i]),
+    "rag_conv3d_pw_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_trilinear_resize_fwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_trilinear_resize_bwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_normalize_pad": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp]),

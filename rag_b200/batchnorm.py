@@ -1,6 +1,7 @@
 """The BatchNorm3d + ReLU of a ``ConvBR_3d`` (operations_3d.py:31-47) with autograd, on csrc/bn3d.cu: batch or running
-statistics, how the running estimates move, and the launches of its forward and backward, for both the fused stem
-(``fused_stem.FusedStemFn``) and the interior layers (``matching_conv.ConvBR3dFn``)."""
+statistics, how the running estimates move, and the launches of its forward and backward, for the fused stem
+(``fused_stem.FusedStemFn``), the interior layers (``matching_conv.ConvBR3dFn``) and the pointwise layers
+(``pointwise_conv.PointwiseBR3dFn``)."""
 from __future__ import annotations
 
 import torch
@@ -13,6 +14,15 @@ from .functional import _stream
 
 def _ptr(t):
     return t.data_ptr() if t is not None else None
+
+
+def bn_relu_qualifies(layer: nn.Module, out_channels: int) -> bool:
+    """The BatchNorm / ReLU half of a ConvBR_3d routing predicate (``matching_conv`` and ``pointwise_conv``): ``layer.bn`` is
+    an affine fp32 BatchNorm3d over ``out_channels`` that tracks running statistics and is in use, followed by a ReLU."""
+    bn = getattr(layer, "bn", None)
+    return bool(getattr(layer, "use_bn", False) and isinstance(bn, nn.BatchNorm3d) and bn.affine and bn.track_running_stats
+                and bn.num_features == out_channels and bn.weight.dtype == torch.float32 and bn.running_mean.dtype == torch.float32
+                and bool(getattr(layer, "relu", False)))
 
 
 def mode(bn: nn.BatchNorm3d) -> tuple[bool, bool, float]:

@@ -35,6 +35,9 @@ int cv_stem_bwd(const float*, const float*, const float*, const float*, const fl
 int conv3d_cc_fwd(const float*, const float*, const float*, const float*, int, float*, int, int, int, int, int, int, cudaStream_t);
 size_t conv3d_cc_bwd_workspace_bytes(int, int, int, int, int, int);
 int conv3d_cc_bwd(const float*, const float*, const float*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
+int conv3d_pw_fwd(const float*, const float*, const float*, const float*, int, float*, int, int, int, int, int, int, cudaStream_t);
+size_t conv3d_pw_bwd_workspace_bytes(int, int, int, int, int, int);
+int conv3d_pw_bwd(const float*, const float*, const float*, const float*, const float*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
 }  // namespace rag
 
 using namespace rag;
@@ -134,6 +137,15 @@ RAG_API size_t rag_conv3d_cc_bwd_workspace_bytes(int B, int C, int O, int D, int
 RAG_API int rag_conv3d_cc_bwd(const float* gz, const float* in, const float* w, float* gin, float* gw, void* workspace,
                       int B, int C, int O, int D, int H, int W, void* stream) {
     return conv3d_cc_bwd(gz, in, w, gin, gw, static_cast<float*>(workspace), B, C, O, D, H, W, ST(stream));
+}
+RAG_API int rag_conv3d_pw_fwd(const float* in, const float* w, const float* scale, const float* shift, int relu, float* out,
+                      int B, int C, int O, int D, int H, int W, void* stream) {
+    return conv3d_pw_fwd(in, w, scale, shift, relu, out, B, C, O, D, H, W, ST(stream));
+}
+RAG_API size_t rag_conv3d_pw_bwd_workspace_bytes(int B, int C, int O, int D, int H, int W) { return conv3d_pw_bwd_workspace_bytes(B, C, O, D, H, W); }
+RAG_API int rag_conv3d_pw_bwd(const float* g, const float* z, const float* consts, const float* in, const float* w, float* gin, float* gw,
+                      void* workspace, int B, int C, int O, int D, int H, int W, void* stream) {
+    return conv3d_pw_bwd(g, z, consts, in, w, gin, gw, static_cast<float*>(workspace), B, C, O, D, H, W, ST(stream));
 }
 RAG_API int rag_bn3d_moments(const float* z, double* sums, double* rows_ws, int B, int O, int D, int H, int W, void* stream) {
     return bn3d_moments(z, sums, rows_ws, B, O, D, H, W, ST(stream));

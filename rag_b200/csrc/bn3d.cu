@@ -6,6 +6,7 @@
 // where the ReLU is off, so the backward needs z, not only the output.  Fixed-order reductions: bitwise repeatable.
 #include <algorithm>
 
+#include "bn3d.cuh"
 #include "common.cuh"
 
 namespace rag {
@@ -146,7 +147,7 @@ __global__ void bn3d_rows_final_kernel(const double* __restrict__ rows, double* 
     if (lane == 0) { sums[2 * o] = a0; sums[2 * o + 1] = a1; }
 }
 
-// gz = a (g' - m1 - zh m2) with consts [O][7] = (a, m1, m2, scale, shift, mean, rstd).  Grid-stride over float4.
+// gz = a (g' - m1 - zh m2) with consts [O][7] = (a, m1, m2, scale, shift, mean, rstd) (bn3d.cuh).  Grid-stride over float4.
 __global__ void __launch_bounds__(256)
 bn3d_bwd_gz_kernel(const float* __restrict__ g, const float* __restrict__ z, const float* __restrict__ consts, float* __restrict__ gz,
                    size_t n4, size_t chan4, int O) {
@@ -157,10 +158,10 @@ bn3d_bwd_gz_kernel(const float* __restrict__ g, const float* __restrict__ z, con
         const float4 zv = ld_stream(reinterpret_cast<const float4*>(z) + i);
         const float4 gv = ld_stream(reinterpret_cast<const float4*>(g) + i);
         float4 r;
-        r.x = a * ((__fmaf_rn(zv.x, sc, sh) > 0.f ? gv.x : 0.f) - m1 - ((zv.x - mu) * rs) * m2);
-        r.y = a * ((__fmaf_rn(zv.y, sc, sh) > 0.f ? gv.y : 0.f) - m1 - ((zv.y - mu) * rs) * m2);
-        r.z = a * ((__fmaf_rn(zv.z, sc, sh) > 0.f ? gv.z : 0.f) - m1 - ((zv.z - mu) * rs) * m2);
-        r.w = a * ((__fmaf_rn(zv.w, sc, sh) > 0.f ? gv.w : 0.f) - m1 - ((zv.w - mu) * rs) * m2);
+        r.x = bn3d_gz(gv.x, zv.x, a, m1, m2, sc, sh, mu, rs);
+        r.y = bn3d_gz(gv.y, zv.y, a, m1, m2, sc, sh, mu, rs);
+        r.z = bn3d_gz(gv.z, zv.z, a, m1, m2, sc, sh, mu, rs);
+        r.w = bn3d_gz(gv.w, zv.w, a, m1, m2, sc, sh, mu, rs);
         reinterpret_cast<float4*>(gz)[i] = r;
     }
 }

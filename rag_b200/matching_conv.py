@@ -107,10 +107,7 @@ def layer_qualifies(layer: nn.Module) -> bool:
             and conv.padding == (1, 1, 1) and conv.dilation == (1, 1, 1) and conv.groups == 1 and conv.padding_mode == "zeros"
             and conv.weight.dtype == torch.float32 and (conv.in_channels, conv.out_channels) in PAIRS):
         return False
-    bn = getattr(layer, "bn", None)
-    return bool(getattr(layer, "use_bn", False) and isinstance(bn, nn.BatchNorm3d) and bn.affine and bn.track_running_stats
-                and bn.num_features == conv.out_channels and bn.weight.dtype == torch.float32 and bn.running_mean.dtype == torch.float32
-                and bool(getattr(layer, "relu", False)))
+    return batchnorm.bn_relu_qualifies(layer, conv.out_channels)
 
 
 def qualifies(layer: nn.Module, x) -> bool:

@@ -79,7 +79,7 @@ def basic_network_forward(self, left, right, fea_ops, mat_ops):
 
 
 def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_stem: bool = False, upsample: bool = False,
-            matching_convs: bool = False) -> dict:
+            matching_convs: bool = False, pointwise_convs: bool = False) -> dict:
     """Bind the B200 hot path onto the reference's modules (pass the imported module objects
     ``models.rag_model`` and/or ``automl.mdenas_basicmodel``).  Returns what was patched.
     New networks constructed afterwards get ``rag_b200.Disp``; existing instances keep working
@@ -103,7 +103,13 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
     ``conv_3x3`` ops -- also those of the search supernet) run on csrc/conv3d_cc.cu in inference and training (folded
     BatchNorm + ReLU in eval(); batch statistics, running-estimate updates and the backward otherwise).  Every call that does
     not qualify (``matching_conv.qualifies``) goes to the ``fuse_stem`` binding unchanged, so the fused stem, ``last_3_3d``
-    and the cuDNN fallback behave as without the flag."""
+    and the cuDNN fallback behave as without the flag.
+
+    ``pointwise_convs=True`` (needs ``operations_3d``) binds ``ConvBR_3d.forward`` to ``rag_b200.pointwise_conv``'s
+    ``pointwise_forward``: the Matching Net's pointwise ``ConvBR_3d(C, O, 1, 1, 0)`` layers (``last_12_3d``, ``last_6_3d``, the
+    cells' 1x1x1 layers) that ``pointwise_conv.qualifies`` accepts run on csrc/conv3d_pw.cu in inference and training.  Every
+    other call goes to the binding this call makes without the flag: ``matching_forward`` with ``matching_convs=True``,
+    else ``stem_forward``."""
     global _FUSE_STEM, _STEM_AWARE
     done = {}
 
@@ -123,6 +129,14 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
         from .matching_conv import matching_forward
 
         bind(operations_3d.ConvBR_3d, "forward", matching_forward)   # delegates to stem_forward: fusion-aware as well
+        _STEM_AWARE = True
+        done["operations_3d"] = ["ConvBR_3d.forward"]
+    if pointwise_convs:
+        if operations_3d is None:
+            raise ValueError("pointwise_convs=True needs operations_3d (the reference's automl.operations_3d module)")
+        from .pointwise_conv import pointwise_forward, pointwise_matching_forward
+
+        bind(operations_3d.ConvBR_3d, "forward", pointwise_matching_forward if matching_convs else pointwise_forward)
         _STEM_AWARE = True
         done["operations_3d"] = ["ConvBR_3d.forward"]
     _FUSE_STEM = bool(fuse_stem)          # always (re)set: install(fuse_stem=False) after a fused install turns it off

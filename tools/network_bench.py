@@ -3,12 +3,14 @@ how much of a full forward / training step the hot path (and the rows next to it
 
     python tools/network_bench.py [--size 288x576] [--batch 4]
 
-Four configurations, same weights and inputs: (a) the unmodified reference (PyTorch eager + cuDNN, TF32 on as by default),
+Five configurations, same weights and inputs: (a) the unmodified reference (PyTorch eager + cuDNN, TF32 on as by default),
 (b) install() -- cost volume + disparity head through the hand-written kernels, (c) install(fuse_stem=True, upsample=True) --
 additionally the first Matching-Net layer fused with the volume (never materialised, forward and backward) and the tail
-(upsample_12/6, last_3_3d), (d) as (c) plus matching_convs=True -- the interior 3x3x3 ConvBR_3d layers on csrc/conv3d_cc.cu.
+(upsample_12/6, last_3_3d), (d) as (c) plus matching_convs=True -- the interior 3x3x3 ConvBR_3d layers on csrc/conv3d_cc.cu,
+(e) as (d) plus pointwise_convs=True -- the pointwise 1x1x1 ConvBR_3d layers on csrc/conv3d_pw.cu.
 Forward = eval() under no_grad (approaches/rag.py:408-441); training step = train() forward +
-masked smooth-L1 + backward (approaches/rag.py:205-216, optimizer step excluded).  Prints one JSON line per configuration."""
+masked smooth-L1 + backward (approaches/rag.py:205-216, optimizer step excluded).  Prints one JSON line per configuration;
+without the reference installed in oracle/_ref it prints one line saying the network was not measured."""
 import argparse
 import json
 import os
@@ -30,6 +32,9 @@ def main():
     a = ap.parse_args()
     H, W = (int(v) for v in a.size.split("x"))
     dev = torch.device("cuda:0")
+    if not R.available():
+        print(json.dumps({"note": "not measured: the unmodified reference is not installed in oracle/_ref"}), flush=True)
+        return
     ref = R.import_reference()
     torch.manual_seed(0)
     net = ref.rag_model.Network(R.make_genotype(ref, 0), dev).to(dev)
@@ -63,7 +68,9 @@ def main():
     for name, kw in (("reference (unpatched)", None), ("install()", {}),
                      ("install(fuse_stem=True, upsample=True)", dict(operations_3d=ref.operations_3d, fuse_stem=True, upsample=True)),
                      ("install(fuse_stem=True, upsample=True, matching_convs=True)",
-                      dict(operations_3d=ref.operations_3d, fuse_stem=True, upsample=True, matching_convs=True))):
+                      dict(operations_3d=ref.operations_3d, fuse_stem=True, upsample=True, matching_convs=True)),
+                     ("install(fuse_stem=True, upsample=True, matching_convs=True, pointwise_convs=True)",
+                      dict(operations_3d=ref.operations_3d, fuse_stem=True, upsample=True, matching_convs=True, pointwise_convs=True))):
         N.uninstall()
         if kw is not None:
             N.install(ref.rag_model, ref.mdenas_basicmodel, **kw)
