@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define RAG_B200_ABI_VERSION 16
+#define RAG_B200_ABI_VERSION 17
 
 #if defined(__GNUC__)
 #define RAG_API __attribute__((visibility("default")))
@@ -304,6 +304,14 @@ RAG_API int rag_trilinear_resize_fwd(const float* in, float* out, int BC, int Di
                              int align_corners, void* stream);
 RAG_API int rag_trilinear_resize_bwd(const float* gout, float* gin, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo,
                              int align_corners, void* stream);
+
+/* Bilinear resize of [B*C, Hi,Wi] -> [B*C, Ho,Wo]: F.interpolate(..., mode='bilinear') on an NCHW tensor, with the same fp32
+ * index arithmetic, argument checks and error codes as the trilinear pair above (the same kernels with the depth axis
+ * compiled out).  The backward is a fixed-order gather per input pixel: bitwise repeatable.  Nothing is allocated. */
+RAG_API int rag_bilinear_resize_fwd(const float* in, float* out, int BC, int Hi, int Wi, int Ho, int Wo, int align_corners,
+                            void* stream);
+RAG_API int rag_bilinear_resize_bwd(const float* gout, float* gin, int BC, int Hi, int Wi, int Ho, int Wo, int align_corners,
+                            void* stream);
 
 /* Eval-time input staging: uint8 HWC image -> ImageNet-normalised fp32 CHW, zero-padded on the
  * top and right.  Replaces src/dataloaders/data_io.py:6-13 + stereo_dataset.py:88-102.

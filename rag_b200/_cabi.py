@@ -12,7 +12,7 @@ import os
 
 from . import build as _build
 
-ABI_VERSION = 16
+ABI_VERSION = 17
 
 _f = C.POINTER(C.c_float)
 _d = C.POINTER(C.c_double)
@@ -63,6 +63,8 @@ SIGNATURES = {
     "rag_conv3d_pw_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_trilinear_resize_fwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_trilinear_resize_bwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
+    "rag_bilinear_resize_fwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "rag_bilinear_resize_bwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_normalize_pad": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp]),
 }
 

@@ -24,6 +24,8 @@ int conv3d_c1_bwd(const float*, const float*, const float*, float*, float*, floa
 size_t conv3d_c1_bwd_workspace_bytes(int);
 int trilinear_resize_fwd(const float*, float*, int, int, int, int, int, int, int, int, cudaStream_t);
 int trilinear_resize_bwd(const float*, float*, int, int, int, int, int, int, int, int, cudaStream_t);
+int bilinear_resize_fwd(const float*, float*, int, int, int, int, int, int, cudaStream_t);
+int bilinear_resize_bwd(const float*, float*, int, int, int, int, int, int, cudaStream_t);
 int bn3d_moments(const float*, double*, double*, int, int, int, int, int, cudaStream_t);
 int bn3d_finalize(const double*, const float*, const float*, float*, float*, float*, int, double, double, double, int, int, cudaStream_t);
 int bn3d_relu(float*, const float*, int, int, int, int, int, cudaStream_t);
@@ -172,6 +174,12 @@ RAG_API int rag_trilinear_resize_fwd(const float* in, float* out, int BC, int Di
 }
 RAG_API int rag_trilinear_resize_bwd(const float* gout, float* gin, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int align_corners, void* stream) {
     return trilinear_resize_bwd(gout, gin, BC, Di, Hi, Wi, Do, Ho, Wo, align_corners, ST(stream));
+}
+RAG_API int rag_bilinear_resize_fwd(const float* in, float* out, int BC, int Hi, int Wi, int Ho, int Wo, int align_corners, void* stream) {
+    return bilinear_resize_fwd(in, out, BC, Hi, Wi, Ho, Wo, align_corners, ST(stream));
+}
+RAG_API int rag_bilinear_resize_bwd(const float* gout, float* gin, int BC, int Hi, int Wi, int Ho, int Wo, int align_corners, void* stream) {
+    return bilinear_resize_bwd(gout, gin, BC, Hi, Wi, Ho, Wo, align_corners, ST(stream));
 }
 RAG_API int rag_normalize_pad(const uint8_t* img, float* out, int B, int H, int W, int top_pad, int right_pad, void* stream) {
     return normalize_pad(img, out, B, H, W, top_pad, right_pad, ST(stream));

@@ -13,6 +13,10 @@
 // L1/L2).  Backward: PyTorch scatters with atomicAdd (arrival order: not reproducible); here every INPUT voxel gathers the
 // output voxels that reference it, in a fixed order -- the per-axis (i0, l1) tables and the first-destination index of
 // every source index are built in shared memory by each CTA -- so the result is bitwise repeatable.
+//
+// Bilinear resize of a [B*C, Hi, Wi] image (rag_bilinear_resize_fwd/bwd: the cells' F.interpolate(..., 'bilinear')) runs the
+// same kernels with the depth axis compiled out (template parameter D3 = false, Di = Do = 1): no depth weights, and an output
+// row blends two input rows, not four.  A D = 1 view of the trilinear kernels would blend two copies of the same plane.
 #include <algorithm>
 #include <vector>
 
@@ -39,7 +43,7 @@ __host__ __device__ inline float tri_scale(int n_in, int n_out, bool ac) {
 }
 
 // grid-stride over (bc, d, h, w-quad); Wo % 4 == 0 not required (scalar tail).
-template <bool AC>
+template <bool AC, bool D3>
 __global__ void __launch_bounds__(256)
 trilinear_fwd_kernel(const float* __restrict__ in, float* __restrict__ out, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo,
                      float sd, float sh, float sw, bool vec) {
@@ -52,9 +56,9 @@ trilinear_fwd_kernel(const float* __restrict__ in, float* __restrict__ out, int 
         const int h = (int)(r % Ho); r /= Ho;
         const int d = (int)(r % Do);
         const size_t bc = r / Do;
-        int d0, d1, h0, h1;
+        int d0 = 0, d1 = 0, h0, h1;
         float t0, t1, e0, e1;
-        tri_src<AC>(sd, d, Di, d0, d1, t0, t1);
+        if constexpr (D3) tri_src<AC>(sd, d, Di, d0, d1, t0, t1);
         tri_src<AC>(sh, h, Hi, h0, h1, e0, e1);
         const float* p = in + bc * in_vol;
         const float* r00 = p + (size_t)d0 * in_plane + (size_t)h0 * Wi;
@@ -68,8 +72,11 @@ trilinear_fwd_kernel(const float* __restrict__ in, float* __restrict__ out, int 
             int w0, w1;
             float f0, f1;
             tri_src<AC>(sw, min(w, Wo - 1), Wi, w0, w1, f0, f1);
-            v[k] = t0 * (e0 * (f0 * __ldg(r00 + w0) + f1 * __ldg(r00 + w1)) + e1 * (f0 * __ldg(r01 + w0) + f1 * __ldg(r01 + w1))) +
-                   t1 * (e0 * (f0 * __ldg(r10 + w0) + f1 * __ldg(r10 + w1)) + e1 * (f0 * __ldg(r11 + w0) + f1 * __ldg(r11 + w1)));
+            if constexpr (D3)
+                v[k] = t0 * (e0 * (f0 * __ldg(r00 + w0) + f1 * __ldg(r00 + w1)) + e1 * (f0 * __ldg(r01 + w0) + f1 * __ldg(r01 + w1))) +
+                       t1 * (e0 * (f0 * __ldg(r10 + w0) + f1 * __ldg(r10 + w1)) + e1 * (f0 * __ldg(r11 + w0) + f1 * __ldg(r11 + w1)));
+            else
+                v[k] = e0 * (f0 * __ldg(r00 + w0) + f1 * __ldg(r00 + w1)) + e1 * (f0 * __ldg(r01 + w0) + f1 * __ldg(r01 + w1));
         }
         float* o = out + ((bc * Do + d) * Ho + h) * (size_t)Wo + 4 * q;
         if (vec) {
@@ -103,7 +110,7 @@ __device__ void tri_tables(float scale, int n_in, int n_out, int* i0t, float* l1
 
 // gin[bc, id, ih, iw] = sum over the output voxels that read it of (weight * gout).  One thread per input voxel.
 // smem: per axis  int i0[n_out] | float l1[n_out] | int first[n_in + 1]
-template <bool AC>
+template <bool AC, bool D3>
 __global__ void __launch_bounds__(256)
 trilinear_bwd_kernel(const float* __restrict__ gout, float* __restrict__ gin, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo,
                      float sd, float sh, float sw) {
@@ -111,7 +118,7 @@ trilinear_bwd_kernel(const float* __restrict__ gout, float* __restrict__ gin, in
     int* d_i0 = tri_smem;            float* d_l1 = reinterpret_cast<float*>(d_i0 + Do); int* d_first = reinterpret_cast<int*>(d_l1 + Do);
     int* h_i0 = d_first + Di + 1;    float* h_l1 = reinterpret_cast<float*>(h_i0 + Ho); int* h_first = reinterpret_cast<int*>(h_l1 + Ho);
     int* w_i0 = h_first + Hi + 1;    float* w_l1 = reinterpret_cast<float*>(w_i0 + Wo); int* w_first = reinterpret_cast<int*>(w_l1 + Wo);
-    tri_tables<AC>(sd, Di, Do, d_i0, d_l1, d_first);
+    if constexpr (D3) tri_tables<AC>(sd, Di, Do, d_i0, d_l1, d_first);
     tri_tables<AC>(sh, Hi, Ho, h_i0, h_l1, h_first);
     tri_tables<AC>(sw, Wi, Wo, w_i0, w_l1, w_first);
     const size_t n = (size_t)BC * Di * Hi * Wi;
@@ -127,7 +134,8 @@ trilinear_bwd_kernel(const float* __restrict__ gout, float* __restrict__ gin, in
         const int ih = (int)(r % Hi); r /= Hi;
         const int id = (int)(r % Di);
         const size_t bc = r / Di;
-        const int dl = d_first[max(id - 1, 0)], dh = d_first[id + 1];      // destinations with i0 in {id-1, id}
+        int dl = 0, dh = 1;                                                 // 2-D: the one plane, weight 1
+        if constexpr (D3) dl = d_first[max(id - 1, 0)], dh = d_first[id + 1];   // destinations with i0 in {id-1, id}
         const int hl = h_first[max(ih - 1, 0)], hh = h_first[ih + 1];
         const int wl = w_first[max(iw - 1, 0)], wh = w_first[iw + 1];
         const float* gp = gout + bc * out_vol;
@@ -144,7 +152,7 @@ trilinear_bwd_kernel(const float* __restrict__ gout, float* __restrict__ gin, in
                 ww[k] = w < wh ? wgt(iw, w_i0[wc[k]], w_l1[wc[k]], Wi) : 0.f;
             }
             for (int d = dl; d < dh; ++d) {
-                const float wd = wgt(id, d_i0[d], d_l1[d], Di);
+                const float wd = D3 ? wgt(id, d_i0[d], d_l1[d], Di) : 1.f;
                 float accd = 0.f;
                 for (int h = hl; h < hh; ++h) {
                     const float whh = wgt(ih, h_i0[h], h_l1[h], Hi);
@@ -158,7 +166,7 @@ trilinear_bwd_kernel(const float* __restrict__ gout, float* __restrict__ gin, in
             }
         } else {
             for (int d = dl; d < dh; ++d) {
-                const float wd = wgt(id, d_i0[d], d_l1[d], Di);
+                const float wd = D3 ? wgt(id, d_i0[d], d_l1[d], Di) : 1.f;
                 if (wd == 0.f) continue;
                 float accd = 0.f;
                 for (int h = hl; h < hh; ++h) {
@@ -196,7 +204,7 @@ constexpr int kTriList = 32;              // output rows per input row the backw
 // NPER / NVI = 128-bit vectors per lane of an output row (ceil(Wo / 128)) / of an input row; PF: fetch the input rows one
 // output row ahead (pays for wide rows -- 0.73 -> 0.54 ms at [8,12,32,80,160] -> [64,160,320] --, costs at narrow ones:
 // 0.093 -> 0.108 ms at [4,12,32,48,96] -> [64,96,192])
-template <bool AC, int NPER, int NVI, bool PF>
+template <bool AC, int NPER, int NVI, bool PF, bool D3>
 __global__ void __launch_bounds__(kTriWarps * 32)
 trilinear_fwd_rows_kernel(const float* __restrict__ in, float* __restrict__ out, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo,
                           float sd, float sh, float sw) {
@@ -241,8 +249,8 @@ trilinear_fwd_rows_kernel(const float* __restrict__ in, float* __restrict__ out,
         f_h += inc_h; if (f_h >= Ho) { f_h -= Ho; ++f_d; }
         f_d += inc_d; if (f_d >= Do) { f_d -= Do; ++f_bc; }
         f_bc += inc_bc;
-        int d0, d1, h0, h1;
-        tri_src<AC>(sd, d, Di, d0, d1, r.t0, r.t1);
+        int d0 = 0, d1 = 0, h0, h1;
+        if constexpr (D3) tri_src<AC>(sd, d, Di, d0, d1, r.t0, r.t1);
         tri_src<AC>(sh, h, Hi, h0, h1, r.e0, r.e1);
         const float* p = in + bc * in_vol;
         const float4* r00 = reinterpret_cast<const float4*>(p + (size_t)d0 * in_plane + (size_t)h0 * Wi);
@@ -252,7 +260,10 @@ trilinear_fwd_rows_kernel(const float* __restrict__ in, float* __restrict__ out,
 #pragma unroll
         for (int j = 0; j < NVI; ++j) {
             const int v = lane + 32 * j;
-            if (v < Wiv) { r.a[j] = __ldg(r00 + v); r.b[j] = __ldg(r01 + v); r.c[j] = __ldg(r10 + v); r.e[j] = __ldg(r11 + v); }
+            if (v < Wiv) {
+                r.a[j] = __ldg(r00 + v); r.b[j] = __ldg(r01 + v);
+                if constexpr (D3) { r.c[j] = __ldg(r10 + v); r.e[j] = __ldg(r11 + v); }
+            }
         }
     };
     long long row = (long long)blockIdx.x * kTriWarps + warp;
@@ -272,10 +283,14 @@ trilinear_fwd_rows_kernel(const float* __restrict__ in, float* __restrict__ out,
                 const float4 a = cur.a[j], b = cur.b[j], c = cur.c[j], e = cur.e[j];
                 const float t0 = cur.t0, t1 = cur.t1, e0 = cur.e0, e1 = cur.e1;
                 float4 o;
-                o.x = t0 * (e0 * a.x + e1 * b.x) + t1 * (e0 * c.x + e1 * e.x);
-                o.y = t0 * (e0 * a.y + e1 * b.y) + t1 * (e0 * c.y + e1 * e.y);
-                o.z = t0 * (e0 * a.z + e1 * b.z) + t1 * (e0 * c.z + e1 * e.z);
-                o.w = t0 * (e0 * a.w + e1 * b.w) + t1 * (e0 * c.w + e1 * e.w);
+                if constexpr (D3) {
+                    o.x = t0 * (e0 * a.x + e1 * b.x) + t1 * (e0 * c.x + e1 * e.x);
+                    o.y = t0 * (e0 * a.y + e1 * b.y) + t1 * (e0 * c.y + e1 * e.y);
+                    o.z = t0 * (e0 * a.z + e1 * b.z) + t1 * (e0 * c.z + e1 * e.z);
+                    o.w = t0 * (e0 * a.w + e1 * b.w) + t1 * (e0 * c.w + e1 * e.w);
+                } else {
+                    o.x = e0 * a.x + e1 * b.x; o.y = e0 * a.y + e1 * b.y; o.z = e0 * a.z + e1 * b.z; o.w = e0 * a.w + e1 * b.w;
+                }
                 reinterpret_cast<float4*>(rb)[v] = o;
                 if (v == Wiv - 1) rb[Wi] = o.w;   // "i0 + 1" of the last source column is the column itself (i1 == i0 there)
             }
@@ -299,7 +314,7 @@ trilinear_fwd_rows_kernel(const float* __restrict__ in, float* __restrict__ out,
 // grid-stride over input rows; smem: the three axes' tables (as trilinear_bwd_kernel) | int wfirst[Wi] | float wk[5][Wi]
 // (per source column: its first destination and the weights of the five destinations from there on, 0 past the last) |
 // float [kTriWarps][Wo + 4]
-template <bool AC, int NPER>   // NPER = 128-bit vectors of an output row per lane
+template <bool AC, int NPER, bool D3>   // NPER = 128-bit vectors of an output row per lane
 __global__ void __launch_bounds__(kTriWarps * 32)
 trilinear_bwd_rows_kernel(const float* __restrict__ gout, float* __restrict__ gin, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo,
                           float sd, float sh, float sw) {
@@ -313,7 +328,7 @@ trilinear_bwd_rows_kernel(const float* __restrict__ gout, float* __restrict__ gi
     // per warp: the output rows that reference the current input row as a flat list (row offset in vectors, depth x height weight)
     int* lst_off = reinterpret_cast<int*>(rows + kTriWarps * (Wo + 4)) + (threadIdx.x >> 5) * kTriList;
     float* lst_w = reinterpret_cast<float*>(reinterpret_cast<int*>(rows + kTriWarps * (Wo + 4)) + kTriWarps * kTriList) + (threadIdx.x >> 5) * kTriList;
-    tri_tables<AC>(sd, Di, Do, d_i0, d_l1, d_first);
+    if constexpr (D3) tri_tables<AC>(sd, Di, Do, d_i0, d_l1, d_first);
     tri_tables<AC>(sh, Hi, Ho, h_i0, h_l1, h_first);
     tri_tables<AC>(sw, Wi, Wo, w_i0, w_l1, w_first);
     auto wgt = [](int i, int a, float l1, int n_in) -> float {
@@ -343,7 +358,8 @@ trilinear_bwd_rows_kernel(const float* __restrict__ gout, float* __restrict__ gi
     int ih = (int)(row % Hi), id = (int)((row / Hi) % Di), ibc = (int)(row / ((long long)Hi * Di));
     for (; row < n_rows; row += stride) {
         const size_t bc = (size_t)ibc;
-        const int dl = d_first[max(id - 1, 0)], dh = d_first[id + 1];      // destinations with i0 in {id-1, id}
+        int dl = 0, dh = 1;                                                 // 2-D: the one plane, weight 1
+        if constexpr (D3) dl = d_first[max(id - 1, 0)], dh = d_first[id + 1];   // destinations with i0 in {id-1, id}
         const int hl = h_first[max(ih - 1, 0)], hh = h_first[ih + 1];
         const float* gp = gout + bc * out_vol;
         const int c_id = id, c_ih = ih;
@@ -363,7 +379,8 @@ trilinear_bwd_rows_kernel(const float* __restrict__ gout, float* __restrict__ gi
             if (lane < n_here) {
                 const int e = base + lane, dd = e / nh, d = dl + dd, h = hl + (e - dd * nh);
                 lst_off[lane] = (int)(((size_t)d * out_plane + (size_t)h * Wo) >> 2);
-                lst_w[lane] = wgt(c_id, d_i0[d], d_l1[d], Di) * wgt(c_ih, h_i0[h], h_l1[h], Hi);
+                if constexpr (D3) lst_w[lane] = wgt(c_id, d_i0[d], d_l1[d], Di) * wgt(c_ih, h_i0[h], h_l1[h], Hi);
+                else lst_w[lane] = wgt(c_ih, h_i0[h], h_l1[h], Hi);
             }
             __syncwarp();
             const float4* g4 = reinterpret_cast<const float4*>(gp) + lane;
@@ -447,8 +464,11 @@ static int check_tri(const char* who, const void* a, const void* b, int BC, int 
     return RAG_OK;
 }
 
-int trilinear_resize_fwd(const float* in, float* out, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int align_corners, cudaStream_t st) {
-    if (int e = check_tri("trilinear_resize_fwd", in, out, BC, Di, Hi, Wi, Do, Ho, Wo)) return e;
+// D3 = false: the bilinear exports (Di = Do = 1, depth compiled out); `who` names the export in errors
+template <bool D3>
+static int resize_fwd(const char* who, const float* in, float* out, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int align_corners,
+                      cudaStream_t st) {
+    if (int e = check_tri(who, in, out, BC, Di, Hi, Wi, Do, Ho, Wo)) return e;
     const bool ac = align_corners != 0;
     const float sd = tri_scale(Di, Do, ac), sh = tri_scale(Hi, Ho, ac), sw = tri_scale(Wi, Wo, ac);
     // row kernel: 128-bit rows on both sides, an input row within 2 and an output row within 4 vectors per lane
@@ -460,7 +480,7 @@ int trilinear_resize_fwd(const float* in, float* out, int BC, int Di, int Hi, in
         auto launch = [&](auto kern) -> int {
             if (smem > 48 * 1024) {
                 cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                if (e != cudaSuccess) return fail((int)e, "trilinear_resize_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+                if (e != cudaSuccess) return fail((int)e, "%s: cudaFuncSetAttribute: %s", who, cudaGetErrorString(e));
             }
             kern<<<grid, kTriWarps * 32, smem, st>>>(in, out, BC, Di, Hi, Wi, Do, Ho, Wo, sd, sh, sw);
             return RAG_OK;
@@ -468,25 +488,29 @@ int trilinear_resize_fwd(const float* in, float* out, int BC, int Di, int Hi, in
         int rc = RAG_OK;
         if (smem <= 160 * 1024) {
 #define RAG_TRI_FWD(ACV, NV)                                                                                              \
-    (nper == 1 ? launch(trilinear_fwd_rows_kernel<ACV, 1, NV, (NV > 1)>) : nper == 2 ? launch(trilinear_fwd_rows_kernel<ACV, 2, NV, (NV > 1)>) \
-     : nper == 3 ? launch(trilinear_fwd_rows_kernel<ACV, 3, NV, (NV > 1)>) : launch(trilinear_fwd_rows_kernel<ACV, 4, NV, (NV > 1)>))
+    (nper == 1 ? launch(trilinear_fwd_rows_kernel<ACV, 1, NV, (NV > 1), D3>) : nper == 2 ? launch(trilinear_fwd_rows_kernel<ACV, 2, NV, (NV > 1), D3>) \
+     : nper == 3 ? launch(trilinear_fwd_rows_kernel<ACV, 3, NV, (NV > 1), D3>) : launch(trilinear_fwd_rows_kernel<ACV, 4, NV, (NV > 1), D3>))
+            // wider input rows (the cells' level-3 rows: 320 at 480x960, 416 at 384x1248) stay on the per-voxel kernel: row
+            // kernels with 3 and 4 input vectors per lane were measured no faster there (DESIGN.md 5.12)
             const bool one = Wi <= 128;
             rc = ac ? (one ? RAG_TRI_FWD(true, 1) : RAG_TRI_FWD(true, 2)) : (one ? RAG_TRI_FWD(false, 1) : RAG_TRI_FWD(false, 2));
 #undef RAG_TRI_FWD
             if (rc) return rc;
-            return check_launch("trilinear_resize_fwd(rows)");
+            return check_launch(D3 ? "trilinear_resize_fwd(rows)" : "bilinear_resize_fwd(rows)");
         }
     }
     const size_t n = (size_t)BC * Do * Ho * ((Wo + 3) / 4);
     const unsigned grid = (unsigned)std::min<size_t>((n + 255) / 256, (size_t)num_sms() * 32);
     const bool vec = Wo % 4 == 0 && aligned(out, 16);
-    if (ac) trilinear_fwd_kernel<true><<<grid, 256, 0, st>>>(in, out, BC, Di, Hi, Wi, Do, Ho, Wo, sd, sh, sw, vec);
-    else trilinear_fwd_kernel<false><<<grid, 256, 0, st>>>(in, out, BC, Di, Hi, Wi, Do, Ho, Wo, sd, sh, sw, vec);
-    return check_launch("trilinear_resize_fwd");
+    if (ac) trilinear_fwd_kernel<true, D3><<<grid, 256, 0, st>>>(in, out, BC, Di, Hi, Wi, Do, Ho, Wo, sd, sh, sw, vec);
+    else trilinear_fwd_kernel<false, D3><<<grid, 256, 0, st>>>(in, out, BC, Di, Hi, Wi, Do, Ho, Wo, sd, sh, sw, vec);
+    return check_launch(who);
 }
 
-int trilinear_resize_bwd(const float* gout, float* gin, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int align_corners, cudaStream_t st) {
-    if (int e = check_tri("trilinear_resize_bwd", gout, gin, BC, Di, Hi, Wi, Do, Ho, Wo)) return e;
+template <bool D3>
+static int resize_bwd(const char* who, const float* gout, float* gin, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int align_corners,
+                      cudaStream_t st) {
+    if (int e = check_tri(who, gout, gin, BC, Di, Hi, Wi, Do, Ho, Wo)) return e;
     const bool ac = align_corners != 0;
     const float sd = tri_scale(Di, Do, ac), sh = tri_scale(Hi, Ho, ac), sw = tri_scale(Wi, Wo, ac);
     const size_t smem = (size_t)(Do + Ho + Wo) * 8 + (size_t)(Di + Hi + Wi + 3) * 4;
@@ -500,28 +524,44 @@ int trilinear_resize_bwd(const float* gout, float* gin, int BC, int Di, int Hi, 
         auto launch = [&](auto kern) -> int {
             if (smem2 > 48 * 1024) {
                 cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-                if (e != cudaSuccess) return fail((int)e, "trilinear_resize_bwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+                if (e != cudaSuccess) return fail((int)e, "%s: cudaFuncSetAttribute: %s", who, cudaGetErrorString(e));
             }
             kern<<<grid, kTriWarps * 32, smem2, st>>>(gout, gin, BC, Di, Hi, Wi, Do, Ho, Wo, sd, sh, sw);
             return RAG_OK;
         };
         if (smem2 <= 160 * 1024) {
             int rc;
-            if (ac) rc = nper == 1 ? launch(trilinear_bwd_rows_kernel<true, 1>) : nper == 2 ? launch(trilinear_bwd_rows_kernel<true, 2>) : nper == 3 ? launch(trilinear_bwd_rows_kernel<true, 3>) : launch(trilinear_bwd_rows_kernel<true, 4>);
-            else rc = nper == 1 ? launch(trilinear_bwd_rows_kernel<false, 1>) : nper == 2 ? launch(trilinear_bwd_rows_kernel<false, 2>) : nper == 3 ? launch(trilinear_bwd_rows_kernel<false, 3>) : launch(trilinear_bwd_rows_kernel<false, 4>);
+            if (ac) rc = nper == 1 ? launch(trilinear_bwd_rows_kernel<true, 1, D3>) : nper == 2 ? launch(trilinear_bwd_rows_kernel<true, 2, D3>) : nper == 3 ? launch(trilinear_bwd_rows_kernel<true, 3, D3>) : launch(trilinear_bwd_rows_kernel<true, 4, D3>);
+            else rc = nper == 1 ? launch(trilinear_bwd_rows_kernel<false, 1, D3>) : nper == 2 ? launch(trilinear_bwd_rows_kernel<false, 2, D3>) : nper == 3 ? launch(trilinear_bwd_rows_kernel<false, 3, D3>) : launch(trilinear_bwd_rows_kernel<false, 4, D3>);
             if (rc) return rc;
-            return check_launch("trilinear_resize_bwd(rows)");
+            return check_launch(D3 ? "trilinear_resize_bwd(rows)" : "bilinear_resize_bwd(rows)");
         }
     }
     const size_t n = (size_t)BC * Di * Hi * Wi;
     const unsigned grid = (unsigned)std::min<size_t>((n + 255) / 256, (size_t)num_sms() * 16);
-    auto kern = ac ? trilinear_bwd_kernel<true> : trilinear_bwd_kernel<false>;
+    auto kern = ac ? trilinear_bwd_kernel<true, D3> : trilinear_bwd_kernel<false, D3>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return fail((int)e, "trilinear_resize_bwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+        if (e != cudaSuccess) return fail((int)e, "%s: cudaFuncSetAttribute: %s", who, cudaGetErrorString(e));
     }
     kern<<<grid, 256, smem, st>>>(gout, gin, BC, Di, Hi, Wi, Do, Ho, Wo, sd, sh, sw);
-    return check_launch("trilinear_resize_bwd");
+    return check_launch(who);
+}
+
+int trilinear_resize_fwd(const float* in, float* out, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int align_corners, cudaStream_t st) {
+    return resize_fwd<true>("trilinear_resize_fwd", in, out, BC, Di, Hi, Wi, Do, Ho, Wo, align_corners, st);
+}
+
+int trilinear_resize_bwd(const float* gout, float* gin, int BC, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int align_corners, cudaStream_t st) {
+    return resize_bwd<true>("trilinear_resize_bwd", gout, gin, BC, Di, Hi, Wi, Do, Ho, Wo, align_corners, st);
+}
+
+int bilinear_resize_fwd(const float* in, float* out, int BC, int Hi, int Wi, int Ho, int Wo, int align_corners, cudaStream_t st) {
+    return resize_fwd<false>("bilinear_resize_fwd", in, out, BC, 1, Hi, Wi, 1, Ho, Wo, align_corners, st);
+}
+
+int bilinear_resize_bwd(const float* gout, float* gin, int BC, int Hi, int Wi, int Ho, int Wo, int align_corners, cudaStream_t st) {
+    return resize_bwd<false>("bilinear_resize_bwd", gout, gin, BC, 1, Hi, Wi, 1, Ho, Wo, align_corners, st);
 }
 
 }  // namespace rag

@@ -79,7 +79,7 @@ def basic_network_forward(self, left, right, fea_ops, mat_ops):
 
 
 def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_stem: bool = False, upsample: bool = False,
-            matching_convs: bool = False, pointwise_convs: bool = False) -> dict:
+            matching_convs: bool = False, pointwise_convs: bool = False, resample: bool = False, resample_modules=()) -> dict:
     """Bind the B200 hot path onto the reference's modules (pass the imported module objects
     ``models.rag_model`` and/or ``automl.mdenas_basicmodel``).  Returns what was patched.
     New networks constructed afterwards get ``rag_b200.Disp``; existing instances keep working
@@ -109,7 +109,14 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
     ``pointwise_forward``: the Matching Net's pointwise ``ConvBR_3d(C, O, 1, 1, 0)`` layers (``last_12_3d``, ``last_6_3d``, the
     cells' 1x1x1 layers) that ``pointwise_conv.qualifies`` accepts run on csrc/conv3d_pw.cu in inference and training.  Every
     other call goes to the binding this call makes without the flag: ``matching_forward`` with ``matching_convs=True``,
-    else ``stem_forward``."""
+    else ``stem_forward``.
+
+    ``resample=True`` binds ``rag_b200.resample.FProxy()`` (``torch.nn.functional`` with ``interpolate`` replaced) as ``F`` in
+    ``rag_model``, if given, and in every module of ``resample_modules`` (for the search supernet's cells:
+    ``automl.build_model_2d`` and ``automl.build_model_3d``).  The cells' ``F.interpolate`` calls in ``bilinear`` (4-D) and
+    ``trilinear`` (5-D) mode then run on csrc/trilinear.cu, forward and fixed-order backward, so a training step runs
+    under ``torch.use_deterministic_algorithms(True)`` on the kernels; every other call is ``F.interpolate`` unchanged.  A
+    module without an ``F`` attribute raises ``ValueError``, as does the flag with no module to bind."""
     global _FUSE_STEM, _STEM_AWARE
     done = {}
 
@@ -153,6 +160,19 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
 
         bind(rag_model, "nn", NNProxy())        # `nn.Upsample(...)` inside matching() now resolves to rag_b200.upsample.Upsample
         done["rag_model"].append("nn.Upsample")
+    if resample:
+        targets = ([rag_model] if rag_model is not None else []) + list(resample_modules)
+        if not targets:
+            raise ValueError("resample=True needs rag_model or resample_modules (the reference modules whose F to bind)")
+        for mod in targets:                     # all checked before any is bound
+            if not hasattr(mod, "F"):
+                raise ValueError(f"resample=True: module {getattr(mod, '__name__', mod)!r} has no attribute F to bind")
+        from .resample import FProxy
+
+        proxy = FProxy()
+        for mod in targets:
+            bind(mod, "F", proxy)               # `F.interpolate(...)` inside the cells now resolves to rag_b200.resample.interpolate
+            done.setdefault("rag_model" if mod is rag_model else getattr(mod, "__name__", repr(mod)), []).append("F.interpolate")
     if mdenas_basicmodel is not None:
         bind(mdenas_basicmodel.BasicNetwork, "forward", basic_network_forward)
         bind(mdenas_basicmodel, "Disp", Disp)
