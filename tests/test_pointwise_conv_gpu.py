@@ -4,6 +4,7 @@ of the reference layer: Conv3d(C -> O, 1x1x1, bias=False) -> BatchNorm3d -> ReLU
 Tolerance: max-norm relative 1e-5 of fp64, the bar of tests/test_matching_conv_gpu.py (our kernels sum the C products of an
 output, and the weight gradient's voxels, in another order than cuDNN, all in fp32 with an fp64 final pass)."""
 import copy
+import zlib
 
 import pytest
 import torch
@@ -133,7 +134,7 @@ def test_training_vs_fp64(pair, shape, mode):
 
     c, o = pair
     b, d, h, w = shape
-    g = gen(hash((pair, shape, mode)) % 991)
+    g = gen(zlib.crc32(repr((pair, shape, mode)).encode()) % 991)      # not hash(): a str's hash changes from run to run
     layer = _layer(c, o, g).train(mode == "train")
     x0 = randn((b, c, d, h, w), g).cuda()
     gout = randn((b, o, d, h, w), g).cuda()
@@ -145,9 +146,10 @@ def test_training_vs_fp64(pair, shape, mode):
     assert not flips.any() or pre64.detach()[flips].abs().max().item() <= 1e-5, "ReLU decision differs from fp64 beyond rounding"
     names = ["out", "gx", "gweight", "ggamma", "gbeta", "running_mean", "running_var"]
     for n, a, r in zip(names, ours, ref64):
-        if n == "gweight" and c == 1 and mode == "train":
-            # one input channel under batch statistics: the layer is invariant to the weight's scale, the exact gradient is
-            # ~0 (eps alone keeps it off zero) and a relative error measures rounding; bound it by the summed |gz x| instead
+        if n == "gweight" and c == 1:
+            # one input channel: each weight's gradient is one dot product over all B*D*H*W voxels, so its relative error
+            # measures cancellation rather than the kernel (under batch statistics the layer is even invariant to the weight's
+            # scale: the exact gradient is ~0, eps alone keeps it off zero); bound it by the summed |gz x| instead
             lay64, x64 = copy.deepcopy(layer).double(), x0.double()
             z64 = lay64.conv(x64).detach().requires_grad_(True)
             (lay64.bn(z64) * mask.double()).backward(gout.double())

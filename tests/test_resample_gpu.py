@@ -1,14 +1,13 @@
 """The drop-in F.interpolate on the GPU (rag_b200/resample.py, csrc/trilinear.cu): bilinear and trilinear forward and
 fixed-order backward against ATen and fp64, repeatability, launch counts, CUDA-graph replay, the routing, and a training
 step of a network with the RAG structure under torch.use_deterministic_algorithms(True)."""
-import types
 from copy import deepcopy
 
 import pytest
 import torch
-import torch.nn as nn
 import torch.nn.functional as F
 
+from tests._stand_in import _stand_in
 from tests._util import gen, randn
 
 pytestmark = pytest.mark.gpu
@@ -151,132 +150,6 @@ def test_routing_on_the_device():
 # ---------------------------------------------------------------------------------------------------------------------
 # A training step under torch.use_deterministic_algorithms(True), on a stand-in with the RAG structure
 # ---------------------------------------------------------------------------------------------------------------------
-_OPS_3D = '''
-import torch.nn as nn
-import torch.nn.functional as F
-
-
-class ConvBR_3d(nn.Module):
-    """The reference's field layout (operations_3d.py): .conv, .bn, .use_bn, .relu."""
-
-    def __init__(self, c, o, k, s, p, bn=True, relu=True):
-        super().__init__()
-        self.conv = nn.Conv3d(c, o, k, stride=s, padding=p, bias=False)
-        self.use_bn = bn
-        self.bn = nn.BatchNorm3d(o) if bn else None
-        self.relu = relu
-
-    def forward(self, x):
-        x = self.conv(x)
-        if self.use_bn:
-            x = self.bn(x)
-        return F.relu(x, inplace=True) if self.relu else x
-'''
-
-_CELLS = '''
-import torch
-import torch.nn as nn
-import torch.nn.functional as F
-
-
-class Cell_2d(nn.Module):
-    """Feature-Net cell: a level-3 and a level-6 branch joined by bilinear resampling."""
-
-    def __init__(self, c):
-        super().__init__()
-        self.a = nn.Sequential(nn.Conv2d(c, c, 3, padding=1, bias=False), nn.BatchNorm2d(c), nn.ReLU())
-        self.b = nn.Sequential(nn.Conv2d(c, c, 3, padding=1, bias=False), nn.BatchNorm2d(c), nn.ReLU())
-        self.out = nn.Conv2d(2 * c, c, 1, bias=False)
-
-    def forward(self, x):
-        h, w = x.shape[2:]
-        s0 = self.a(x)
-        s1 = self.b(F.interpolate(s0, (h // 2, w // 2), mode="bilinear", align_corners=True))
-        s1 = F.interpolate(s1, (h, w), mode="bilinear", align_corners=True)
-        return self.out(torch.cat([s0, s0 + s1], 1))
-
-
-class Cell_3d(nn.Module):
-    """Matching-Net cell: a 1x1x1 preprocess, 3x3x3 ops, trilinear down- and up-sampling, step sums and a cat."""
-
-    def __init__(self, c, k):
-        super().__init__()
-        self.pre = ConvBR_3d(c, k, 1, 1, 0)
-        self.op0 = ConvBR_3d(k, k, 3, 1, 1)
-        self.op1 = ConvBR_3d(k, k, 3, 1, 1)
-        self.op2 = ConvBR_3d(k, k, 3, 1, 1)
-
-    def forward(self, x):
-        d, h, w = x.shape[2:]
-        s0 = self.pre(x)
-        s1 = self.op0(s0)
-        low = self.op1(F.interpolate(s1, [d // 2, h // 2, w // 2], mode="trilinear", align_corners=True))
-        s2 = self.op2(s0 + s1) + F.interpolate(low, [d, h, w], mode="trilinear", align_corners=True)
-        return torch.cat([s0, s1, s2], 1), low
-'''
-
-_RAG_MODEL = '''
-import torch.nn as nn
-import torch.nn.functional as F
-
-
-class Disp(nn.Module):
-    def __init__(self, maxdisp):
-        super().__init__()
-        self.maxdisp = maxdisp
-
-
-class DisparityRegression(nn.Module):
-    pass
-
-
-class Network(nn.Module):
-    """The growable network's structure: feature net (stem + a 2-D cell), cost volume, matching net (stem3d0/1, a 3-D cell,
-    last_6_3d, upsample_6, last_3_3d) and the head; forward / search_forward are bound by install()."""
-
-    def __init__(self, maxdisp=48, c=12, k=4):
-        super().__init__()
-        self.maxdisp = maxdisp
-        self.stem2d = nn.Sequential(nn.Conv2d(3, c, 3, stride=3, bias=False), nn.BatchNorm2d(c), nn.ReLU())
-        self.cell2d = cells.Cell_2d(c)
-        self.stem3d0 = ConvBR_3d(2 * c, c, 3, 1, 1)
-        self.stem3d1 = ConvBR_3d(c, c, 3, 1, 1)
-        self.cell3d = cells.Cell_3d(c, k)
-        self.last_6_3d = ConvBR_3d(k, 3 * k, 1, 1, 0)
-        self.last_3_3d = ConvBR_3d(3 * k, 1, 3, 1, 1, bn=False, relu=False)
-        self.disp = Disp(maxdisp)
-
-    def feature(self, x, task_arch=None, path=None):
-        return self.cell2d(self.stem2d(x))
-
-    def matching(self, cost, task_arch=None, path=None):
-        x = self.stem3d1(self.stem3d0(cost))
-        x3, x6 = self.cell3d(x)
-        upsample_6 = nn.Upsample(size=x3.size()[2:], mode="trilinear", align_corners=True)
-        return self.last_3_3d(x3 + upsample_6(self.last_6_3d(x6)))
-
-    def forward(self, *a):
-        raise NotImplementedError("bound by rag_b200.network.install")
-
-    def search_forward(self, *a):
-        raise NotImplementedError("bound by rag_b200.network.install")
-'''
-
-
-def _module(name, src, **inject):
-    m = types.ModuleType(name)
-    m.__dict__.update(inject)
-    exec(compile(src, f"<stand-in {name}>", "exec"), m.__dict__)
-    return m
-
-
-def _stand_in():
-    ops3d = _module("automl.operations_3d", _OPS_3D)
-    cells = _module("automl.build_model_3d", _CELLS, ConvBR_3d=ops3d.ConvBR_3d)
-    rag_model = _module("models.rag_model", _RAG_MODEL, ConvBR_3d=ops3d.ConvBR_3d, cells=cells)
-    return rag_model, ops3d, cells
-
-
 class _CountDecomposition:
     """Counts the calls F.interpolate makes, under deterministic mode, into torch's linear-mode decomposition."""
 
