@@ -19,6 +19,7 @@ import pytest
 import torch
 
 from oracle import rag_oracle as O
+from tests import _grids
 from tests._util import gen, maxnorm_rel, randn, sparse_grad
 
 pytestmark = pytest.mark.gpu
@@ -305,6 +306,16 @@ def test_forward_and_backward_parity_at_baseline_sizes(F_, size):
     assert frac >= 0.999
     assert worst["grad"] <= TOL_GRAD
     assert maxnorm_rel(co.grad.cpu().numpy(), gref.cpu().numpy()) <= 2 * TOL_GRAD
+    # the persistent variants of the co-resident training schedule (RAG_HEAD_FWD_SHARED, RAG_HEAD_BWD_SHARED) loop over tiles /
+    # CTA-tasks at these sizes; every tile is independent and the backward adds two commutative contributions per element
+    # into a zeroed buffer, so they give the default grids' bits
+    fwd_span = _grids.loops(*_grids.head_fwd(b, hl, wl, cost.device))
+    bwd_span = _grids.loops(*_grids.head_bwd(b, dl, hl, wl, cost.device))
+    print(f"persistent forward: {fwd_span}; persistent backward: {bwd_span}")
+    disp, stats = F_.disp_head_forward(cost, md, want_stats=True)
+    disp4, stats4 = F_.disp_head_forward(cost, md, want_stats=True, variant=4)
+    assert torch.equal(disp, out.detach()) and torch.equal(disp4, disp) and torch.equal(stats4, stats)
+    assert torch.equal(F_.disp_head_backward(cost, gd, disp4, stats4, md, variant=3), co.grad)
 
 
 def test_module_hygiene(F_):

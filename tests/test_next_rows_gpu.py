@@ -8,6 +8,7 @@ import torch
 import torch.nn.functional as F
 
 from oracle import rag_oracle as O
+from tests import _grids
 from tests._mirror_net import MirrorNet, arch
 from tests._util import gen, randn
 
@@ -212,25 +213,35 @@ def test_host_train_pipeline_matches_the_functions(dev):
     assert np.array_equal(r["gx"].numpy(), gx_ref) and np.array_equal(r["gy"].numpy(), gy_ref)
 
 
-@pytest.mark.parametrize("schedule", ["launch-order", "coresident", "slim-volume"])
-def test_overlapped_train_path_matches_the_serial_functions(dev, schedule):
+# (id prefix, (B, C, Hf, Wf, maxdisp, steps)).  The small shape gives every persistent CTA at most one item; at the bench's
+# training shape (B=4 288x576) the co-resident head kernels loop over tiles / CTA-tasks (fewer steps there bound the memory)
+OVERLAP_SHAPES = [("", (2, 12, 9, 64, 96, 10)), ("B4-288x576-", (4, 12, 96, 192, 192, 3))]
+OVERLAP_CASES = [(p, s, k) for p, s in OVERLAP_SHAPES for k in ("launch-order", "coresident", "slim-volume")]
+
+
+@pytest.mark.parametrize("shape, schedule", [(s, k) for _, s, k in OVERLAP_CASES], ids=[p + k for p, _, k in OVERLAP_CASES])
+def test_overlapped_train_path_matches_the_serial_functions(dev, shape, schedule):
     """Every schedule of the two-stream training step (rag_b200.pipeline.SCHEDULES: persistent / co-resident kernel
     variants) gives the bits of the plain serial calls."""
     from rag_b200 import functional as F_
     from rag_b200.pipeline import OverlappedTrainPath
 
+    b, c, hf, wf, md, steps = shape
+    dl = md // 3
+    if shape == OVERLAP_SHAPES[1][1]:
+        print(f"\npersistent head forward: {_grids.loops(*_grids.head_fwd(b, hf, wf, dev))}; "
+              f"backward: {_grids.loops(*_grids.head_bwd(b, dl, hf, wf, dev))}")
     g = gen(37)
-    md = 96
     op = OverlappedTrainPath(md, dev, schedule=schedule)
-    x, y = randn((2, 12, 9, 64), g).to(dev), randn((2, 12, 9, 64), g).to(dev)
-    cl = randn((2, 1, 32, 9, 64), g).to(dev)
-    gd = randn((2, 27, 192), g).to(dev)
-    gcost = randn((2, 24, 32, 9, 64), g).to(dev)
-    outs = [op.step(x, y, cl, gcost, gd) for _ in range(10)]
+    x, y = randn((b, c, hf, wf), g).to(dev), randn((b, c, hf, wf), g).to(dev)
+    cl = randn((b, 1, dl, hf, wf), g).to(dev)
+    gd = randn((b, 3 * hf, 3 * wf), g).to(dev)
+    gcost = randn((b, 2 * c, dl, hf, wf), g).to(dev)
+    outs = [op.step(x, y, cl, gcost, gd) for _ in range(steps)]
     op.join()
     torch.cuda.synchronize()
     disp, stats = F_.disp_head_forward(cl, md, True)
-    want = (F_.cost_volume_forward(x, y, md // 3, variant=0), disp, F_.disp_head_backward(cl, gd, disp, stats, md)) + F_.cost_volume_backward(gcost, 12, variant=1)
+    want = (F_.cost_volume_forward(x, y, md // 3, variant=0), disp, F_.disp_head_backward(cl, gd, disp, stats, md)) + F_.cost_volume_backward(gcost, c, variant=1)
     for o in outs:
         for a, b_ in zip(o, want):
             assert torch.equal(a, b_)
