@@ -313,6 +313,30 @@ RAG_API int rag_bilinear_resize_fwd(const float* in, float* out, int BC, int Hi,
 RAG_API int rag_bilinear_resize_bwd(const float* gout, float* gin, int BC, int Hi, int Wi, int Ho, int Wo, int align_corners,
                             void* stream);
 
+/* 4-D bilinear grid sampling: F.grid_sample(input, grid, mode='bilinear', padding_mode=..., align_corners=...), the warp that
+ * synthesises one view from the other and a predicted disparity in the self-supervised loss (src_self/models/loss.py; that the
+ * warp is F.grid_sample is inferred, the reference's loss is unread).  Contract: ATen's grid_sampler_2d with its fp32 index
+ * arithmetic (csrc/grid_sample.cu states it).  in [N,C,Hi,Wi]; grid [N,Ho,Wo,2] (x, y in [-1, 1]); out [N,C,Ho,Wo].
+ * padding_mode: 0 = 'zeros', 1 = 'border' (anything else RAG_E_SHAPE); align_corners: 0 / 1.  grid and ggrid 8-byte aligned.
+ * Sizes: 4*N*Ho*Wo, N*Hi*Wi, N*C*Hi*Wi and N*C*Ho*Wo must be below 2^31 (RAG_E_SHAPE, checked on the host).  A grid value of
+ * any size, NaN or infinite, reads nothing out of bounds.  Stateless and capturable.
+ * rag_grid_sample_bwd, from gout [N,C,Ho,Wo]:
+ *   ggrid [N,Ho,Wo,2] (nullable; needs in): ATen's grid gradient, per sample over the channels in ascending order;
+ *   gin [N,C,Hi,Wi] (nullable; needs workspace): gin[n,c,y,x] = sum of w * gout[n,c,ho,wo] over every (sample, corner) that reads
+ *     (y, x), in ascending flat sample index (n*Ho + ho)*Wo + wo and within a sample in the corner order nw, ne, sw, se --
+ *     a fixed order, so the result is bitwise repeatable (ATen's backward adds with atomicAdd in arrival order).  No float atomics.
+ * workspace: caller-owned DEVICE buffer of rag_grid_sample_bwd_workspace_bytes(N,C,Hi,Wi,Ho,Wo) bytes (0 = outside the limits),
+ *   256-byte aligned, contents undefined on return; workspace_bytes is its size (a smaller one is RAG_E_SHAPE).  It holds 20 bytes
+ *   per sample-corner (4*N*Ho*Wo of them: sort keys and values, each double-buffered, and a weight), 8 bytes per input pixel
+ *   (N*Hi*Wi segment bounds) and the radix sort's own storage (a few KB); each region rounded up to 256 bytes.  The query needs
+ *   no device.  Not needed (may be NULL) when gin is NULL. */
+RAG_API int rag_grid_sample_fwd(const float* in, const float* grid, float* out, int N, int C, int Hi, int Wi, int Ho, int Wo,
+                        int padding_mode, int align_corners, void* stream);
+RAG_API size_t rag_grid_sample_bwd_workspace_bytes(int N, int C, int Hi, int Wi, int Ho, int Wo);
+RAG_API int rag_grid_sample_bwd(const float* gout, const float* in, const float* grid, float* gin, float* ggrid, void* workspace,
+                        size_t workspace_bytes, int N, int C, int Hi, int Wi, int Ho, int Wo, int padding_mode, int align_corners,
+                        void* stream);
+
 /* Eval-time input staging: uint8 HWC image -> ImageNet-normalised fp32 CHW, zero-padded on the
  * top and right.  Replaces src/dataloaders/data_io.py:6-13 + stereo_dataset.py:88-102.
  * img [B,H,W,3] uint8; out [B,3,H+top_pad,W+right_pad] fp32. */

@@ -65,6 +65,9 @@ SIGNATURES = {
     "rag_trilinear_resize_bwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_bilinear_resize_fwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_bilinear_resize_bwd": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "rag_grid_sample_fwd": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
+    "rag_grid_sample_bwd_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i, _i]),
+    "rag_grid_sample_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, C.c_size_t, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_normalize_pad": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp]),
 }
 

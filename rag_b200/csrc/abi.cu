@@ -40,6 +40,9 @@ int conv3d_cc_bwd(const float*, const float*, const float*, float*, float*, floa
 int conv3d_pw_fwd(const float*, const float*, const float*, const float*, int, float*, int, int, int, int, int, int, cudaStream_t);
 size_t conv3d_pw_bwd_workspace_bytes(int, int, int, int, int, int);
 int conv3d_pw_bwd(const float*, const float*, const float*, const float*, const float*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
+int grid_sample_fwd(const float*, const float*, float*, int, int, int, int, int, int, int, int, cudaStream_t);
+size_t grid_sample_bwd_workspace_bytes(int, int, int, int, int, int);
+int grid_sample_bwd(const float*, const float*, const float*, float*, float*, void*, size_t, int, int, int, int, int, int, int, int, cudaStream_t);
 }  // namespace rag
 
 using namespace rag;
@@ -180,6 +183,18 @@ RAG_API int rag_bilinear_resize_fwd(const float* in, float* out, int BC, int Hi,
 }
 RAG_API int rag_bilinear_resize_bwd(const float* gout, float* gin, int BC, int Hi, int Wi, int Ho, int Wo, int align_corners, void* stream) {
     return bilinear_resize_bwd(gout, gin, BC, Hi, Wi, Ho, Wo, align_corners, ST(stream));
+}
+RAG_API int rag_grid_sample_fwd(const float* in, const float* grid, float* out, int N, int C, int Hi, int Wi, int Ho, int Wo,
+                        int padding_mode, int align_corners, void* stream) {
+    return grid_sample_fwd(in, grid, out, N, C, Hi, Wi, Ho, Wo, padding_mode, align_corners, ST(stream));
+}
+RAG_API size_t rag_grid_sample_bwd_workspace_bytes(int N, int C, int Hi, int Wi, int Ho, int Wo) {
+    return grid_sample_bwd_workspace_bytes(N, C, Hi, Wi, Ho, Wo);
+}
+RAG_API int rag_grid_sample_bwd(const float* gout, const float* in, const float* grid, float* gin, float* ggrid, void* workspace,
+                        size_t workspace_bytes, int N, int C, int Hi, int Wi, int Ho, int Wo, int padding_mode, int align_corners,
+                        void* stream) {
+    return grid_sample_bwd(gout, in, grid, gin, ggrid, workspace, workspace_bytes, N, C, Hi, Wi, Ho, Wo, padding_mode, align_corners, ST(stream));
 }
 RAG_API int rag_normalize_pad(const uint8_t* img, float* out, int B, int H, int W, int top_pad, int right_pad, void* stream) {
     return normalize_pad(img, out, B, H, W, top_pad, right_pad, ST(stream));

@@ -79,7 +79,8 @@ def basic_network_forward(self, left, right, fea_ops, mat_ops):
 
 
 def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_stem: bool = False, upsample: bool = False,
-            matching_convs: bool = False, pointwise_convs: bool = False, resample: bool = False, resample_modules=()) -> dict:
+            matching_convs: bool = False, pointwise_convs: bool = False, resample: bool = False, resample_modules=(),
+            grid_sample: bool = False, grid_sample_modules=()) -> dict:
     """Bind the B200 hot path onto the reference's modules (pass the imported module objects
     ``models.rag_model`` and/or ``automl.mdenas_basicmodel``).  Returns what was patched.
     New networks constructed afterwards get ``rag_b200.Disp``; existing instances keep working
@@ -116,7 +117,16 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
     ``automl.build_model_2d`` and ``automl.build_model_3d``).  The cells' ``F.interpolate`` calls in ``bilinear`` (4-D) and
     ``trilinear`` (5-D) mode then run on csrc/trilinear.cu, forward and fixed-order backward, so a training step runs
     under ``torch.use_deterministic_algorithms(True)`` on the kernels; every other call is ``F.interpolate`` unchanged.  A
-    module without an ``F`` attribute raises ``ValueError``, as does the flag with no module to bind."""
+    module without an ``F`` attribute raises ``ValueError``, as does the flag with no module to bind.
+
+    ``grid_sample=True`` binds ``rag_b200.grid_sample.GridSampleProxy(module.F)`` as ``F`` in every module of
+    ``grid_sample_modules`` (the self-supervised variant's loss module, ``models.loss`` of ``src_self``).  Its
+    ``F.grid_sample`` calls that ``grid_sample.routes`` accepts (4-D bilinear, zeros or border padding, CUDA fp32) then run on
+    csrc/grid_sample.cu, forward and fixed-order backward, so the warp of the self-supervised loss runs under
+    ``torch.use_deterministic_algorithms(True)``; every other call is ``F.grid_sample`` unchanged.  The proxy wraps the module's
+    current ``F``, so a module bound by ``resample=True`` keeps its ``interpolate``, in either order of the two flags, and a
+    module already holding a ``GridSampleProxy`` is not wrapped again.  A module without ``F`` raises ``ValueError``, as does
+    the flag with no module; all modules are checked before any is bound."""
     global _FUSE_STEM, _STEM_AWARE
     done = {}
 
@@ -167,12 +177,28 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
         for mod in targets:                     # all checked before any is bound
             if not hasattr(mod, "F"):
                 raise ValueError(f"resample=True: module {getattr(mod, '__name__', mod)!r} has no attribute F to bind")
+        from .grid_sample import GridSampleProxy
         from .resample import FProxy
 
         proxy = FProxy()
-        for mod in targets:
-            bind(mod, "F", proxy)               # `F.interpolate(...)` inside the cells now resolves to rag_b200.resample.interpolate
+        for mod in targets:                     # `F.interpolate(...)` inside the cells now resolves to rag_b200.resample.interpolate
+            bind(mod, "F", GridSampleProxy(proxy) if isinstance(mod.F, GridSampleProxy) else proxy)   # keeps an earlier grid_sample=True
             done.setdefault("rag_model" if mod is rag_model else getattr(mod, "__name__", repr(mod)), []).append("F.interpolate")
+    if grid_sample:
+        targets = list(grid_sample_modules)
+        if not targets:
+            raise ValueError("grid_sample=True needs grid_sample_modules (the reference modules whose F to bind, e.g. src_self's models.loss)")
+        for mod in targets:                     # all checked before any is bound
+            if not hasattr(mod, "F"):
+                raise ValueError(f"grid_sample=True: module {getattr(mod, '__name__', mod)!r} has no attribute F to bind")
+        from .grid_sample import GridSampleProxy
+
+        for mod in targets:
+            if not isinstance(mod.F, GridSampleProxy):
+                bind(mod, "F", GridSampleProxy(mod.F))   # `F.grid_sample(...)` now resolves to rag_b200.grid_sample.grid_sample
+            key = "rag_model" if mod is rag_model else getattr(mod, "__name__", repr(mod))
+            if "F.grid_sample" not in done.setdefault(key, []):
+                done[key].append("F.grid_sample")
     if mdenas_basicmodel is not None:
         bind(mdenas_basicmodel.BasicNetwork, "forward", basic_network_forward)
         bind(mdenas_basicmodel, "Disp", Disp)
