@@ -18,16 +18,21 @@ __device__ __forceinline__ double warp_sum(double v) {
 }
 
 // rows[B,H,O,2] fp64 = per (b,o,h) row (sum z, sum z^2).  grid (H, O, B), 256 threads; W % 4 == 0.
+// The fp32 part (four elements at a time) works on z - k, k = the row's first element: var = E[z^2] - mean^2 cancels all but
+// a std^2/mean^2 share of the fp32 partials of z^2 itself, so their rounding would reach the variance magnified (mean/std)^2
+// times.  The row's raw sums are restored in fp64, where that cancellation is harmless.
 __global__ void __launch_bounds__(256)
 bn3d_moments_rows_kernel(const float* __restrict__ z, double* __restrict__ rows, int O, int D, int H, int W) {
     const int h = blockIdx.x, o = blockIdx.y, b = blockIdx.z, tid = threadIdx.x;
     const int Wv = W >> 2;
     const size_t plane = (size_t)H * W;
     const size_t base = ((size_t)(b * O + o) * D) * plane + (size_t)h * W;
+    const float k = __ldg(z + base);
     double s0 = 0.0, s1 = 0.0;
     for (int i = tid; i < D * Wv; i += 256) {
         const int d = i / Wv, v = i - d * Wv;
-        const float4 zv = __ldg(reinterpret_cast<const float4*>(z + base + (size_t)d * plane + 4 * v));   // just written: L2
+        float4 zv = __ldg(reinterpret_cast<const float4*>(z + base + (size_t)d * plane + 4 * v));   // just written: L2
+        zv.x -= k; zv.y -= k; zv.z -= k; zv.w -= k;
         const float a = (zv.x + zv.y) + (zv.z + zv.w);
         const float q = __fmaf_rn(zv.x, zv.x, zv.y * zv.y) + __fmaf_rn(zv.z, zv.z, zv.w * zv.w);
         s0 += (double)a;
@@ -41,8 +46,9 @@ bn3d_moments_rows_kernel(const float* __restrict__ z, double* __restrict__ rows,
         double a0 = 0.0, a1 = 0.0;
 #pragma unroll
         for (int i = 0; i < 8; ++i) { a0 += red[0][i]; a1 += red[1][i]; }
+        const double kd = (double)k, m = (double)D * W;       // sum z = a0 + m k, sum z^2 = a1 + 2 k a0 + m k^2
         double* r = rows + ((size_t)(b * H + h) * O + o) * 2;
-        r[0] = a0; r[1] = a1;
+        r[0] = a0 + m * kd; r[1] = a1 + kd * (2.0 * a0 + m * kd);
     }
 }
 

@@ -395,12 +395,12 @@ int cv_stem_bwd(const float* g, const float* out, const float* consts, const flo
     {
         const int nt = ((Wf + 4 + 31) / 32) * 32;
         const int U = Df % 8 == 0 ? 8 : Df % 4 == 0 ? 4 : Df % 2 == 0 ? 2 : 1;   // rows per batch: must divide Df
-        const size_t smem = ((size_t)2 * U + 5) * Wf * sizeof(float);
-        if (U == 8) stem_bwd_maps_kernel<8><<<dim3(Hf, O, B), nt, smem, st>>>(g, out, consts, tmap, umap, O, Df, Hf, Wf);
-        else if (U == 4) stem_bwd_maps_kernel<4><<<dim3(Hf, O, B), nt, smem, st>>>(g, out, consts, tmap, umap, O, Df, Hf, Wf);
-        else if (U == 2) stem_bwd_maps_kernel<2><<<dim3(Hf, O, B), nt, smem, st>>>(g, out, consts, tmap, umap, O, Df, Hf, Wf);
-        else stem_bwd_maps_kernel<1><<<dim3(Hf, O, B), nt, smem, st>>>(g, out, consts, tmap, umap, O, Df, Hf, Wf);
-        if (int e = check_launch("cv_stem_bwd(maps)")) return e;
+        const size_t smem = ((size_t)2 * U + 5) * Wf * sizeof(float);   // up to 85,344 bytes (Wf = 1016, U = 8): past the 48 KB default
+        auto kern = U == 8 ? stem_bwd_maps_kernel<8> : U == 4 ? stem_bwd_maps_kernel<4> : U == 2 ? stem_bwd_maps_kernel<2> : stem_bwd_maps_kernel<1>;
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return fail((int)e, "cv_stem_bwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+        kern<<<dim3(Hf, O, B), nt, smem, st>>>(g, out, consts, tmap, umap, O, Df, Hf, Wf);
+        if (int rc = check_launch("cv_stem_bwd(maps)")) return rc;
     }
     const int R = 9 * O, Rp = (R + 3) & ~3;
     if (gx) {
