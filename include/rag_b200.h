@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define RAG_B200_ABI_VERSION 17
+#define RAG_B200_ABI_VERSION 18
 
 #if defined(__GNUC__)
 #define RAG_API __attribute__((visibility("default")))
@@ -113,20 +113,21 @@ RAG_API int rag_upsample_trilinear(const float* cost_lr, float* out, int B, int 
                            int maxdisp, int fma_index, void* stream);
 
 /* ---- variants (A/B measurement and fallbacks; the functions above pick the default) ----------
- * Variant ids (-1 = the default; ids outside a range return RAG_E_VARIANT):
+ * Variant ids (-1 = the default; any other id not listed here returns RAG_E_VARIANT):
  *   rag_cost_volume_fwd_v  0 = any width / alignment (items dealt to threads); 1 = lean thread-stationary kernel, one CTA
- *                          per item (default without a workspace when Wf % 4 == 0); 2 = lean persistent, 256 threads x 2
- *                          vectors, one CTA per SM; 3 = lean persistent, 512 threads (SM sharing, launch order);
- *                          4 = TMA bulk-store kernel (cp.async.bulk shared->global); 5 = lean persistent, 256 threads x 1
- *                          vector at 48 registers, 32 disparities per item (default with a workspace; co-resident SM
- *                          sharing).  2-5 need the workspace.
+ *                          per item (default without a workspace when Wf % 4 == 0); 3 = lean persistent, 512 threads (SM
+ *                          sharing, launch order); 5 = lean persistent, 256 threads x 1 vector at 48 registers, 32
+ *                          disparities per item (default with a workspace; co-resident SM sharing).  3 and 5 need the
+ *                          workspace.  Ids 2 (lean persistent, 256 threads x 2 vectors) and 4 (TMA bulk-store kernel) were
+ *                          retired in ABI version 18: slower than 5 on every measured shape.
  *   rag_cost_volume_bwd_v  0 = 128-bit vector kernel (default when Wf % 4 == 0), 1 = scalar (any width),
  *                          2 = the vector kernel as a persistent grid of 4 CTAs per SM (SM sharing, launch order);
  *                          3 = cp.async ring in shared memory, one 256-thread CTA per SM at 64 registers (co-resident SM
  *                          sharing)
  *   rag_disp_head_fwd_v    0 = any (Dl, maxdisp); 1 = first x3 kernel (any width); 2 = cube-root tiled kernel (default when
- *                          maxdisp == 3*Dl and Wl % 4 == 0); 3 = as 2 with the lambda correction at every step + TwoSum totals;
- *                          4 = 2 as a persistent grid of 3 CTAs per SM (co-resident SM sharing)
+ *                          maxdisp == 3*Dl and Wl % 4 == 0); 4 = 2 as a persistent grid of 3 CTAs per SM (co-resident SM
+ *                          sharing).  Id 3 (2 with the lambda correction at every step + TwoSum totals) was retired in ABI
+ *                          version 18.
  *   rag_disp_head_bwd_v    0 = any-ratio gather; 1 = block-row tasks, parts added in place (default when maxdisp == 3*Dl);
  *                          2 = same with scratch + combine kernel; 3 = 1 as a persistent grid of 3 CTAs per SM (co-resident)
  *   rag_cv_stem_fwd_v      0 = direct (any shape); 1 = collapsed, scalar; 2 = default (packed phase 1)
@@ -139,7 +140,6 @@ RAG_API int rag_upsample_trilinear(const float* cost_lr, float* out, int B, int 
  *    x 48 registers; RAG_CV_BWD_SLIM: 256 threads x 64 registers, its ~96 KB of in-flight reads parked in SHARED memory by
  *    cp.async instead of in registers), three 128-thread x 128-register head CTAs in the rest (RAG_HEAD_FWD_SHARED,
  *    RAG_HEAD_BWD_SHARED) -- so they overlap whichever is launched first.  Every variant gives the same bits as the default. */
-#define RAG_CV_FWD_LEAN 2     /* persistent, one 256-thread CTA per SM, 2 vectors per thread (the default of round 1) */
 #define RAG_CV_FWD_SHARED 3   /* same kernel, one 512-thread CTA per SM: best when launched before the head forward */
 #define RAG_CV_FWD_SLIM 5     /* default with a workspace: 256 threads x 1 vector, 32 disparities per item -- a quarter of
                                * the register file (co-resident SM sharing) and the fastest geometry alone as well    */

@@ -12,7 +12,7 @@ import os
 
 from . import build as _build
 
-ABI_VERSION = 17
+ABI_VERSION = 18
 
 _f = C.POINTER(C.c_float)
 _d = C.POINTER(C.c_double)

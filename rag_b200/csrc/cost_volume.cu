@@ -21,7 +21,6 @@
 #include <algorithm>
 
 #include "common.cuh"
-#include "cv_tma.cuh"
 #include "cv_lean.cuh"
 
 namespace rag {
@@ -437,11 +436,11 @@ static int arm_counter(void* workspace, cudaStream_t st, const char* who) {
     return RAG_OK;
 }
 
-// lean thread-stationary kernel.  ctr == nullptr: one CTA per item (hardware dispatch order keeps the resident
-// CTAs on neighbouring rows; stateless).  ctr != nullptr: persistent grid of `per_sm` CTAs per SM that takes its
-// items IN ORDER from the caller's counter (3 % faster at B=8 480x960, and resident at once, which is what lets the
+// lean thread-stationary kernel.  !DYN: one CTA per item (hardware dispatch order keeps the resident CTAs on
+// neighbouring rows; stateless; ctr unused).  DYN: persistent grid of `per_sm` CTAs per SM that takes its items IN
+// ORDER from the caller's counter `ctr` (3 % faster at B=8 480x960, and resident at once, which is what lets the
 // disparity head share the SMs on a second stream).
-template <int NT, int VPT>
+template <int NT, int VPT, bool DYN>
 static int launch_cv_fwd_lean(const float* x, const float* y, float* cost, int B, int C, int Df, int Hf, int Wf,
                               int per_sm, unsigned int* ctr, cudaStream_t st, int dchunk_max = 16) {
     const int Wv = Wf / 4, Df4 = (Df + 3) & ~3;
@@ -451,8 +450,7 @@ static int launch_cv_fwd_lean(const float* x, const float* y, float* cost, int B
     while (R > 1 && R * row_bytes > 64 * 1024) --R;
     const size_t smem = R * row_bytes;
     if (smem > 200 * 1024) return fail(RAG_E_SHAPE, "cost_volume_fwd(lean): Df=%d Wf=%d do not fit shared memory", Df, Wf);
-    const bool dyn = ctr != nullptr;
-    auto kern = dyn ? cv_fwd_lean_kernel<NT, VPT, true> : cv_fwd_lean_kernel<NT, VPT, false>;
+    auto kern = cv_fwd_lean_kernel<NT, VPT, DYN>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     // the L1/shared split of an SM cannot change while CTAs are resident: ask for the largest shared-memory
     // carve-out so that this kernel and the disparity head (which does the same) can share an SM
@@ -463,62 +461,31 @@ static int launch_cv_fwd_lean(const float* x, const float* y, float* cost, int B
     const int n_dchunks = (Df + dchunk - 1) / dchunk;
     const long long n_items = (long long)B * C * n_tiles * n_dchunks;
     if (n_items >= (1LL << 31)) return fail(RAG_E_SHAPE, "cost_volume_fwd(lean): too many work items");
-    const int grid = (int)(dyn ? std::min<long long>(n_items, (long long)num_sms() * per_sm) : n_items);
-    if (dyn) if (int rc = arm_counter(ctr, st, "cost_volume_fwd(lean)")) return rc;
+    const int grid = (int)(DYN ? std::min<long long>(n_items, (long long)num_sms() * per_sm) : n_items);
+    if (DYN) if (int rc = arm_counter(ctr, st, "cost_volume_fwd(lean)")) return rc;
     kern<<<grid, NT, smem, st>>>(x, y, cost, B * C, C, Df, Hf, Wf, R, n_tiles, dchunk, n_dchunks, ctr);
     return check_launch("cost_volume_fwd(lean)");
 }
 
-static bool cv_tma_ok(const float* x, const float* y, const float* cost, int Df, int Wf) {
-    return Wf % 4 == 0 && Df % 4 == 0 && Df <= Wf && aligned(x, 16) && aligned(y, 16) && aligned(cost, 16);
-}
-
-static int launch_cv_fwd_tma(const float* x, const float* y, float* cost, int B, int C, int Df, int Hf, int Wf,
-                             unsigned int* ctr, cudaStream_t st) {
-    constexpr int NT = 128;
-    int R = std::min(4, Hf);
-    const int per_sm = 2;
-    const size_t row_floats = (size_t)Wf + 4 * (size_t)(Df + Wf + 4);
-    while (R > 1 && 4 * (Df + 2 * R * row_floats) > 200 * 1024) --R;
-    const size_t smem = 4 * (Df + 2 * R * row_floats);
-    if (smem > 200 * 1024) return fail(RAG_E_SHAPE, "cost_volume_fwd(tma): Wf=%d too wide for shared memory", Wf);
-    auto kern = cv_fwd_tma_kernel<NT>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return fail((int)e, "cost_volume_fwd(tma): cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    const int n_tiles = (Hf + R - 1) / R;
-    const int dchunk = std::min(16, Df), n_dchunks = (Df + dchunk - 1) / dchunk;
-    const long long n_items = (long long)B * C * n_tiles * n_dchunks;
-    if (n_items >= (1LL << 31)) return fail(RAG_E_SHAPE, "cost_volume_fwd(tma): too many work items");
-    const int grid = (int)std::min<long long>(n_items, (long long)num_sms() * per_sm);
-    if (int rc = arm_counter(ctr, st, "cost_volume_fwd(tma)")) return rc;
-    kern<<<grid, NT, smem, st>>>(x, y, cost, B, C, Df, Hf, Wf, R, n_tiles, dchunk, n_dchunks, ctr);
-    return check_launch("cost_volume_fwd(tma)");
-}
-
 // variant: -1 = default (lean persistent (variant 5) when a workspace is given, lean one-CTA-per-item without, generic when the
-// lean preconditions fail); 0 = generic; 1 = lean one CTA per item; 2 = lean persistent 256 threads (needs workspace);
-// 3 = lean persistent 512 threads, RAG_CV_FWD_SHARED (needs workspace); 4 = TMA bulk-store kernel (needs workspace);
-// 5 = lean persistent 256 threads x 1 vector, RAG_CV_FWD_SLIM (needs workspace)
+// lean preconditions fail); 0 = generic; 1 = lean one CTA per item; 3 = lean persistent 512 threads, RAG_CV_FWD_SHARED (needs
+// workspace); 5 = lean persistent 256 threads x 1 vector, RAG_CV_FWD_SLIM (needs workspace).  Ids 2 (lean persistent 256
+// threads x 2 vectors) and 4 (TMA bulk stores) were retired: slower than 5 on every measured shape (DESIGN.md section 5.1).
 int cost_volume_fwd(const float* x, const float* y, float* cost, int B, int C, int Df, int Hf, int Wf,
                     void* workspace, int variant, cudaStream_t st) {
     if (int e = check_cv_args(x, y, cost, B, C, Df, Hf, Wf)) return e;
-    if (variant < -1 || variant > 5) return fail(RAG_E_VARIANT, "cost_volume_fwd: unknown variant %d", variant);
+    if (variant < -1 || variant > 5 || variant == 2 || variant == 4)
+        return fail(RAG_E_VARIANT, "cost_volume_fwd: unknown variant %d (ids 2 and 4 were retired)", variant);
     unsigned int* ctr = static_cast<unsigned int*>(workspace);
     const bool lean = cv_lean_ok(x, y, cost, Wf) && (Wf / 4) <= 512;
     if (variant == -1) variant = lean ? (ctr ? RAG_CV_FWD_SLIM : 1) : 0;   // the slim geometry is also the fastest alone
-    if (variant >= 2 && !ctr) return fail(RAG_E_NULL, "cost_volume_fwd: variant %d needs a workspace of RAG_CV_FWD_WORKSPACE_BYTES", variant);
-    if (((variant >= 1 && variant <= 3) || variant == 5) && !lean)
+    if (variant >= 3 && !ctr) return fail(RAG_E_NULL, "cost_volume_fwd: variant %d needs a workspace of RAG_CV_FWD_WORKSPACE_BYTES", variant);
+    if (variant >= 1 && !lean)
         return fail(RAG_E_VARIANT, "cost_volume_fwd: lean variants need Wf %% 4 == 0, Wf <= 2048 and 16-byte aligned pointers");
-    if (variant == 1) return launch_cv_fwd_lean<256, 2>(x, y, cost, B, C, Df, Hf, Wf, 0, nullptr, st);
-    if (variant == 2) return launch_cv_fwd_lean<256, 2>(x, y, cost, B, C, Df, Hf, Wf, 1, ctr, st);
-    if (variant == 3) return launch_cv_fwd_lean<512, 1>(x, y, cost, B, C, Df, Hf, Wf, 1, ctr, st);
+    if (variant == 1) return launch_cv_fwd_lean<256, 2, false>(x, y, cost, B, C, Df, Hf, Wf, 0, nullptr, st);
+    if (variant == 3) return launch_cv_fwd_lean<512, 1, true>(x, y, cost, B, C, Df, Hf, Wf, 1, ctr, st);
     // RAG_CV_FWD_SLIM: 256 threads x 1 vector (at most 64 registers: a quarter of the register file per SM), 32 disparities per item
-    if (variant == 5) return launch_cv_fwd_lean<256, 1>(x, y, cost, B, C, Df, Hf, Wf, 1, ctr, st, 32);
-    if (variant == 4) {
-        if (!cv_tma_ok(x, y, cost, Df, Wf))
-            return fail(RAG_E_VARIANT, "cost_volume_fwd: the TMA variant needs Wf %% 4 == 0, Df %% 4 == 0, Df <= Wf and 16-byte aligned pointers");
-        return launch_cv_fwd_tma(x, y, cost, B, C, Df, Hf, Wf, ctr, st);
-    }
+    if (variant == 5) return launch_cv_fwd_lean<256, 1, true>(x, y, cost, B, C, Df, Hf, Wf, 1, ctr, st, 32);
     const bool a16 = aligned(x, 16) && aligned(y, 16) && aligned(cost, 16);
     const bool a8 = aligned(x, 8) && aligned(y, 8) && aligned(cost, 8);
     if (Wf % 4 == 0 && a16) return launch_cv_fwd<4, 256>(x, y, cost, B, C, Df, Hf, Wf, st);

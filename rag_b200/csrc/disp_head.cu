@@ -238,14 +238,15 @@ int upsample_trilinear(const float* cost, float* out, int B, int Dl, int Hl, int
 }
 
 // variant: -1 = default; 0 = any (Dl, maxdisp) (one thread per output pixel, fp64 sums); 1 = first x3 kernel (any width);
-// 2 = cube-root tiled kernel (default when maxdisp == 3*Dl, Wl % 4 == 0, 16-byte aligned input); 3 = as 2 with the
-// fp32-lambda correction at every step and TwoSum totals (most accurate, A/B); 4 = RAG_HEAD_FWD_SHARED: variant 2 as a
-// persistent grid of 3 CTAs per SM (SM sharing)
+// 2 = cube-root tiled kernel (default when maxdisp == 3*Dl, Wl % 4 == 0, 16-byte aligned input); 4 = RAG_HEAD_FWD_SHARED:
+// variant 2 as a persistent grid of 3 CTAs per SM (SM sharing).  Id 3 (variant 2 with the lambda correction at every step
+// and TwoSum totals) was retired: no default or schedule selected it.
 int disp_head_fwd(const float* cost, float* disp, float* stats, int B, int Dl, int Hl, int Wl, int D,
                   int variant, cudaStream_t st) {
     if (!cost || !disp) return fail(RAG_E_NULL, "disp_head_fwd: null pointer");
     if (int e = check_head_args(B, Dl, Hl, Wl, D)) return e;
-    if (variant < -1 || variant > 4) return fail(RAG_E_VARIANT, "disp_head_fwd: unknown variant %d", variant);
+    if (variant < -1 || variant > 4 || variant == 3)
+        return fail(RAG_E_VARIANT, "disp_head_fwd: unknown variant %d (id 3 was retired)", variant);
     const float sd = (float)Dl / (float)D, sh = (float)Hl / (float)(3 * Hl), sw = (float)Wl / (float)(3 * Wl);
     const bool x3 = (D == 3 * Dl);
     if (variant >= 1 && !x3) return fail(RAG_E_VARIANT, "disp_head_fwd: variant %d needs maxdisp == 3*Dl", variant);
@@ -254,7 +255,7 @@ int disp_head_fwd(const float* cost, float* disp, float* stats, int B, int Dl, i
     const bool tiled_ok = x3 && (Wl % 4 == 0) && aligned(cost, 16);
     if (variant >= 2 && !tiled_ok) return fail(RAG_E_VARIANT, "disp_head_fwd: variant %d needs maxdisp == 3*Dl, Wl %% 4 == 0 and 16-byte aligned cost_lr", variant);
     if (variant == -1) variant = tiled_ok ? 2 : (x3 ? 1 : 0);
-    if (variant >= 2) {
+    if (variant == 2) {
         // (5 block rows per CTA would fill the last wave of the 480x960 B=8 grid better, but 5 warps do not
         // spread evenly over the 4 SM sub-partitions: measured 202 us vs 165 us.)
         constexpr int warps = 4;
@@ -263,15 +264,11 @@ int disp_head_fwd(const float* cost, float* disp, float* stats, int B, int Dl, i
         if (n_tl >= (1LL << 31)) return fail(RAG_E_SHAPE, "disp_head_fwd: too many tiles");
         const int grid = (int)(persistent ? std::min<long long>(n_tl, (long long)num_sms() * 3) : n_tl);
         const size_t smem = (size_t)2 * 16 * (warps + 2) * kTCols * sizeof(float) + ((size_t)18 * 32 * warps + 2 * Dl) * sizeof(float2);
-        auto launch = [&](auto kern) -> int {
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-            if (e != cudaSuccess) return fail((int)e, "disp_head_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-            kern<<<grid, 32 * warps, smem, st>>>(cost, disp, stats, Dl, Hl, Wl, sd, nbx, nby, (int)n_tl);
-            return RAG_OK;
-        };
-        const int e = variant == 3 ? launch(head_fwd_x3r_kernel<4, 4, 16, 2, 1, true>) : launch(head_fwd_x3r_kernel<4, 4, 16, 2, 2, false>);
-        if (e) return e;
+        auto kern = head_fwd_x3r_kernel<warps, 4, 16, 2>;
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        if (e != cudaSuccess) return fail((int)e, "disp_head_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+        kern<<<grid, 32 * warps, smem, st>>>(cost, disp, stats, Dl, Hl, Wl, sd, nbx, nby, (int)n_tl);
     } else if (variant == 1) {
         constexpr int WARPS = 4;
         dim3 grid((Wl + 1 + 31) / 32, (Hl + 1 + WARPS - 1) / WARPS, B);
@@ -307,7 +304,7 @@ int disp_head_bwd(const float* cost, const float* gdisp, const float* disp, cons
         if (n_ct >= (1LL << 31)) return fail(RAG_E_SHAPE, "disp_head_bwd: too many tasks");
         const int grid = (int)(persistent ? std::min<long long>(n_ct, (long long)num_sms() * 3) : n_ct);
         const size_t smem = (size_t)3 * (D + 3) * sizeof(float2) + (size_t)4 * kBwWin * sizeof(float);
-        auto kern = persistent ? head_bwd_x3w_kernel<true, true, true> : variant == 1 ? head_bwd_x3w_kernel<true, true> : head_bwd_x3w_kernel<true, false>;
+        auto kern = persistent ? head_bwd_x3w_kernel<true, true> : variant == 1 ? head_bwd_x3w_kernel<true> : head_bwd_x3w_kernel<false>;
         if (variant == 1) {   // two commutative contributions per element into a zeroed buffer (see the kernel's header)
             cudaError_t e = cudaMemsetAsync(gcost, 0, (size_t)B * Dl * Hl * Wl * sizeof(float), st);
             if (e != cudaSuccess) return fail((int)e, "disp_head_bwd: cudaMemsetAsync: %s", cudaGetErrorString(e));

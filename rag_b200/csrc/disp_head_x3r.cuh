@@ -21,17 +21,17 @@
 // (measured in fp64), so the first-order term is applied: bin 3j+2 gets the factor
 // 1 + ln2*d1_j*(z_{j+1}-z_j), bin 3j+3 the factor 1 + ln2*d2_j*(z_{j+1}-z_j), d = lambda_fp32 - q/3
 // (|d| < 4e-6, the neglected second-order term is < 1e-9 relative).  +5 operations per step.
-// CORR: 0 = never, 1 = every step, 2 = from the second window chunk on (d < 1e-6 below bin 48: the
-// uncorrected first chunk costs < 4e-6 px at sigma = 1).
+// The correction runs from the second window chunk on (d < 1e-6 below bin 48: the uncorrected first
+// chunk costs < 4e-6 px at sigma = 1); x3r_step's CORR switches it per chunk.
 //
 // In the H and W axes the phase-1 rows/columns (dst = 3i+1) have lambda == 0 exactly for i >= 1
 // (fma(fl(1/3), 3i+1.5, -0.5) rounds to i because the excess (i+0.5)*2^-25 is below half an ulp of i)
 // and 1.5e-8 for i == 0, so the centre row/column of a 3x3 block is the low-res value itself: the
 // bilinear stage needs 14 packed operations instead of 22.
 //
-// Everything else -- centred 3x3 blocks, 4x32 blocks per CTA, 2-stage cp.async window of 16 low-res
-// bins, lazily moved per-pixel reference exponent, fp32 group sums folded with TwoSum into (hi,lo)
-// totals in shared memory, regression centred on D/2 -- is the plan of disp_head_x3v.cuh.
+// Everything else: centred 3x3 blocks, 4x32 blocks per CTA, 2-stage cp.async window of 16 low-res
+// bins, lazily moved per-pixel reference exponent, fp32 group sums added once per chunk into fp32
+// totals in shared memory, regression centred on D/2.
 //
 // Pixel pairs (p<row><col>):  Q0=(p00,p02) Q1=(p10,p12) Q2=(p20,p22) Q3=(p01,p21) S=p11.
 #pragma once
@@ -102,7 +102,8 @@ __device__ __forceinline__ void x3r_step(const float& c, float& cn, float& c2, f
 // tiles: ceil(Wl/32) x ceil(Hl/WARPS) x B; 32*WARPS threads (a tile is WARPS block rows x 32 block columns); 1-D grid,
 // one tile per CTA or a persistent grid (see the tile loop).
 // smem: tile[STAGES][BINS][WARPS+2][kTCols] | float2 tot[18][NT] | float2 kap[Dl][2] ((k1,k1),(k2,k2))
-template <int WARPS, int MINB, int BINS, int STAGES, int CORR, bool TWOSUM>
+// tot keeps (hi, lo) slots per total; only the hi words are accumulated, the lo words stay zero.
+template <int WARPS, int MINB, int BINS, int STAGES>
 __global__ void __launch_bounds__(32 * WARPS, MINB)
 head_fwd_x3r_kernel(const float* __restrict__ cost, float* __restrict__ disp, float* __restrict__ stats,
                     int Dl, int Hl, int Wl, float scale, int nbx, int nby, int n_tl) {
@@ -225,31 +226,16 @@ head_fwd_x3r_kernel(const float* __restrict__ cost, float* __restrict__ disp, fl
         o[3] = fma2(hM, f2b(v1c), fma2(hO, v1e, mn[3]));
         oS = __fmaf_rn(kS3, v1c, mnS);
     };
-    // group sums -> totals.  TWOSUM keeps (hi, lo) totals with an error-free TwoSum; otherwise the four
-    // chunk sums are simply added in fp32 (at most ~1.5 ulp on top of the in-chunk rounding).
+    // group sums -> totals: the chunk sums are simply added in fp32 (at most ~1.5 ulp on top of the in-chunk rounding).
     auto fold = [&]() {
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-            if (TWOSUM) {
-                float2 hi = mytot[(4 * i + 0) * NT], lo = mytot[(4 * i + 1) * NT];
-                two_sum_acc(hi, lo, st[i].S);
-                mytot[(4 * i + 0) * NT] = hi; mytot[(4 * i + 1) * NT] = lo;
-                hi = mytot[(4 * i + 2) * NT]; lo = mytot[(4 * i + 3) * NT];
-                two_sum_acc(hi, lo, st[i].T);
-                mytot[(4 * i + 2) * NT] = hi; mytot[(4 * i + 3) * NT] = lo;
-            } else {
-                mytot[(4 * i + 0) * NT] = add2(mytot[(4 * i + 0) * NT], st[i].S);
-                mytot[(4 * i + 2) * NT] = add2(mytot[(4 * i + 2) * NT], st[i].T);
-            }
+            mytot[(4 * i + 0) * NT] = add2(mytot[(4 * i + 0) * NT], st[i].S);
+            mytot[(4 * i + 2) * NT] = add2(mytot[(4 * i + 2) * NT], st[i].T);
             st[i].S = f2b(0.f); st[i].T = f2b(0.f);
         }
         float2 d = mytot[16 * NT], n = mytot[17 * NT];
-        if (TWOSUM) {
-            two_sum_acc(d.x, d.y, so.S);
-            two_sum_acc(n.x, n.y, so.T);
-        } else {
-            d.x += so.S; n.x += so.T;
-        }
+        d.x += so.S; n.x += so.T;
         mytot[16 * NT] = d; mytot[17 * NT] = n;
         so.S = 0.f; so.T = 0.f;
     };
@@ -258,14 +244,14 @@ head_fwd_x3r_kernel(const float* __restrict__ cost, float* __restrict__ disp, fl
     // `cur` = which half of the c ping-pong holds c_j.
     auto rescale = [&](auto cur_tag, float2 (&t)[4], float& tS, float2 (&a)[4], float& aS) {
         constexpr int cur = decltype(cur_tag)::value;
-        // the running group sums (registers) and the chunk totals (shared memory; the lo words only exist with
-        // TWOSUM) are both scaled in place -- no fold, so an event costs ~160 instead of ~270 instructions
+        // the running group sums (registers) and the chunk totals (shared memory; hi words only, the lo words are
+        // zero) are both scaled in place -- no fold, so an event costs ~160 instead of ~270 instructions
         auto fix = [&](float& tt, float& aa, float& mn, float& cc, float& c2, float& ps, float& q, float& gs, float& gt,
                        int slot, bool hi_lane) {
             if (tt > kX3rPiggy) {
                 const float f = ex2_approx(-tt), f3 = ex2_approx(-3.f * tt);
 #pragma unroll
-                for (int s = 0; s < 4; s += (TWOSUM ? 1 : 2)) {
+                for (int s = 0; s < 4; s += 2) {
                     float2 v = mytot[(slot + s) * NT];
                     if (hi_lane) v.y *= f3; else v.x *= f3;
                     mytot[(slot + s) * NT] = v;
@@ -387,7 +373,7 @@ head_fwd_x3r_kernel(const float* __restrict__ cost, float* __restrict__ disp, fl
         }
         const int n_it = jend - max(jbeg, 1);
         const float2* kp = kap + 2 * (max(jbeg, 1) - 1);
-        if (CORR == 1 || (CORR == 2 && ch > 0)) run_chunk(std::true_type{}, p, n_it, kp);
+        if (ch > 0) run_chunk(std::true_type{}, p, n_it, kp);
         else run_chunk(std::false_type{}, p, n_it, kp);
         fold();
         __syncthreads();

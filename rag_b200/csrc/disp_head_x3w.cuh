@@ -1,4 +1,4 @@
-// x3 disparity-head backward, second generation (default when a scratch buffer is supplied: <CUBE = true>).
+// x3 disparity-head backward, second generation (the default whenever maxdisp == 3*Dl: <RED = true>).
 //
 // Same maths as head_bwd_x3_kernel (disp_head_x3.cuh): deterministic, atomics-free transpose of the
 // upsample applied to -g p_k (k - disp), p_k rebuilt from cost_lr and the forward's stats.  What the
@@ -26,7 +26,7 @@ constexpr int kBwCols = 34;              // window width: 32 block columns + 1 +
 constexpr int kBwWin = kBwBins * 2 * kBwCols;
 
 //
-// CUBE (default): the three full-res bins of a k-block come from ONE exp2 per pixel instead of three.  With
+// Cube root: the three full-res bins of a k-block come from ONE exp2 per pixel instead of three.  With
 // c_j = 2^(e_j/3) (e_j = relative exponent of low-res bin j) and PyTorch's lambdas (0, ~1/3, ~2/3),
 //   2^e(3j+1) = c_j^3,   2^e(3j+2) = c_j^2 c_j+1 (1 + kap2 du),   2^e(3j+3) = c_j c_j+1^2 (1 + kap3 du),
 // du = (e_j+1 - e_j)/3, kap_q = 3 ln2 (lambda_fp32 - q/3): the first-order term restores the reference's
@@ -46,14 +46,14 @@ constexpr int kBwWin = kBwBins * 2 * kBwCols;
 // few CTAs per SM that is resident at once, which is what lets the kernel share the SMs with a cost-volume kernel on
 // another stream whichever of the two is launched first (RAG_HEAD_BWD_SHARED, rag_b200.pipeline).  The warps of a CTA
 // walk their task lists independently: the depth tables are built once per CTA, nothing else is shared between tasks.
-template <bool CUBE, bool RED, bool PERSIST = false>
+template <bool RED, bool PERSIST = false>
 __global__ void __launch_bounds__(128, 4)
 head_bwd_x3w_kernel(const float* __restrict__ cost, const float* __restrict__ gdisp, const float* __restrict__ disp,
                     const float* __restrict__ stats, float* __restrict__ gcost, float* __restrict__ scratch,
                     int Dl, int Hl, int Wl, float scale, int nJ, int n_tasks, int strips, int n_ct) {
     extern __shared__ __align__(16) float x3w_smem[];
     const int D = 3 * Dl, H = 3 * Hl, W = 3 * Wl;
-    float2* lzb = reinterpret_cast<float2*>(x3w_smem);   // [D+3] (lambda1, lambda1) of bin k
+    float2* lzb = reinterpret_cast<float2*>(x3w_smem);   // [D+3] kap_q of bin k (see above), broadcast
     float2* dAb = lzb + (D + 3);                          // [D+3] weight of bin k into cell (k-1)/3, broadcast
     float2* dBb = dAb + (D + 3);                          // [D+3] ... into cell (k-1)/3 + 1
     float* win_all = reinterpret_cast<float*>(dBb + (D + 3));
@@ -65,13 +65,11 @@ head_bwd_x3w_kernel(const float* __restrict__ cost, const float* __restrict__ gd
             const int jb = k == 0 ? 0 : (k - 1) / 3;
             wa = (t0 == jb ? l0 : 0.f) + (t1 == jb ? l1 : 0.f);
             wb = (t0 == jb + 1 ? l0 : 0.f) + (t1 == jb + 1 ? l1 : 0.f);
-            if (CUBE) {
-                // lambda - fl(q/3) is exact in fp32 (Sterbenz); fl(1/3) - 1/3 = 2^-25/3, fl(2/3) - 2/3 = 2^-24/3
-                const int q = k == 0 ? 0 : (k - 1) % 3;
-                const float third = q == 1 ? 0.333333343267440796f : 0.666666686534881592f;
-                const float resid = q == 1 ? 9.934107e-9f : 1.9868214e-8f;
-                l1 = (q != 0 && t1 > t0) ? 2.0794415416798357f * ((l1 - third) + resid) : 0.f;
-            }
+            // lambda - fl(q/3) is exact in fp32 (Sterbenz); fl(1/3) - 1/3 = 2^-25/3, fl(2/3) - 2/3 = 2^-24/3
+            const int q = k == 0 ? 0 : (k - 1) % 3;
+            const float third = q == 1 ? 0.333333343267440796f : 0.666666686534881592f;
+            const float resid = q == 1 ? 9.934107e-9f : 1.9868214e-8f;
+            l1 = (q != 0 && t1 > t0) ? 2.0794415416798357f * ((l1 - third) + resid) : 0.f;
         }
         lzb[k] = f2b(l1); dAb[k] = f2b(wa); dBb[k] = f2b(wb);
     }
@@ -150,7 +148,7 @@ head_bwd_x3w_kernel(const float* __restrict__ cost, const float* __restrict__ gd
                 const int i = ph * 3 + pw;
                 const size_t o = (size_t)ah.idx[ph] * W + aw.idx[pw];   // clamped -> always a real pixel
                 const bool ok = ah.valid[ph] && aw.valid[pw];
-                m9[i] = -__ldg(sm + o) * (CUBE ? 0.333333343267440796f : 1.f);   // CUBE works on exponent / 3
+                m9[i] = -__ldg(sm + o) * 0.333333343267440796f;   // the cube-root form works on exponent / 3
                 d9[i] = __ldg(dp + o);
                 g9[i] = ok ? -__ldg(gd + o) * __ldg(sm + img + o) : 0.f;
                 gabs = fmaxf(gabs, fabsf(g9[i]));
@@ -185,7 +183,7 @@ head_bwd_x3w_kernel(const float* __restrict__ cost, const float* __restrict__ gd
     float2 h0b[3], h1b[3], hAb[3], hBb[3];
 #pragma unroll
     for (int i = 0; i < 3; ++i) {
-        constexpr float ks = CUBE ? kX3NegLog2e / 3.0f : kX3NegLog2e;
+        constexpr float ks = kX3NegLog2e / 3.0f;
         h0b[i] = f2b(ah.l0[i] * ks); h1b[i] = f2b(ah.l1[i] * ks);
         hAb[i] = f2b(ah.wa[i]); hBb[i] = f2b(ah.wb[i]);
     }
@@ -236,21 +234,18 @@ head_bwd_x3w_kernel(const float* __restrict__ cost, const float* __restrict__ gd
     // bin 0 and feeds cell 0 only: its share is the initial value (cell 0 = k-block 0's "A" part + this)
     float2 pg[4] = {f2b(0.f), f2b(0.f), f2b(0.f), f2b(0.f)};
     float pgS = 0.f;
-    // CUBE: c = 2^(a) with a = exponent / 3 of the k-block's lower bin, and its square, carried across k-blocks
+    // c = 2^(a) with a = exponent / 3 of the k-block's lower bin, carried across k-blocks
     float2 ca[4];
-    float caS = 0.f;
-    if (CUBE) {
 #pragma unroll
-        for (int i = 0; i < 4; ++i) ca[i] = ex2_2(a[i]);
-        caS = ex2_approx(aS);
-    }
+    for (int i = 0; i < 4; ++i) ca[i] = ex2_2(a[i]);
+    float caS = ex2_approx(aS);
     if (jb0 == 0 && j0 == 0) {
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-            const float2 e0 = CUBE ? mul2(mul2(ca[i], ca[i]), ca[i]) : ex2_2(a[i]);
+            const float2 e0 = mul2(mul2(ca[i], ca[i]), ca[i]);
             pg[i] = mul2(gneg[i], mul2(dAb[0], mul2(e0, fma2(dsp[i], neg1, f2b(0.f)))));
         }
-        pgS = gnegS * (dAb[0].x * ((CUBE ? caS * caS * caS : ex2_approx(aS)) * (0.f - dspS)));
+        pgS = gnegS * (dAb[0].x * ((caS * caS * caS) * (0.f - dspS)));
     }
     // the upstream factor -g/sum is folded into (k - disp): gdk = gneg*k - gneg*disp, so the bin terms come out
     // already scaled (two multiplications per pixel pair and k-block fewer)
@@ -263,74 +258,44 @@ head_bwd_x3w_kernel(const float* __restrict__ cost, const float* __restrict__ gd
     for (int jb = jb0; jb < j1; ++jb) {
         if (wp < wlast) wp += 2 * kBwCols;   // upper bin min(jb+1, Dl-1)
         blend(wp, t, tS);
-        const float2 l1 = CUBE ? f2b(0.f) : lp[0], l2 = lp[1], l3 = lp[2];   // CUBE: (-, kap2, kap3)
-        const float2 a1 = CUBE ? f2b(1.f) : ap[0], a2 = ap[1], a3 = ap[2];
-        const float2 b1 = CUBE ? f2b(0.f) : bp[0], b2 = bp[1], b3 = bp[2];
+        const float2 l2 = lp[1], l3 = lp[2];   // (kap2, kap3); the centre bin lp[0] needs no correction
+        const float2 a2 = ap[1], a3 = ap[2];
+        const float2 b2 = bp[1], b3 = bp[2];
         lp += 3; ap += 3; bp += 3;
         const float2 kfb = f2b(kf);
         float2 g0[4], g1[4];
         float g0S, g1S;
-        if (CUBE) {
-            // the centre bin k1 = 3 jb + 1 has lambda1 == 0 exactly (it IS low-res bin jb): weight 1 into cell jb,
-            // none into cell jb + 1, so its term starts the "A" chain together with the previous k-block's "B" part
+        // the centre bin k1 = 3 jb + 1 has lambda1 == 0 exactly (it IS low-res bin jb): weight 1 into cell jb,
+        // none into cell jb + 1, so its term starts the "A" chain together with the previous k-block's "B" part.
+        // Cell jb = this k-block's "A" bin part + the previous k-block's "B" bin part: the spatial transpose is
+        // linear, so the two parts are added per pixel first and transposed ONCE
 #pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const float2 ct = ex2_2(t[i]);
-                const float2 du = fma2(a[i], neg1, t[i]);
-                const float2 x = mul2(ca[i], ct), c2 = mul2(ca[i], ca[i]);
-                const float2 dk = fma2(gneg[i], kfb, ngd[i]);        // gneg * (k1 - disp)
-                const float2 dk1 = add2(dk, gneg[i]), dk2 = add2(dk1, gneg[i]);
-                const float2 q2 = mul2(x, ca[i]), q3 = mul2(x, ct);
-                const float2 u2 = mul2(fma2(q2, mul2(l2, du), q2), dk1);
-                const float2 u3 = mul2(fma2(q3, mul2(l3, du), q3), dk2);
-                g0[i] = fma2(a3, u3, fma2(a2, u2, fma2(mul2(c2, ca[i]), dk, pg[i])));
-                g1[i] = fma2(b3, u3, mul2(b2, u2));
-                a[i] = t[i]; ca[i] = ct;
-            }
-            {
-                const float ct = ex2_approx(tS);
-                const float du = tS - aS;
-                const float x = caS * ct;
-                const float dk = __fmaf_rn(gnegS, kf, ngdS);
-                const float q2 = x * caS, q3 = x * ct;
-                const float u2 = __fmaf_rn(q2, l2.x * du, q2) * (dk + gnegS);
-                const float u3 = __fmaf_rn(q3, l3.x * du, q3) * ((dk + gnegS) + gnegS);
-                g0S = __fmaf_rn(a3.x, u3, __fmaf_rn(a2.x, u2, __fmaf_rn(caS * caS * caS, dk, pgS)));
-                g1S = __fmaf_rn(b3.x, u3, b2.x * u2);
-                aS = tS; caS = ct;
-            }
-        } else {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const float2 dlt = fma2(a[i], neg1, t[i]);
-                const float2 dk = fma2(gneg[i], kfb, ngd[i]);        // gneg * (k1 - disp)
-                const float2 dk1 = add2(dk, gneg[i]), dk2 = add2(dk1, gneg[i]);
-                const float2 u1 = mul2(ex2_2(fma2(l1, dlt, a[i])), dk);
-                const float2 u2 = mul2(ex2_2(fma2(l2, dlt, a[i])), dk1);
-                const float2 u3 = mul2(ex2_2(fma2(l3, dlt, a[i])), dk2);
-                g0[i] = fma2(a3, u3, fma2(a2, u2, mul2(a1, u1)));
-                g1[i] = fma2(b3, u3, fma2(b2, u2, mul2(b1, u1)));
-                a[i] = t[i];
-            }
-            {
-                const float dlt = tS - aS;
-                const float dk = __fmaf_rn(gnegS, kf, ngdS);
-                const float u1 = ex2_approx(__fmaf_rn(l1.x, dlt, aS)) * dk;
-                const float u2 = ex2_approx(__fmaf_rn(l2.x, dlt, aS)) * (dk + gnegS);
-                const float u3 = ex2_approx(__fmaf_rn(l3.x, dlt, aS)) * ((dk + gnegS) + gnegS);
-                g0S = __fmaf_rn(a3.x, u3, __fmaf_rn(a2.x, u2, a1.x * u1));
-                g1S = __fmaf_rn(b3.x, u3, __fmaf_rn(b2.x, u2, b1.x * u1));
-                aS = tS;
-            }
+        for (int i = 0; i < 4; ++i) {
+            const float2 ct = ex2_2(t[i]);
+            const float2 du = fma2(a[i], neg1, t[i]);
+            const float2 x = mul2(ca[i], ct), c2 = mul2(ca[i], ca[i]);
+            const float2 dk = fma2(gneg[i], kfb, ngd[i]);        // gneg * (k1 - disp)
+            const float2 dk1 = add2(dk, gneg[i]), dk2 = add2(dk1, gneg[i]);
+            const float2 q2 = mul2(x, ca[i]), q3 = mul2(x, ct);
+            const float2 u2 = mul2(fma2(q2, mul2(l2, du), q2), dk1);
+            const float2 u3 = mul2(fma2(q3, mul2(l3, du), q3), dk2);
+            g0[i] = fma2(a3, u3, fma2(a2, u2, fma2(mul2(c2, ca[i]), dk, pg[i])));
+            g1[i] = fma2(b3, u3, mul2(b2, u2));
+            a[i] = t[i]; ca[i] = ct;
+        }
+        {
+            const float ct = ex2_approx(tS);
+            const float du = tS - aS;
+            const float x = caS * ct;
+            const float dk = __fmaf_rn(gnegS, kf, ngdS);
+            const float q2 = x * caS, q3 = x * ct;
+            const float u2 = __fmaf_rn(q2, l2.x * du, q2) * (dk + gnegS);
+            const float u3 = __fmaf_rn(q3, l3.x * du, q3) * ((dk + gnegS) + gnegS);
+            g0S = __fmaf_rn(a3.x, u3, __fmaf_rn(a2.x, u2, __fmaf_rn(caS * caS * caS, dk, pgS)));
+            g1S = __fmaf_rn(b3.x, u3, b2.x * u2);
+            aS = tS; caS = ct;
         }
         kf += 3.f;
-        // cell jb = this k-block's "A" bin part + the previous k-block's "B" bin part: the spatial transpose is
-        // linear, so the two parts are added per pixel first and transposed ONCE
-        if (!CUBE) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) g0[i] = add2(g0[i], pg[i]);
-            g0S += pgS;
-        }
         if (jb >= j0) {
             float vA, vB;
             transpose(g0, g0S, vA, vB);

@@ -1,6 +1,6 @@
 // Helpers shared by the x3 disparity-head kernels (disp_head_x3.cuh, disp_head_x3r.cuh, disp_head_x3w.cuh):
-// packed-FP32 wrappers (FFMA2 / FADD2 / FMUL2 on sm_100a), the error-free accumulation used for the softmax
-// totals, and the geometry of the shared-memory window of the tiled forward kernel.
+// packed-FP32 wrappers (FFMA2 / FADD2 / FMUL2 on sm_100a) and the geometry of the shared-memory window of the
+// tiled forward kernel.
 #pragma once
 #include "common.cuh"
 
@@ -17,22 +17,5 @@ __device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c) { return __
 __device__ __forceinline__ float2 add2(float2 a, float2 b) { return __fadd2_rn(a, b); }
 __device__ __forceinline__ float2 mul2(float2 a, float2 b) { return __fmul2_rn(a, b); }
 __device__ __forceinline__ float2 ex2_2(float2 z) { return make_float2(ex2_approx(z.x), ex2_approx(z.y)); }
-
-// error-free accumulation of g into (hi, lo):  hi + lo + g  ==  hi' + lo'  up to O(eps^2)
-__device__ __forceinline__ void two_sum_acc(float2& hi, float2& lo, float2 g) {
-    const float2 neg1 = f2b(-1.f);
-    const float2 s = add2(hi, g);
-    const float2 bb = fma2(hi, neg1, s);                       // s - hi
-    const float2 e1 = fma2(fma2(bb, neg1, s), neg1, hi);       // hi - (s - bb)
-    const float2 e2 = fma2(bb, neg1, g);                       // g - bb
-    lo = add2(lo, add2(e1, e2));
-    hi = s;
-}
-__device__ __forceinline__ void two_sum_acc(float& hi, float& lo, float g) {
-    const float s = hi + g;
-    const float bb = s - hi;
-    lo += (hi - (s - bb)) + (g - bb);
-    hi = s;
-}
 
 }  // namespace rag

@@ -7,7 +7,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))  # tests/ -> 
 sys.path.insert(0, ROOT)
 from rag_b200 import functional as F_
 from oracle import rag_oracle as O
-vs = [int(a) for a in sys.argv[1:]] or [9, 10, 11, 12]
+vs = [int(a) for a in sys.argv[1:]] or [0, 1, 2, 4]
 for (dl, hl, wl, md, sigma) in ((64, 48, 96, 192, 1.0), (64, 48, 96, 192, 5.0), (96, 24, 64, 288, 1.0), (64, 48, 96, 192, 20.0)):
     g = torch.Generator().manual_seed(7)
     cost = torch.randn(2, 1, dl, hl, wl, generator=g) * sigma

@@ -44,8 +44,15 @@ SHAPES = [
     (1, 4, 3, 10, 48),       # Wf < Df
     (3, 1, 1, 4, 3),         # Df = 1
     (1, 12, 33, 64, 100),    # Df = 33 (not a multiple of 4), ragged row tile
-    (2, 5, 11, 36, 48),      # TMA kernel: ragged row tiles (Hf % R != 0), Df = 16
-    (1, 2, 6, 64, 192),      # TMA kernel: Df == Wf (last disparity keeps a single column)
+    (2, 5, 11, 36, 48),      # ragged row tiles (Hf % R != 0), Df = 16
+    (1, 2, 6, 64, 192),      # Df == Wf (last disparity keeps a single column)
+    (1, 12, 4, 1024, 192),   # widest row the slim persistent geometry takes (256 vectors: one row per tile)
+    (2, 3, 5, 8, 96),        # Wf < Df on the lean kernels
+    (1, 2, 1, 12, 6),        # Hf = 1, Df = 2
+    (2, 12, 3, 96, 195),     # Df = 65: one disparity past the last full disparity chunk
+    (1, 1, 50, 44, 96),      # C = 1, 11 vectors per row: many ragged rows per tile
+    (1, 5, 17, 132, 120),    # Df = 40, Hf prime
+    (3, 2, 2, 4, 192),       # Wf = 4: one vector per row, Df = 64 >> Wf
 ]
 
 
@@ -55,10 +62,8 @@ def test_forward_bit_exact(F_, shape):
     g = gen(hash(shape) % 1000)
     x, y = randn((b, c, hf, wf), g), randn((b, c, hf, wf), g)
     ref = O.cost_volume_ref(x, y, md)
-    df = int(md / 3)
-    tma = (4,) if (wf % 4 == 0 and df % 4 == 0 and df <= wf) else ()
     # None = default with a workspace (persistent lean kernel), "plain" = the stateless entry point without one
-    for variant in (None, "plain", 0) + ((1, 2, 3, 5) if wf % 4 == 0 else ()) + tma:
+    for variant in (None, "plain", 0) + ((1, 3, 5) if wf % 4 == 0 else ()):
         if variant == "plain":
             out = F_.cost_volume_forward(x.cuda(), y.cuda(), int(md / 3), workspace=False)
         else:
@@ -166,6 +171,10 @@ def test_errors_are_loud(F_):
         F_.cost_volume(torch.zeros(1, 2, 3, 4, device="cuda"), torch.zeros(1, 2, 3, 5, device="cuda"))
     with pytest.raises(RuntimeError):
         F_.cost_volume_forward(torch.zeros(1, 2, 3, 4, device="cuda"), torch.zeros(1, 2, 3, 4, device="cuda"), 4, variant=99)
+    # retired ids (2: lean persistent 256 x 2, 4: TMA bulk stores) are refused, with a workspace and on a lean-capable shape
+    for v in (2, 4):
+        with pytest.raises(RuntimeError, match="unknown variant"):
+            F_.cost_volume_forward(torch.zeros(1, 2, 3, 4, device="cuda"), torch.zeros(1, 2, 3, 4, device="cuda"), 4, variant=v)
 
 
 def test_deterministic(F_):

@@ -15,7 +15,7 @@ def test_exports_answer_errors_without_gpu():
     from rag_b200 import _cabi
 
     L = _cabi.lib()
-    assert _cabi.ABI_VERSION == 17 and L.rag_abi_version() == 17
+    assert _cabi.ABI_VERSION == 18 and L.rag_abi_version() == 18
     fwd, bwd, ws = L.rag_grid_sample_fwd, L.rag_grid_sample_bwd, L.rag_grid_sample_bwd_workspace_bytes
     shape = (2, 3, 8, 16, 8, 16)
     # null pointers: -1

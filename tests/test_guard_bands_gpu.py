@@ -32,14 +32,15 @@ def st():
     return torch.cuda.current_stream().cuda_stream
 
 
-@pytest.mark.parametrize("shape", [(2, 12, 9, 36, 96), (1, 3, 5, 37, 30), (1, 4, 7, 70, 192), (1, 2, 3, 10, 48), (1, 12, 33, 64, 100), (1, 3, 9, 64, 192)], ids=str)
+@pytest.mark.parametrize("shape", [(2, 12, 9, 36, 96), (1, 3, 5, 37, 30), (1, 4, 7, 70, 192), (1, 2, 3, 10, 48), (1, 12, 33, 64, 100), (1, 3, 9, 64, 192),
+                                   (2, 3, 5, 8, 96), (1, 5, 17, 132, 120), (3, 2, 2, 4, 192)], ids=str)
 def test_cost_volume_guards(L, shape):
     b, c, hf, wf, md = shape
     df = int(md / 3)
     g = gen(1)
     x, y = randn((b, c, hf, wf), g).cuda(), randn((b, c, hf, wf), g).cuda()
     n = b * 2 * c * df * hf * wf
-    variants = [-1, 0] + ([1, 2, 3, 5] if wf % 4 == 0 else []) + ([4] if (wf % 4 == 0 and df % 4 == 0 and df <= wf) else [])
+    variants = [-1, 0] + ([1, 3, 5] if wf % 4 == 0 else [])
     for v in variants:
         buf, out = window(n)
         wbuf, ws = window(4)                       # the 16-byte work-counter workspace, itself behind guard bands
@@ -60,14 +61,15 @@ def test_cost_volume_guards(L, shape):
         assert not (gx == CANARY).any() and not (gy == CANARY).any()
 
 
-@pytest.mark.parametrize("shape", [(1, 16, 5, 36, 48), (2, 8, 3, 7, 24), (1, 20, 9, 4, 60), (1, 12, 3, 4, 48), (1, 64, 7, 33, 192), (2, 64, 6, 64, 192)], ids=str)
+@pytest.mark.parametrize("shape", [(1, 16, 5, 36, 48), (2, 8, 3, 7, 24), (1, 20, 9, 4, 60), (1, 12, 3, 4, 48), (1, 64, 7, 33, 192), (2, 64, 6, 64, 192),
+                                   (1, 64, 4, 32, 192), (2, 17, 3, 12, 51), (1, 32, 12, 8, 96)], ids=str)
 def test_head_guards(L, shape):
     b, dl, hl, wl, md = shape
     g = gen(2)
     cl = randn((b, 1, dl, hl, wl), g).cuda()
     npx = b * 9 * hl * wl
     x3 = md == 3 * dl
-    fv = [0] + ([1] if x3 else []) + ([2, 3, 4] if x3 and wl % 4 == 0 else [])
+    fv = [0] + ([1] if x3 else []) + ([2, 4] if x3 and wl % 4 == 0 else [])
     for v in fv:
         bd, disp = window(npx)
         bs, stats = window(2 * npx)

@@ -18,7 +18,7 @@ def test_exports_answer_errors_without_gpu():
     from rag_b200 import _cabi
 
     L = _cabi.lib()
-    assert _cabi.ABI_VERSION == 17 and L.rag_abi_version() == 17
+    assert _cabi.ABI_VERSION == 18 and L.rag_abi_version() == 18
     for fn in (L.rag_bilinear_resize_fwd, L.rag_bilinear_resize_bwd):
         # null pointers: -1 with "null" in the text
         assert fn(None, FAKE, 1, 4, 8, 8, 16, 1, None) == -1

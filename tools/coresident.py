@@ -78,7 +78,7 @@ def main():
 
     # ---- 2. each kernel alone (back-to-back launches; the volume kernels' own traffic keeps everything cold) ----
     k = {}
-    for v in (None, 2, P_.CV_FWD_SHARED, P_.CV_FWD_SLIM):
+    for v in (None, P_.CV_FWD_SHARED, P_.CV_FWD_SLIM):
         k[f"cv_fwd v{v}"] = alone(lambda v=v: F_.cost_volume_forward(x, y, df, variant=v))
     for v in (None, P_.CV_BWD_SHARED) + cvbs:
         k[f"cv_bwd v{v}"] = alone(lambda v=v: F_.cost_volume_backward(gc, c, variant=v))
@@ -107,7 +107,7 @@ def main():
 
     sets = dict(P_.SCHEDULES)
     if a.infer_only:
-        sets = {f"cf{vcf} hf{vhf}": (vcf, vhf, None, None) for vcf in (2, P_.CV_FWD_SHARED, P_.CV_FWD_SLIM) for vhf in (None, P_.HEAD_FWD_SHARED)}
+        sets = {f"cf{vcf} hf{vhf}": (vcf, vhf, None, None) for vcf in (P_.CV_FWD_SHARED, P_.CV_FWD_SLIM) for vhf in (None, P_.HEAD_FWD_SHARED)}
     elif a.full:
         for vcf, vhf, vcb, vhb in itertools.product((P_.CV_FWD_SLIM,), (None, P_.HEAD_FWD_SHARED),
                                                     (None,) + cvbs, (None, P_.HEAD_BWD_SHARED)):

@@ -79,7 +79,7 @@ def main():
     hbw = lambda: F_.disp_head_backward(cl, gd, disp, stats, md)  # noqa: E731
     out["head_fwd_alone"] = round(alone(hfw), 4)
     out["head_bwd_alone"] = round(alone(hbw), 4)
-    for v in (1, 2, 3):
+    for v in (1, 3):
         f = lambda v=v: F_.cost_volume_forward(x, y, df, variant=v)  # noqa: E731
         out[f"cv_fwd_v{v}_alone"] = round(alone(f), 4)
         for first in (True, False):

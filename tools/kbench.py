@@ -82,7 +82,7 @@ def main():
         return not a.only or k in a.only.split(",")
 
     if want("cv_fwd"):
-        for v in (0, 1, 2, 3, 4):
+        for v in (0, 1, 3):
             med, best = timeit(lambda: F_.cost_volume_forward(x, y, df, variant=v), a.iters, flush)
             report("cv_fwd", v, med, best, vol_bytes)
         # torch baseline for scale: a plain device copy of the same number of bytes
@@ -136,7 +136,7 @@ def main():
             torch.backends.cudnn.allow_tf32 = True
         del feat
     if want("head_fwd"):
-        for v in (2, 3, 1):
+        for v in (2, 1):
             try:
                 med, best = timeit(lambda: F_.disp_head_forward(cost_lr, md, True, variant=v), a.iters, flush)
                 report("head_fwd", v, med, best, hf_bytes)

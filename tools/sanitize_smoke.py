@@ -27,9 +27,7 @@ g = torch.Generator(device=dev).manual_seed(0)
 for (b, c, hf, wf, md) in [(1, 12, 9, 36, 96), (2, 3, 5, 37, 30), (1, 4, 7, 70, 192), (1, 2, 3, 10, 48)]:
     x = torch.randn(b, c, hf, wf, device=dev, generator=g); y = torch.randn(b, c, hf, wf, device=dev, generator=g)
     df = int(md / 3)
-    lean = tuple(range(18, 37)) + (4, 8, 9, 10) if wf % 4 == 0 else ()
-    tma = (11, 12, 13, 14) if (wf % 4 == 0 and df % 4 == 0 and df <= wf) else ()
-    for v in (None, 0, 1, 2, 3) + lean + tma:
+    for v in (None, 0, 1, 3, 5):
         cost = run(F_.cost_volume_forward, x, y, df, variant=v)
     cost = F_.cost_volume_forward(x, y, df)
     gc = torch.randn_like(cost)
@@ -39,10 +37,10 @@ for (b, dl, hl, wl, md) in [(1, 16, 5, 36, 48), (2, 8, 3, 7, 24), (1, 20, 9, 4, 
     cl = torch.randn(b, 1, dl, hl, wl, device=dev, generator=g)
     gd = torch.randn(b, 3 * hl, 3 * wl, device=dev, generator=g)
     x3 = md == 3 * dl
-    for vf in [None, 0] + ([1, 2, 3] if x3 else []) + ([4, 5, 6, 7, 9, 10, 11, 12, 13, 14, 15, 16] if x3 and wl % 4 == 0 else []):
+    for vf in [None, 0] + ([1, 2, 4] if x3 else []):
         run(F_.disp_head_forward, cl, md, True, variant=vf)
     disp, st = F_.disp_head_forward(cl, md, True)
-    for vb in [None, 0] + ([1, 2, 3, 4] if x3 else []):
+    for vb in [None, 0] + ([1, 2, 3] if x3 else []):
         run(F_.disp_head_backward, cl, gd, disp, st, md, variant=vb)
     F_.upsample_trilinear(cl, md, True)
 p = torch.softmax(torch.randn(1, 24, 6, 10, device=dev, generator=g), 1).contiguous().requires_grad_(True)

@@ -24,12 +24,11 @@ summ() {  # $1 = regex on the mangled name, $2 = output stem
   done
 }
 rm -f $OUT/r2_*.txt
-summ "cv_fwd_lean_kernelILi256ELi2ELb1ELi0" r2_cv_fwd_lean
-summ "cv_fwd_tma_kernel" r2_cv_fwd_tma
+summ "cv_fwd_lean_kernelILi256ELi1ELb1ELi0" r2_cv_fwd_lean
 summ "cv_bwd_v4_kernel" r2_cv_bwd_v4
 summ "cv_bwd_v4_persistent" r2_cv_bwd_v4
-summ "head_fwd_x3r_kernelILi4ELi4ELi16ELi2ELi2ELb0" r2_head_fwd_x3r
-summ "head_bwd_x3w_kernelILb1ELb1" r2_head_bwd_x3w
+summ "head_fwd_x3r_kernelILi4ELi4ELi16ELi2EE" r2_head_fwd_x3r
+summ "head_bwd_x3w_kernelILb1E" r2_head_bwd_x3w
 summ "stem_bwd_maps_kernelILi8" r2_stem_train
 summ "stem_bwd_inputs_kernel" r2_stem_train
 summ "stem_bwd_weight_kernel" r2_stem_train
