@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "librag_b200.so")
-SOURCES = ["abi.cu", "cost_volume.cu", "disp_head.cu", "extras.cu", "cv_stem.cu", "cv_stem_train.cu", "last_conv.cu", "last_conv_bwd.cu", "trilinear.cu", "conv3d_cc.cu", "bn3d.cu", "conv3d_pw.cu", "grid_sample.cu"]
+SOURCES = ["abi.cu", "cost_volume.cu", "disp_head.cu", "extras.cu", "cv_stem.cu", "cv_stem_train.cu", "last_conv.cu", "last_conv_bwd.cu", "trilinear.cu", "conv3d_cc.cu", "conv3d_cc_tf32.cu", "bn3d.cu", "conv3d_pw.cu", "grid_sample.cu"]
 FLAGS = [
     "-O3", "-std=c++17", "-lineinfo",
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -289,7 +289,7 @@ __global__ void __launch_bounds__(256) conv3d_cc_wgrad_final_kernel(const float*
 // ---- host ---------------------------------------------------------------------------------------------------------------
 static bool cc_pair(int C, int O) { return C == O && (C == 4 || C == 8 || C == 12); }
 
-static int cc_check(const char* who, int B, int C, int O, int D, int H, int W) {
+int cc_check(const char* who, int B, int C, int O, int D, int H, int W) {
     if (B <= 0 || C <= 0 || O <= 0 || D <= 0 || H <= 0 || W <= 0) return fail(RAG_E_SHAPE, "%s: non-positive dimension", who);
     if (!cc_pair(C, O)) return fail(RAG_E_SHAPE, "%s: (C, O) = (%d, %d) is not compiled; have (4,4), (8,8), (12,12)", who, C, O);
     if (W % 4 != 0) return fail(RAG_E_SHAPE, "%s: W=%d must be a multiple of 4", who, W);

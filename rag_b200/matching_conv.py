@@ -11,6 +11,11 @@ runs them in fp32 for (C, O) in ``PAIRS``:
   convolution output once (``batchnorm.backward``), runs the forward kernel on it with the weights transposed and flipped for
   the data gradient, and reduces the weight gradient in a fixed order (bitwise repeatable).
 
+With ``install(..., matching_convs=True, matching_tf32=True)`` the convolutions of a qualifying call run on the tensor cores
+in TF32 (csrc/conv3d_cc_tf32.cu: the forward, and the data gradient) while ``torch.backends.cudnn.allow_tf32`` is on, read
+at call time -- the switch that makes the reference's own cuDNN convolutions TF32.  The BatchNorm and the weight gradient
+stay fp32, and so does 4 -> 4 (``use_tf32``).
+
 ``qualifies(layer, x)`` is the only routing decision; ``matching_forward`` -- bound onto ``ConvBR_3d.forward`` by
 ``rag_b200.network.install(..., matching_convs=True)`` -- sends qualifying plain-tensor calls here and everything else to
 ``fused_stem.stem_forward`` unchanged.
@@ -25,11 +30,26 @@ from .functional import _require, _stream
 from .fused_stem import stem_forward
 
 PAIRS = ((4, 4), (8, 8), (12, 12))     # the (C, O) instantiations of csrc/conv3d_cc.cu (16 -> 16 lost to cuDNN: DESIGN.md 5.10)
+_TF32 = False                           # set by network.install(matching_tf32=...), cleared by network.uninstall()
 
 
-def conv3d_cc_forward(x: torch.Tensor, weight: torch.Tensor, scale=None, shift=None, relu: bool = False) -> torch.Tensor:
+def set_tf32(on: bool) -> None:
+    global _TF32
+    _TF32 = bool(on)
+
+
+def use_tf32(c: int) -> bool:
+    """True when a qualifying call with C input channels runs its convolutions in TF32: ``install(..., matching_tf32=True)``
+    and torch's cuDNN TF32 switch (``torch.backends.cudnn.allow_tf32``) both on, and C > 4.  At C = 4 the TF32 kernel is no
+    faster than the fp32 one on the measured shapes (DESIGN.md 5.10), so 4 -> 4 stays fp32."""
+    return _TF32 and torch.backends.cudnn.allow_tf32 and c > 4
+
+
+def conv3d_cc_forward(x: torch.Tensor, weight: torch.Tensor, scale=None, shift=None, relu: bool = False,
+                      tf32: bool = False) -> torch.Tensor:
     """out = relu?(fma(conv3d(x, weight, padding=1), scale, shift)) for weight [O,C,3,3,3]; x [B,C,D,H,W] CUDA fp32.
-    scale / shift [O] (both or neither) fold an eval-mode BatchNorm into the store."""
+    scale / shift [O] (both or neither) fold an eval-mode BatchNorm into the store.  ``tf32`` runs the convolution on the
+    tensor cores (``rag_conv3d_cc_tf32_fwd``), else in fp32 (``rag_conv3d_cc_fwd``)."""
     _require(x, "x"), _require(weight, "weight")
     if x.dim() != 5:
         raise RuntimeError(f"rag_b200: conv3d_cc wants a [B,C,D,H,W] input, got {tuple(x.shape)}")
@@ -46,11 +66,12 @@ def conv3d_cc_forward(x: torch.Tensor, weight: torch.Tensor, scale=None, shift=N
     if scale is not None:
         scale, shift = scale.contiguous(), shift.contiguous()
     L = _cabi.lib()
+    name = "rag_conv3d_cc_tf32_fwd" if tf32 else "rag_conv3d_cc_fwd"
     with torch.cuda.device(x.device):
-        rc = L.rag_conv3d_cc_fwd(x.data_ptr(), weight.data_ptr(), scale.data_ptr() if scale is not None else None,
-                                 shift.data_ptr() if shift is not None else None, int(bool(relu)), out.data_ptr(),
-                                 b, c, o, d, h, w, _stream(x))
-    _cabi.check(rc, "rag_conv3d_cc_fwd")
+        rc = getattr(L, name)(x.data_ptr(), weight.data_ptr(), scale.data_ptr() if scale is not None else None,
+                              shift.data_ptr() if shift is not None else None, int(bool(relu)), out.data_ptr(),
+                              b, c, o, d, h, w, _stream(x))
+    _cabi.check(rc, name)
     return out
 
 
@@ -61,11 +82,13 @@ class ConvBR3dFn(torch.autograd.Function):
     the running statistics (eval-mode BatchNorm behind trainable layers).  Saved for the backward: x, the convolution output z
     and the [O,4] table (scale, shift, mean, rstd) -- the reference's own layer keeps its conv output too, so no fourth
     convolution pass is spent on recomputing z.  The backward re-evaluates the forward's own ``fma(z, scale, shift) > 0`` for
-    the ReLU decision (bit-identical)."""
+    the ReLU decision (bit-identical).  ``use_tf32``, read once in the forward, puts z and the data gradient on the TF32
+    kernels; the weight gradient is the fp32 kernel's either way."""
 
     @staticmethod
     def forward(ctx, x, weight, gamma, beta, running_mean, running_var, batch_stats, update_running, momentum, eps):
-        z = conv3d_cc_forward(x, weight)
+        ctx.tf32 = use_tf32(x.shape[1])
+        z = conv3d_cc_forward(x, weight, tf32=ctx.tf32)
         out = z.clone()
         bn = batchnorm.forward(z, out, gamma, beta, running_mean, running_var, batch_stats, update_running, momentum, eps)
         ctx.save_for_backward(x, weight, z, bn)
@@ -87,10 +110,14 @@ class ConvBR3dFn(torch.autograd.Function):
                 gx = torch.empty_like(x) if need_x else None
                 gw = torch.empty_like(weight) if need_w else None
                 ws = torch.empty(int(L.rag_conv3d_cc_bwd_workspace_bytes(b, c, o, d, h, w)) // 4, dtype=torch.float32, device=x.device) if need_w else None
-                rc = L.rag_conv3d_cc_bwd(gz.data_ptr(), x.data_ptr(), weight.data_ptr(), gx.data_ptr() if gx is not None else None,
-                                         gw.data_ptr() if gw is not None else None, ws.data_ptr() if ws is not None else None,
-                                         b, c, o, d, h, w, _stream(x))
-            _cabi.check(rc, "rag_conv3d_cc_bwd")
+                if ctx.tf32 and gx is not None:      # TF32 data gradient; the fp32 call below then takes the weight gradient only
+                    _cabi.check(L.rag_conv3d_cc_tf32_bwd_data(gz.data_ptr(), weight.data_ptr(), gx.data_ptr(), b, c, o, d, h, w, _stream(x)),
+                                "rag_conv3d_cc_tf32_bwd_data")
+                gin = None if ctx.tf32 or gx is None else gx.data_ptr()
+                if gin is not None or gw is not None:
+                    _cabi.check(L.rag_conv3d_cc_bwd(gz.data_ptr(), x.data_ptr(), weight.data_ptr(), gin,
+                                                    gw.data_ptr() if gw is not None else None, ws.data_ptr() if ws is not None else None,
+                                                    b, c, o, d, h, w, _stream(x)), "rag_conv3d_cc_bwd")
         return gx, gw, ggamma if need_gamma else None, gbeta if need_beta else None, None, None, None, None, None, None
 
 
@@ -136,7 +163,7 @@ def convbr_forward(layer: nn.Module, x: torch.Tensor) -> torch.Tensor:
     """A qualifying ConvBR_3d call on the kernels.  Updates the running statistics exactly like nn.BatchNorm3d does in
     train() (momentum or cumulative average, unbiased variance, batch count)."""
     if not layer.bn.training and not _wants_grad(layer, x):
-        return conv3d_cc_forward(x, layer.conv.weight, *batchnorm.eval_fold(layer.bn), relu=True)
+        return conv3d_cc_forward(x, layer.conv.weight, *batchnorm.eval_fold(layer.bn), relu=True, tf32=use_tf32(x.shape[1]))
     return batchnorm.apply(ConvBR3dFn, layer.bn, x.contiguous(), layer.conv.weight)
 
 

@@ -80,7 +80,7 @@ def basic_network_forward(self, left, right, fea_ops, mat_ops):
 
 def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_stem: bool = False, upsample: bool = False,
             matching_convs: bool = False, pointwise_convs: bool = False, resample: bool = False, resample_modules=(),
-            grid_sample: bool = False, grid_sample_modules=()) -> dict:
+            grid_sample: bool = False, grid_sample_modules=(), matching_tf32: bool = False) -> dict:
     """Bind the B200 hot path onto the reference's modules (pass the imported module objects
     ``models.rag_model`` and/or ``automl.mdenas_basicmodel``).  Returns what was patched.
     New networks constructed afterwards get ``rag_b200.Disp``; existing instances keep working
@@ -106,6 +106,11 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
     not qualify (``matching_conv.qualifies``) goes to the ``fuse_stem`` binding unchanged, so the fused stem, ``last_3_3d``
     and the cuDNN fallback behave as without the flag.
 
+    ``matching_tf32=True`` (needs ``matching_convs=True``, else ``ValueError``) runs those layers' convolutions on the tensor
+    cores in TF32 (csrc/conv3d_cc_tf32.cu): the forward and the data gradient, while ``torch.backends.cudnn.allow_tf32`` is on
+    at call time -- the precision the reference's cuDNN convolutions get by default.  BatchNorm and the weight gradient stay
+    fp32.  Every install() sets it, so a later install() without it, or uninstall(), turns it off.
+
     ``pointwise_convs=True`` (needs ``operations_3d``) binds ``ConvBR_3d.forward`` to ``rag_b200.pointwise_conv``'s
     ``pointwise_forward``: the Matching Net's pointwise ``ConvBR_3d(C, O, 1, 1, 0)`` layers (``last_12_3d``, ``last_6_3d``, the
     cells' 1x1x1 layers) that ``pointwise_conv.qualifies`` accepts run on csrc/conv3d_pw.cu in inference and training.  Every
@@ -128,6 +133,8 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
     module already holding a ``GridSampleProxy`` is not wrapped again.  A module without ``F`` raises ``ValueError``, as does
     the flag with no module; all modules are checked before any is bound."""
     global _FUSE_STEM, _STEM_AWARE
+    if matching_tf32 and not matching_convs:
+        raise ValueError("matching_tf32=True needs matching_convs=True (it selects the precision of those layers)")
     done = {}
 
     def bind(owner, name, value):
@@ -157,6 +164,9 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
         _STEM_AWARE = True
         done["operations_3d"] = ["ConvBR_3d.forward"]
     _FUSE_STEM = bool(fuse_stem)          # always (re)set: install(fuse_stem=False) after a fused install turns it off
+    from .matching_conv import set_tf32
+
+    set_tf32(matching_tf32)               # likewise
     if rag_model is not None:
         bind(rag_model.Network, "forward", network_forward)
         bind(rag_model.Network, "search_forward", network_search_forward)
@@ -218,6 +228,9 @@ def uninstall() -> int:
     _ORIGINALS.clear()
     _FUSE_STEM = False
     _STEM_AWARE = False
+    from .matching_conv import set_tf32
+
+    set_tf32(False)
     return n
 
 
