@@ -276,12 +276,20 @@ RAG_API int rag_conv3d_cc_bwd(const float* gz, const float* in, const float* w, 
 /* The same layers on the tensor cores in TF32 (csrc/conv3d_cc_tf32.cu): tcgen05.mma kind::tf32, both operands rounded to
  * TF32 with round-to-nearest (ties away) and summed in fp32 -- the precision cuDNN uses for these convolutions by default.
  * Same pairs, arguments, limits and errors as rag_conv3d_cc_fwd / the gin half of rag_conv3d_cc_bwd; stateless, capturable,
- * bitwise repeatable.  There is no TF32 weight gradient: rag_conv3d_cc_bwd with gin = NULL gives the fp32 one.
+ * bitwise repeatable.
  *   rag_conv3d_cc_tf32_fwd:      out = relu?( fma(z, scale, shift) ), z = the forward convolution of in by w.
- *   rag_conv3d_cc_tf32_bwd_data: gin[b,c,p] = sum_{o,k} w[o,c,k] gz[b,o,p-k+1]  (gz [B,O,D,H,W], gin [B,C,D,H,W]). */
+ *   rag_conv3d_cc_tf32_bwd_data: gin[b,c,p] = sum_{o,k} w[o,c,k] gz[b,o,p-k+1]  (gz [B,O,D,H,W], gin [B,C,D,H,W]).
+ *   rag_conv3d_cc_tf32_bwd_weight: gw[o,c,k] = sum_{b,p} gz[b,o,p] in[b,c,p+k-1]  (gw [O,C,3,3,3]), compiled for (8,8) and
+ *     (12,12) only: any other pair, (4,4) included, is RAG_E_SHAPE.  Otherwise the arguments, limits and errors of the gw half
+ *     of rag_conv3d_cc_bwd; gz / in 16-byte aligned, gw / workspace 4-byte.  workspace:
+ *     rag_conv3d_cc_tf32_bwd_weight_workspace_bytes(B,C,O,D,H,W) bytes (0 = unsupported pair; needs no device),
+ *     caller-owned.  Fixed-order per-CTA partials added in fp64, no atomics: the same bits on any device. */
 RAG_API int rag_conv3d_cc_tf32_fwd(const float* in, const float* w, const float* scale, const float* shift, int relu, float* out,
                            int B, int C, int O, int D, int H, int W, void* stream);
 RAG_API int rag_conv3d_cc_tf32_bwd_data(const float* gz, const float* w, float* gin, int B, int C, int O, int D, int H, int W, void* stream);
+RAG_API size_t rag_conv3d_cc_tf32_bwd_weight_workspace_bytes(int B, int C, int O, int D, int H, int W);
+RAG_API int rag_conv3d_cc_tf32_bwd_weight(const float* gz, const float* in, float* gw, void* workspace, int B, int C, int O, int D,
+                                  int H, int W, void* stream);
 
 /* The Matching Net's pointwise layers: ConvBR_3d(C, O, 1, 1, 0) of src/automl/operations_3d.py:31-47 = bias-free Conv3d
  * C -> O (1x1x1) + BatchNorm3d + ReLU -- `last_12_3d` (48 -> 24) and `last_6_3d` (24 -> 12) of src/models/rag_model.py.

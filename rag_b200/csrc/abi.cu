@@ -39,6 +39,8 @@ size_t conv3d_cc_bwd_workspace_bytes(int, int, int, int, int, int);
 int conv3d_cc_bwd(const float*, const float*, const float*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
 int conv3d_cc_tf32_fwd(const float*, const float*, const float*, const float*, int, float*, int, int, int, int, int, int, cudaStream_t);
 int conv3d_cc_tf32_bwd_data(const float*, const float*, float*, int, int, int, int, int, int, cudaStream_t);
+size_t conv3d_cc_tf32_bwd_weight_workspace_bytes(int, int, int, int, int, int);
+int conv3d_cc_tf32_bwd_weight(const float*, const float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
 int conv3d_pw_fwd(const float*, const float*, const float*, const float*, int, float*, int, int, int, int, int, int, cudaStream_t);
 size_t conv3d_pw_bwd_workspace_bytes(int, int, int, int, int, int);
 int conv3d_pw_bwd(const float*, const float*, const float*, const float*, const float*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
@@ -151,6 +153,13 @@ RAG_API int rag_conv3d_cc_tf32_fwd(const float* in, const float* w, const float*
 }
 RAG_API int rag_conv3d_cc_tf32_bwd_data(const float* gz, const float* w, float* gin, int B, int C, int O, int D, int H, int W, void* stream) {
     return conv3d_cc_tf32_bwd_data(gz, w, gin, B, C, O, D, H, W, ST(stream));
+}
+RAG_API size_t rag_conv3d_cc_tf32_bwd_weight_workspace_bytes(int B, int C, int O, int D, int H, int W) {
+    return conv3d_cc_tf32_bwd_weight_workspace_bytes(B, C, O, D, H, W);
+}
+RAG_API int rag_conv3d_cc_tf32_bwd_weight(const float* gz, const float* in, float* gw, void* workspace, int B, int C, int O, int D, int H,
+                                  int W, void* stream) {
+    return conv3d_cc_tf32_bwd_weight(gz, in, gw, static_cast<float*>(workspace), B, C, O, D, H, W, ST(stream));
 }
 RAG_API int rag_conv3d_pw_fwd(const float* in, const float* w, const float* scale, const float* shift, int relu, float* out,
                       int B, int C, int O, int D, int H, int W, void* stream) {

@@ -14,7 +14,9 @@ runs them in fp32 for (C, O) in ``PAIRS``:
 With ``install(..., matching_convs=True, matching_tf32=True)`` the convolutions of a qualifying call run on the tensor cores
 in TF32 (csrc/conv3d_cc_tf32.cu: the forward, and the data gradient) while ``torch.backends.cudnn.allow_tf32`` is on, read
 at call time -- the switch that makes the reference's own cuDNN convolutions TF32.  The BatchNorm and the weight gradient
-stay fp32, and so does 4 -> 4 (``use_tf32``).
+stay fp32, and so does 4 -> 4 (``use_tf32``).  With ``matching_tf32_wgrad=True`` as well, the weight gradient of such a call
+runs in TF32 too (``use_tf32_wgrad``; csrc/conv3d_cc_tf32.cu's weight-gradient kernel), so all three convolutions of a
+training step run at the precision cuDNN gives the reference.
 
 ``qualifies(layer, x)`` is the only routing decision; ``matching_forward`` -- bound onto ``ConvBR_3d.forward`` by
 ``rag_b200.network.install(..., matching_convs=True)`` -- sends qualifying plain-tensor calls here and everything else to
@@ -31,6 +33,7 @@ from .fused_stem import stem_forward
 
 PAIRS = ((4, 4), (8, 8), (12, 12))     # the (C, O) instantiations of csrc/conv3d_cc.cu (16 -> 16 lost to cuDNN: DESIGN.md 5.10)
 _TF32 = False                           # set by network.install(matching_tf32=...), cleared by network.uninstall()
+_TF32_WGRAD = False                     # likewise, by network.install(matching_tf32_wgrad=...)
 
 
 def set_tf32(on: bool) -> None:
@@ -38,11 +41,22 @@ def set_tf32(on: bool) -> None:
     _TF32 = bool(on)
 
 
+def set_tf32_wgrad(on: bool) -> None:
+    global _TF32_WGRAD
+    _TF32_WGRAD = bool(on)
+
+
 def use_tf32(c: int) -> bool:
     """True when a qualifying call with C input channels runs its convolutions in TF32: ``install(..., matching_tf32=True)``
     and torch's cuDNN TF32 switch (``torch.backends.cudnn.allow_tf32``) both on, and C > 4.  At C = 4 the TF32 kernel is no
     faster than the fp32 one on the measured shapes (DESIGN.md 5.10), so 4 -> 4 stays fp32."""
     return _TF32 and torch.backends.cudnn.allow_tf32 and c > 4
+
+
+def use_tf32_wgrad(c: int) -> bool:
+    """True when a qualifying training call with C input channels also takes its weight gradient from the TF32 kernel:
+    ``install(..., matching_tf32_wgrad=True)`` and ``use_tf32(c)``, both read at call time."""
+    return _TF32_WGRAD and use_tf32(c)
 
 
 def conv3d_cc_forward(x: torch.Tensor, weight: torch.Tensor, scale=None, shift=None, relu: bool = False,
@@ -83,11 +97,12 @@ class ConvBR3dFn(torch.autograd.Function):
     and the [O,4] table (scale, shift, mean, rstd) -- the reference's own layer keeps its conv output too, so no fourth
     convolution pass is spent on recomputing z.  The backward re-evaluates the forward's own ``fma(z, scale, shift) > 0`` for
     the ReLU decision (bit-identical).  ``use_tf32``, read once in the forward, puts z and the data gradient on the TF32
-    kernels; the weight gradient is the fp32 kernel's either way."""
+    kernels; ``use_tf32_wgrad``, read with it, puts the weight gradient there too, else it is the fp32 kernel's."""
 
     @staticmethod
     def forward(ctx, x, weight, gamma, beta, running_mean, running_var, batch_stats, update_running, momentum, eps):
         ctx.tf32 = use_tf32(x.shape[1])
+        ctx.tf32_wgrad = use_tf32_wgrad(x.shape[1])
         z = conv3d_cc_forward(x, weight, tf32=ctx.tf32)
         out = z.clone()
         bn = batchnorm.forward(z, out, gamma, beta, running_mean, running_var, batch_stats, update_running, momentum, eps)
@@ -109,14 +124,19 @@ class ConvBR3dFn(torch.autograd.Function):
             with torch.cuda.device(x.device):
                 gx = torch.empty_like(x) if need_x else None
                 gw = torch.empty_like(weight) if need_w else None
-                ws = torch.empty(int(L.rag_conv3d_cc_bwd_workspace_bytes(b, c, o, d, h, w)) // 4, dtype=torch.float32, device=x.device) if need_w else None
+                ws_bytes = L.rag_conv3d_cc_tf32_bwd_weight_workspace_bytes if ctx.tf32_wgrad else L.rag_conv3d_cc_bwd_workspace_bytes
+                ws = torch.empty(int(ws_bytes(b, c, o, d, h, w)) // 4, dtype=torch.float32, device=x.device) if need_w else None
                 if ctx.tf32 and gx is not None:      # TF32 data gradient; the fp32 call below then takes the weight gradient only
                     _cabi.check(L.rag_conv3d_cc_tf32_bwd_data(gz.data_ptr(), weight.data_ptr(), gx.data_ptr(), b, c, o, d, h, w, _stream(x)),
                                 "rag_conv3d_cc_tf32_bwd_data")
+                if ctx.tf32_wgrad and gw is not None:   # TF32 weight gradient: no fp32 call below
+                    _cabi.check(L.rag_conv3d_cc_tf32_bwd_weight(gz.data_ptr(), x.data_ptr(), gw.data_ptr(), ws.data_ptr(),
+                                                                b, c, o, d, h, w, _stream(x)), "rag_conv3d_cc_tf32_bwd_weight")
                 gin = None if ctx.tf32 or gx is None else gx.data_ptr()
-                if gin is not None or gw is not None:
-                    _cabi.check(L.rag_conv3d_cc_bwd(gz.data_ptr(), x.data_ptr(), weight.data_ptr(), gin,
-                                                    gw.data_ptr() if gw is not None else None, ws.data_ptr() if ws is not None else None,
+                gwp = None if ctx.tf32_wgrad or gw is None else gw.data_ptr()
+                if gin is not None or gwp is not None:
+                    _cabi.check(L.rag_conv3d_cc_bwd(gz.data_ptr(), x.data_ptr(), weight.data_ptr(), gin, gwp,
+                                                    ws.data_ptr() if gwp is not None else None,
                                                     b, c, o, d, h, w, _stream(x)), "rag_conv3d_cc_bwd")
         return gx, gw, ggamma if need_gamma else None, gbeta if need_beta else None, None, None, None, None, None, None
 
