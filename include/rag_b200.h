@@ -273,6 +273,17 @@ RAG_API size_t rag_conv3d_cc_bwd_workspace_bytes(int B, int C, int O, int D, int
 RAG_API int rag_conv3d_cc_bwd(const float* gz, const float* in, const float* w, float* gin, float* gw, void* workspace,
                       int B, int C, int O, int D, int H, int W, void* stream);
 
+/* The level-12 op, (C, O) = (16, 16), on a small-volume geometry (csrc/conv3d_cc.cu): the arguments, results, limits and
+ * errors of rag_conv3d_cc_fwd / rag_conv3d_cc_bwd, compiled for (16,16) only -- any other pair is RAG_E_SHAPE -- plus a
+ * weight-gradient tile count B*D*ceil(H/2)*ceil(W/32) < 2^31.  fp32, stateless, capturable; the weight gradient is fixed-order
+ * per-CTA partials added in fp64, no atomics: the same bits on any device.  workspace:
+ * rag_conv3d_cc16_bwd_workspace_bytes(B,C,O,D,H,W) bytes (0 = unsupported pair; needs no device), caller-owned. */
+RAG_API int rag_conv3d_cc16_fwd(const float* in, const float* w, const float* scale, const float* shift, int relu, float* out,
+                        int B, int C, int O, int D, int H, int W, void* stream);
+RAG_API size_t rag_conv3d_cc16_bwd_workspace_bytes(int B, int C, int O, int D, int H, int W);
+RAG_API int rag_conv3d_cc16_bwd(const float* gz, const float* in, const float* w, float* gin, float* gw, void* workspace,
+                        int B, int C, int O, int D, int H, int W, void* stream);
+
 /* The same layers on the tensor cores in TF32 (csrc/conv3d_cc_tf32.cu): tcgen05.mma kind::tf32, both operands rounded to
  * TF32 with round-to-nearest (ties away) and summed in fp32 -- the precision cuDNN uses for these convolutions by default.
  * Same pairs, arguments, limits and errors as rag_conv3d_cc_fwd / the gin half of rag_conv3d_cc_bwd; stateless, capturable,

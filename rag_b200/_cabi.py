@@ -58,6 +58,9 @@ SIGNATURES = {
     "rag_conv3d_cc_fwd": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_conv3d_cc_bwd_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i, _i]),
     "rag_conv3d_cc_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "rag_conv3d_cc16_fwd": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "rag_conv3d_cc16_bwd_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i, _i]),
+    "rag_conv3d_cc16_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_conv3d_cc_tf32_fwd": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_conv3d_cc_tf32_bwd_data": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "rag_conv3d_cc_tf32_bwd_weight_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i, _i]),

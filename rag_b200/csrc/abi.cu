@@ -37,6 +37,9 @@ int cv_stem_bwd(const float*, const float*, const float*, const float*, const fl
 int conv3d_cc_fwd(const float*, const float*, const float*, const float*, int, float*, int, int, int, int, int, int, cudaStream_t);
 size_t conv3d_cc_bwd_workspace_bytes(int, int, int, int, int, int);
 int conv3d_cc_bwd(const float*, const float*, const float*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
+size_t conv3d_cc16_bwd_workspace_bytes(int, int, int, int, int, int);
+int conv3d_cc16_fwd(const float*, const float*, const float*, const float*, int, float*, int, int, int, int, int, int, cudaStream_t);
+int conv3d_cc16_bwd(const float*, const float*, const float*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
 int conv3d_cc_tf32_fwd(const float*, const float*, const float*, const float*, int, float*, int, int, int, int, int, int, cudaStream_t);
 int conv3d_cc_tf32_bwd_data(const float*, const float*, float*, int, int, int, int, int, int, cudaStream_t);
 size_t conv3d_cc_tf32_bwd_weight_workspace_bytes(int, int, int, int, int, int);
@@ -146,6 +149,15 @@ RAG_API size_t rag_conv3d_cc_bwd_workspace_bytes(int B, int C, int O, int D, int
 RAG_API int rag_conv3d_cc_bwd(const float* gz, const float* in, const float* w, float* gin, float* gw, void* workspace,
                       int B, int C, int O, int D, int H, int W, void* stream) {
     return conv3d_cc_bwd(gz, in, w, gin, gw, static_cast<float*>(workspace), B, C, O, D, H, W, ST(stream));
+}
+RAG_API int rag_conv3d_cc16_fwd(const float* in, const float* w, const float* scale, const float* shift, int relu, float* out,
+                        int B, int C, int O, int D, int H, int W, void* stream) {
+    return conv3d_cc16_fwd(in, w, scale, shift, relu, out, B, C, O, D, H, W, ST(stream));
+}
+RAG_API size_t rag_conv3d_cc16_bwd_workspace_bytes(int B, int C, int O, int D, int H, int W) { return conv3d_cc16_bwd_workspace_bytes(B, C, O, D, H, W); }
+RAG_API int rag_conv3d_cc16_bwd(const float* gz, const float* in, const float* w, float* gin, float* gw, void* workspace,
+                        int B, int C, int O, int D, int H, int W, void* stream) {
+    return conv3d_cc16_bwd(gz, in, w, gin, gw, static_cast<float*>(workspace), B, C, O, D, H, W, ST(stream));
 }
 RAG_API int rag_conv3d_cc_tf32_fwd(const float* in, const float* w, const float* scale, const float* shift, int relu, float* out,
                            int B, int C, int O, int D, int H, int W, void* stream) {

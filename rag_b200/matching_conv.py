@@ -18,9 +18,13 @@ stay fp32, and so does 4 -> 4 (``use_tf32``).  With ``matching_tf32_wgrad=True``
 runs in TF32 too (``use_tf32_wgrad``; csrc/conv3d_cc_tf32.cu's weight-gradient kernel), so all three convolutions of a
 training step run at the precision cuDNN gives the reference.
 
-``qualifies(layer, x)`` is the only routing decision; ``matching_forward`` -- bound onto ``ConvBR_3d.forward`` by
-``rag_b200.network.install(..., matching_convs=True)`` -- sends qualifying plain-tensor calls here and everything else to
-``fused_stem.stem_forward`` unchanged.
+The level-12 cells' ``conv_3x3`` op, ``ConvBR_3d(16, 16, 3, 1, 1)``, runs on entries of its own (``rag_conv3d_cc16_*``: the
+same kernels on a geometry for small volumes) under ``install(..., matching_convs=True, level12_convs=True)``
+(``level12_qualifies``); it stays fp32 under the TF32 flags, which have no 16 -> 16 kernels.
+
+``qualifies(layer, x)`` -- and, with ``level12_convs``, ``level12_qualifies(layer, x)`` -- is the only routing decision;
+``matching_forward`` -- bound onto ``ConvBR_3d.forward`` by ``rag_b200.network.install(..., matching_convs=True)`` -- sends
+qualifying plain-tensor calls here and everything else to ``fused_stem.stem_forward`` unchanged.
 """
 from __future__ import annotations
 
@@ -32,8 +36,11 @@ from .functional import _require, _stream
 from .fused_stem import stem_forward
 
 PAIRS = ((4, 4), (8, 8), (12, 12))     # the (C, O) instantiations of csrc/conv3d_cc.cu (16 -> 16 lost to cuDNN: DESIGN.md 5.10)
+LEVEL12_PAIR = (16, 16)                 # the level-12 op: its own entries, rag_conv3d_cc16_* (DESIGN.md 5.10.3)
+LEVEL12_MIN_VOXELS = 2 ** 17            # B*D*H*W from which the level-12 op trains faster than on cuDNN TF32 (DESIGN.md 5.10.3)
 _TF32 = False                           # set by network.install(matching_tf32=...), cleared by network.uninstall()
 _TF32_WGRAD = False                     # likewise, by network.install(matching_tf32_wgrad=...)
+_LEVEL12 = False                        # likewise, by network.install(level12_convs=...)
 
 
 def set_tf32(on: bool) -> None:
@@ -46,11 +53,16 @@ def set_tf32_wgrad(on: bool) -> None:
     _TF32_WGRAD = bool(on)
 
 
+def set_level12(on: bool) -> None:
+    global _LEVEL12
+    _LEVEL12 = bool(on)
+
+
 def use_tf32(c: int) -> bool:
     """True when a qualifying call with C input channels runs its convolutions in TF32: ``install(..., matching_tf32=True)``
     and torch's cuDNN TF32 switch (``torch.backends.cudnn.allow_tf32``) both on, and C > 4.  At C = 4 the TF32 kernel is no
-    faster than the fp32 one on the measured shapes (DESIGN.md 5.10), so 4 -> 4 stays fp32."""
-    return _TF32 and torch.backends.cudnn.allow_tf32 and c > 4
+    faster than the fp32 one on the measured shapes (DESIGN.md 5.10), so 4 -> 4 stays fp32; 16 -> 16 has no TF32 kernel."""
+    return _TF32 and torch.backends.cudnn.allow_tf32 and c > 4 and c != LEVEL12_PAIR[0]
 
 
 def use_tf32_wgrad(c: int) -> bool:
@@ -63,7 +75,7 @@ def conv3d_cc_forward(x: torch.Tensor, weight: torch.Tensor, scale=None, shift=N
                       tf32: bool = False) -> torch.Tensor:
     """out = relu?(fma(conv3d(x, weight, padding=1), scale, shift)) for weight [O,C,3,3,3]; x [B,C,D,H,W] CUDA fp32.
     scale / shift [O] (both or neither) fold an eval-mode BatchNorm into the store.  ``tf32`` runs the convolution on the
-    tensor cores (``rag_conv3d_cc_tf32_fwd``), else in fp32 (``rag_conv3d_cc_fwd``)."""
+    tensor cores (``rag_conv3d_cc_tf32_fwd``), else in fp32 (``rag_conv3d_cc_fwd``; ``rag_conv3d_cc16_fwd`` for 16 -> 16)."""
     _require(x, "x"), _require(weight, "weight")
     if x.dim() != 5:
         raise RuntimeError(f"rag_b200: conv3d_cc wants a [B,C,D,H,W] input, got {tuple(x.shape)}")
@@ -80,7 +92,7 @@ def conv3d_cc_forward(x: torch.Tensor, weight: torch.Tensor, scale=None, shift=N
     if scale is not None:
         scale, shift = scale.contiguous(), shift.contiguous()
     L = _cabi.lib()
-    name = "rag_conv3d_cc_tf32_fwd" if tf32 else "rag_conv3d_cc_fwd"
+    name = "rag_conv3d_cc_tf32_fwd" if tf32 else "rag_conv3d_cc16_fwd" if (c, o) == LEVEL12_PAIR else "rag_conv3d_cc_fwd"
     with torch.cuda.device(x.device):
         rc = getattr(L, name)(x.data_ptr(), weight.data_ptr(), scale.data_ptr() if scale is not None else None,
                               shift.data_ptr() if shift is not None else None, int(bool(relu)), out.data_ptr(),
@@ -97,7 +109,8 @@ class ConvBR3dFn(torch.autograd.Function):
     and the [O,4] table (scale, shift, mean, rstd) -- the reference's own layer keeps its conv output too, so no fourth
     convolution pass is spent on recomputing z.  The backward re-evaluates the forward's own ``fma(z, scale, shift) > 0`` for
     the ReLU decision (bit-identical).  ``use_tf32``, read once in the forward, puts z and the data gradient on the TF32
-    kernels; ``use_tf32_wgrad``, read with it, puts the weight gradient there too, else it is the fp32 kernel's."""
+    kernels; ``use_tf32_wgrad``, read with it, puts the weight gradient there too, else it is the fp32 kernel's.  16 -> 16 runs
+    on the fp32 ``rag_conv3d_cc16_*`` entries."""
 
     @staticmethod
     def forward(ctx, x, weight, gamma, beta, running_mean, running_var, batch_stats, update_running, momentum, eps):
@@ -124,7 +137,8 @@ class ConvBR3dFn(torch.autograd.Function):
             with torch.cuda.device(x.device):
                 gx = torch.empty_like(x) if need_x else None
                 gw = torch.empty_like(weight) if need_w else None
-                ws_bytes = L.rag_conv3d_cc_tf32_bwd_weight_workspace_bytes if ctx.tf32_wgrad else L.rag_conv3d_cc_bwd_workspace_bytes
+                bwd = "rag_conv3d_cc16_bwd" if (c, o) == LEVEL12_PAIR else "rag_conv3d_cc_bwd"
+                ws_bytes = L.rag_conv3d_cc_tf32_bwd_weight_workspace_bytes if ctx.tf32_wgrad else getattr(L, bwd + "_workspace_bytes")
                 ws = torch.empty(int(ws_bytes(b, c, o, d, h, w)) // 4, dtype=torch.float32, device=x.device) if need_w else None
                 if ctx.tf32 and gx is not None:      # TF32 data gradient; the fp32 call below then takes the weight gradient only
                     _cabi.check(L.rag_conv3d_cc_tf32_bwd_data(gz.data_ptr(), weight.data_ptr(), gx.data_ptr(), b, c, o, d, h, w, _stream(x)),
@@ -135,9 +149,8 @@ class ConvBR3dFn(torch.autograd.Function):
                 gin = None if ctx.tf32 or gx is None else gx.data_ptr()
                 gwp = None if ctx.tf32_wgrad or gw is None else gw.data_ptr()
                 if gin is not None or gwp is not None:
-                    _cabi.check(L.rag_conv3d_cc_bwd(gz.data_ptr(), x.data_ptr(), weight.data_ptr(), gin, gwp,
-                                                    ws.data_ptr() if gwp is not None else None,
-                                                    b, c, o, d, h, w, _stream(x)), "rag_conv3d_cc_bwd")
+                    _cabi.check(getattr(L, bwd)(gz.data_ptr(), x.data_ptr(), weight.data_ptr(), gin, gwp,
+                                                ws.data_ptr() if gwp is not None else None, b, c, o, d, h, w, _stream(x)), bwd)
         return gx, gw, ggamma if need_gamma else None, gbeta if need_beta else None, None, None, None, None, None, None
 
 
@@ -145,16 +158,20 @@ def _wants_grad(layer: nn.Module, x: torch.Tensor) -> bool:
     return torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in layer.parameters()))
 
 
+def _layer_is(layer: nn.Module, pairs) -> bool:
+    conv = getattr(layer, "conv", None)
+    if not (isinstance(conv, nn.Conv3d) and conv.bias is None and conv.kernel_size == (3, 3, 3) and conv.stride == (1, 1, 1)
+            and conv.padding == (1, 1, 1) and conv.dilation == (1, 1, 1) and conv.groups == 1 and conv.padding_mode == "zeros"
+            and conv.weight.dtype == torch.float32 and (conv.in_channels, conv.out_channels) in pairs):
+        return False
+    return batchnorm.bn_relu_qualifies(layer, conv.out_channels)
+
+
 def layer_qualifies(layer: nn.Module) -> bool:
     """The layer half of ``qualifies``, independent of devices: ``layer`` (a ConvBR_3d: .conv, .bn, .use_bn, .relu) is a
     Conv3d 3x3x3 / stride 1 / padding 1 / dilation 1 / groups 1, bias-free (the kernels have no bias term), zero padding,
     fp32, with (C, O) in PAIRS, followed by an affine fp32 BatchNorm3d that tracks running statistics and a ReLU."""
-    conv = getattr(layer, "conv", None)
-    if not (isinstance(conv, nn.Conv3d) and conv.bias is None and conv.kernel_size == (3, 3, 3) and conv.stride == (1, 1, 1)
-            and conv.padding == (1, 1, 1) and conv.dilation == (1, 1, 1) and conv.groups == 1 and conv.padding_mode == "zeros"
-            and conv.weight.dtype == torch.float32 and (conv.in_channels, conv.out_channels) in PAIRS):
-        return False
-    return batchnorm.bn_relu_qualifies(layer, conv.out_channels)
+    return _layer_is(layer, PAIRS)
 
 
 def qualifies(layer: nn.Module, x) -> bool:
@@ -162,7 +179,22 @@ def qualifies(layer: nn.Module, x) -> bool:
     and x a CUDA fp32 [B,C,D,H,W] tensor on the weight's device with W % 4 == 0 and within the kernels' limits.  Whenever
     batch statistics are used or a gradient is wanted, also the limits of the BatchNorm kernels (csrc/bn3d.cu):
     O <= 32, D >= 3, 8 <= W <= 1016."""
-    if not layer_qualifies(layer) or not layer.conv.weight.is_cuda:
+    return layer_qualifies(layer) and _input_qualifies(layer, x)
+
+
+def level12_qualifies(layer: nn.Module, x) -> bool:
+    """``qualifies`` for the level-12 op: the same layer, BatchNorm / ReLU and input clauses and limits, with (C, O) =
+    LEVEL12_PAIR -- the layer the ``rag_conv3d_cc16_*`` entries implement -- for training calls (batch statistics or a
+    gradient) of at least LEVEL12_MIN_VOXELS voxels.  The eval forward, and training below that size, are faster on cuDNN
+    TF32 at the measured shapes (DESIGN.md 5.10.3), so they stay there."""
+    if not (_layer_is(layer, (LEVEL12_PAIR,)) and _input_qualifies(layer, x)):
+        return False
+    b, _, d, h, w = x.shape
+    return (layer.bn.training or _wants_grad(layer, x)) and b * d * h * w >= LEVEL12_MIN_VOXELS
+
+
+def _input_qualifies(layer: nn.Module, x) -> bool:
+    if not layer.conv.weight.is_cuda:
         return False
     conv, bn = layer.conv, layer.bn
     if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() == 5 and x.device == conv.weight.device
@@ -189,6 +221,6 @@ def convbr_forward(layer: nn.Module, x: torch.Tensor) -> torch.Tensor:
 
 def matching_forward(self, x):
     """Replacement for ConvBR_3d.forward (operations_3d.py:41-47) under ``install(..., matching_convs=True)``."""
-    if isinstance(x, torch.Tensor) and qualifies(self, x):
+    if isinstance(x, torch.Tensor) and (qualifies(self, x) or _LEVEL12 and level12_qualifies(self, x)):
         return convbr_forward(self, x)
     return stem_forward(self, x)

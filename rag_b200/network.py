@@ -81,7 +81,7 @@ def basic_network_forward(self, left, right, fea_ops, mat_ops):
 def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_stem: bool = False, upsample: bool = False,
             matching_convs: bool = False, pointwise_convs: bool = False, resample: bool = False, resample_modules=(),
             grid_sample: bool = False, grid_sample_modules=(), matching_tf32: bool = False,
-            matching_tf32_wgrad: bool = False) -> dict:
+            matching_tf32_wgrad: bool = False, level12_convs: bool = False) -> dict:
     """Bind the B200 hot path onto the reference's modules (pass the imported module objects
     ``models.rag_model`` and/or ``automl.mdenas_basicmodel``).  Returns what was patched.
     New networks constructed afterwards get ``rag_b200.Disp``; existing instances keep working
@@ -116,6 +116,10 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
     TF32 as well (``matching_conv.use_tf32_wgrad``: the same call-time rule), so a training step's three convolutions all
     run at cuDNN's default precision.  It changes results, so it is a flag of its own; every install() sets it too.
 
+    ``level12_convs=True`` (needs ``matching_convs=True``, else ``ValueError``) also routes the level-12 cells' ``conv_3x3``
+    op, ``ConvBR_3d(16, 16, 3, 1, 1)`` (``matching_conv.level12_qualifies``), onto the kernels, in fp32 under any TF32 flag.
+    Every install() sets it, so a later install() without it, or uninstall(), turns it off.
+
     ``pointwise_convs=True`` (needs ``operations_3d``) binds ``ConvBR_3d.forward`` to ``rag_b200.pointwise_conv``'s
     ``pointwise_forward``: the Matching Net's pointwise ``ConvBR_3d(C, O, 1, 1, 0)`` layers (``last_12_3d``, ``last_6_3d``, the
     cells' 1x1x1 layers) that ``pointwise_conv.qualifies`` accepts run on csrc/conv3d_pw.cu in inference and training.  Every
@@ -142,6 +146,8 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
         raise ValueError("matching_tf32=True needs matching_convs=True (it selects the precision of those layers)")
     if matching_tf32_wgrad and not matching_tf32:
         raise ValueError("matching_tf32_wgrad=True needs matching_tf32=True (it extends TF32 to those layers' weight gradient)")
+    if level12_convs and not matching_convs:
+        raise ValueError("level12_convs=True needs matching_convs=True (it extends that binding to the 16 -> 16 layers)")
     done = {}
 
     def bind(owner, name, value):
@@ -171,10 +177,11 @@ def install(rag_model=None, mdenas_basicmodel=None, operations_3d=None, fuse_ste
         _STEM_AWARE = True
         done["operations_3d"] = ["ConvBR_3d.forward"]
     _FUSE_STEM = bool(fuse_stem)          # always (re)set: install(fuse_stem=False) after a fused install turns it off
-    from .matching_conv import set_tf32, set_tf32_wgrad
+    from .matching_conv import set_level12, set_tf32, set_tf32_wgrad
 
     set_tf32(matching_tf32)               # likewise
     set_tf32_wgrad(matching_tf32_wgrad)
+    set_level12(level12_convs)
     if rag_model is not None:
         bind(rag_model.Network, "forward", network_forward)
         bind(rag_model.Network, "search_forward", network_search_forward)
@@ -236,10 +243,11 @@ def uninstall() -> int:
     _ORIGINALS.clear()
     _FUSE_STEM = False
     _STEM_AWARE = False
-    from .matching_conv import set_tf32, set_tf32_wgrad
+    from .matching_conv import set_level12, set_tf32, set_tf32_wgrad
 
     set_tf32(False)
     set_tf32_wgrad(False)
+    set_level12(False)
     return n
 
 
